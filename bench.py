@@ -4,6 +4,8 @@
   python bench.py [--gpus N] [--steps K] [--warmup W]            our sm_100a path, training step (headline)
   python bench.py --workload infer [--gpus N] ...                batched inference + greedy CTC decode (config 4)
   python bench.py --impl reference ...                           the reference algorithm on the host CPU
+  python bench.py ... --dump-outputs DIR                         also write what the last timed step returned as
+                                                                 DIR/<name>.npy (same arguments -> same inputs)
 
 Workload (BASELINE.json configs[1]): one HTR-VT IAM-shape training step = encoder forward (train mode,
 span masking 0.4/8) + CTC loss + backward of every trainable parameter, batch 128 per GPU, 1x64x512
@@ -181,13 +183,14 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
-def inference_metrics(torch, dist, dev, h, ops, model, world, rank, steps, lines_per_gpu=512):
+def inference_metrics(torch, dist, dev, h, ops, model, world, rank, steps, lines_per_gpu=512, keep=None):
     """BASELINE.json config 4: batched inference + greedy CTC decode, 512 synthetic lines per GPU (4096 over 8 GPUs),
     sharded by batch with NO collective on the data path (ddp.shard_batch); each rank decodes its own shard to Python
     strings.  Two timings, both max over ranks between barriers:
       value : images resident in HBM, eval forward + decode kernels (ids stay on the device);
       e2e   : through the public API with HOST buffers - pinned fp32 images -> H2D -> model(image) ->
-              converter.decode_logits (argmax + collapse on device, ONE D2H copy of ids + lengths, id -> str)."""
+              converter.decode_logits (argmax + collapse on device, ONE D2H copy of ids + lengths, id -> str).
+    keep: a dict that receives the logits, ids and lengths of the last resident batch."""
     conv = h.CTCLabelConverter("".join(chr(33 + i) for i in range(NB_CLS - 1)))
     img_h = synth_batch(lines_per_gpu, 1000 + rank)[0].pin_memory()
     img_d = img_h.to(dev)
@@ -196,7 +199,11 @@ def inference_metrics(torch, dist, dev, h, ops, model, world, rank, steps, lines
 
     def resident():
         with torch.no_grad():
-            return h.greedy_decode(model(img_d).float(), NB_CLS)
+            logits = model(img_d).float()
+            ids, lens = h.greedy_decode(logits, NB_CLS)
+        if keep is not None:
+            keep.update(logits=logits, ids=ids, lens=lens)
+        return ids, lens
 
     pf = h.HostPrefetcher(dev)                   # batch i+1's 67 MB H2D copy runs under batch i's kernels
     pf.put(img_h)
@@ -704,6 +711,38 @@ def load_peaks():
     return json.load(open(p)) if os.path.exists(p) else {}
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+GRAD_SAMPLE = 1 << 22              # gradient entries --dump-outputs writes (16.8 MB of the 214 MB of one step)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy.  float64 stays float64, other floating point becomes float32,
+    integers (token ids, lengths) become float64, which holds them exactly."""
+    import numpy as np
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        out[name] = a if a.dtype == np.float64 else a.astype(np.float64 if a.dtype.kind in "iub" else np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def train_step_outputs(torch, loss, logits, params):
+    """What one training step hands its caller: the loss, the model's logits and every parameter's .grad.  The
+    gradients are written as their per-tensor L2 norms (all tensors) and the entries at a fixed, seeded sample of
+    positions in their concatenation (model.parameters() order, ascending positions)."""
+    import numpy as np
+    flat = torch.cat([p.grad.reshape(-1) for p in params])
+    idx = np.sort(np.random.default_rng(0).choice(flat.numel(), min(GRAD_SAMPLE, flat.numel()), replace=False))
+    return {"loss": loss, "logits": logits,
+            "grad_norms": torch.stack([p.grad.double().norm() for p in params]),
+            "grad_sample": flat[torch.from_numpy(idx).to(flat.device)]}
+
+
 def run_infer(args):
     """--workload infer: BASELINE.json config 4 as its own JSON line (batched inference + greedy CTC decode, 512
     lines per GPU, batch sharding, no collective)."""
@@ -714,8 +753,11 @@ def run_infer(args):
     if rank == 0:
         clocks.start()
     clocks.mark()                         # (inference_metrics warms up inside; its two timed legs follow back to back)
-    m = inference_metrics(torch, dist, dev, h, ops, model, world, rank, steps=args.steps)
+    last = {}
+    m = inference_metrics(torch, dist, dev, h, ops, model, world, rank, steps=args.steps, keep=last)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     # roofline of the tap-GEMM family inside one inference batch (CUDA events per op on the launching stream)
     img = synth_batch(m["lines_per_gpu"], 1000 + rank)[0].to(dev)
     ops.PROFILE = []
@@ -800,11 +842,13 @@ def run_ours(args):
     img_h, tg_h, tl_h = img_h.pin_memory(), tg_h.pin_memory(), tl_h.pin_memory()
     img_d, tg_d, tl_d = img_h.to(dev), tg_h.to(dev), tl_h.to(dev)
     params = [p for p in model.parameters() if p.requires_grad]
+    last = {}                                    # the latest step's logits and loss (--dump-outputs)
 
     def compute_loss(image, text, length):
         # model_v1/train.py:21-30 with the drop-in model / criterion
         preds = model(image, MASK_RATIO, MAX_SPAN, use_masking=True)
         preds = preds.float()
+        last["logits"] = preds.detach()
         preds_size = torch.full((B,), preds.size(1), dtype=torch.int32, device=dev)
         preds = preds.permute(1, 0, 2).log_softmax(2)
         return criterion(preds, text, preds_size, length).mean()
@@ -814,6 +858,7 @@ def run_ours(args):
             p.grad = None
         loss = compute_loss(img_d, tg_d, tl_d)
         loss.backward()
+        last["loss"] = loss
         return loss
 
     # end to end: every step copies ITS inputs from pinned host memory (16.8 MB) and reads its loss back.  The copies
@@ -873,6 +918,8 @@ def run_ours(args):
     total_ms = timed(step_resident, args.steps)
     launches = ops.launch_count() - n0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:          # before the next step clears .grad
+        dump_outputs(args.dump_outputs, train_step_outputs(torch, last["loss"], last["logits"], params))
     step_e2e()
     e2e_ms = timed(step_e2e, args.steps, meter.total)
     import math
@@ -999,7 +1046,15 @@ def main():
                          "infer: eval forward + greedy decode, 512 lines/GPU (config 4)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the CTC / inference / window-variant side metrics")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (train: loss, logits, gradient norms "
+                         "and a seeded gradient sample; infer: logits, ids, lengths) as DIR/<name>.npy, rank 0 only; "
+                         "bench_outputs/ in the checkout is git-ignored")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this project's GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "infer":

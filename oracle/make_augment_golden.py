@@ -5,9 +5,12 @@ scikit-image, is replaced by oracle/skimage_stub (a restatement of the four symb
 projective-warp leg is therefore "parity unpinned", oracle/augment_oracle.py header).
 
 Writes tests/golden/augment_cases.npz: inputs, per-case (numpy, torch) seeds and the collate's outputs for seeds that
-cover all eight gate combinations.  Usage: python oracle/make_augment_golden.py
+cover all eight gate combinations; and tests/golden/augment_rng_after.json: per seed, the next np.random.rand() and
+torch.rand(1) after the collate (checked against the same draws after draw_collate_params).
+Usage: python oracle/make_augment_golden.py
 """
 import importlib
+import json
 import os
 import sys
 import types
@@ -67,17 +70,23 @@ def main():
     B, H, W = 3, 64, 256
     imgs = synthetic_lines(rs, B, H, W)
     batch = [(imgs[i], "label%d" % i) for i in range(B)]
-    seen, seeds, outs = set(), [], []
+    seen, seeds, outs, after = set(), [], [], []
     seed = 0
     while len(seen) < 8 and seed < 400:
         seed += 1
         np.random.seed(seed); torch.manual_seed(seed)
         p = aug.draw_collate_params(B, H, W, args)
+        mine = [np.random.rand(), float(torch.rand(1))]
         combo = tuple(p[k] is not None for k in ("warp", "morph", "jitter"))
         if combo in seen and not (combo[1] and len(seeds) < 14):
             continue
         np.random.seed(seed); torch.manual_seed(seed)
         out, labels = collate(batch, args)
+        # the next draw of each global generator: where the collate leaves them, including draws that do not change
+        # the output (saturation / hue factors on grey images)
+        nxt = [np.random.rand(), float(torch.rand(1))]
+        assert mine == nxt, (seed, combo, mine, nxt)
+        after.append(nxt)
         assert list(labels) == ["label%d" % i for i in range(B)]
         got = np.round(out.numpy()[:, 0] * 255).astype(np.uint8)
         # the product's draw order + the oracle's pixel arithmetic reproduce the reference's output
@@ -89,6 +98,10 @@ def main():
                         seeds=np.array(seeds, dtype=np.int64), outputs=np.stack(outs),
                         args=np.array([args.proj, args.dila_ero_max_kernel, args.dila_ero_iter, args.jitter_brightness,
                                        args.jitter_contrast, args.jitter_saturation, args.jitter_hue]))
+    with open(os.path.join(OUT, "augment_rng_after.json"), "w") as fh:
+        json.dump({"source": "the reference SameTrCollate (oracle/make_augment_golden.py)", "seeds": seeds,
+                   "next_np_torch": after}, fh, indent=1)
+        fh.write("\n")
     print(len(seeds), "cases, all", len(seen), "gate combinations")
 
 

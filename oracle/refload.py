@@ -1,8 +1,7 @@
-"""Import the UNMODIFIED reference modules from /root/reference (dev container only).
+"""Import the UNMODIFIED reference modules from an upstream HTR-VT source tree (set HTRVT_REFERENCE to it).
 
-TEST INFRASTRUCTURE ONLY. /root/reference does not exist on the GPU box, so nothing in
-`-m gpu` tests, smoke() or bench.py may call this; it is used by oracle/make_golden.py and
-by `-m "not gpu"` tests that skip when the tree is absent.
+TEST INFRASTRUCTURE ONLY: oracle/make_golden.py uses it to regenerate tests/golden/.  The tree is not part of this
+repository, so nothing in the test suite, smoke() or bench.py may call this.
 """
 import importlib
 import os

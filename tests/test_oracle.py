@@ -129,24 +129,6 @@ def test_argmax_semantics_match_torch_max():
     np.testing.assert_array_equal(O.argmax_first(g["logits"]), g["index"])
 
 
-def test_live_reference_when_present():
-    """If the reference tree is mounted (dev container), compare against it live on a fresh seed."""
-    import refload
-    if not refload.available():
-        pytest.skip("reference tree not mounted")
-    htr, utl = refload.load_variant("model_v1")
-    sd = O.init_state_dict(80, [64, 512], seed=77)
-    ref = htr.create_model(80, [64, 512])
-    ref.load_state_dict(sd, strict=True)
-    ref.eval()
-    x = _images(78, 1, 512)
-    with torch.no_grad():
-        a = ref(x)
-        b = O.forward(sd, x)
-    np.testing.assert_allclose(a.numpy(), b.numpy(), atol=2e-4)
-    assert list(ref.state_dict().keys()) == list(O.reorder_like(sd, ref.state_dict().keys()).keys())
-
-
 def test_metrics_oracle_matches_reference_formatting_and_known_answers():
     """format_string_for_wer against strings produced by the reference's own function; Levenshtein against
     classic known answers, a brute-force check and metric axioms; the valid.py:49-75 accumulation."""

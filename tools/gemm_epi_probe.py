@@ -1,6 +1,6 @@
 """Timing of fc2's input-gradient GEMM with the fused activation backward (EPI 4) against the plain GEMM."""
 import sys, os, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from importlib import import_module
 import htrvt_b200
 o = import_module("htr-vt_b200.ops")

@@ -1,5 +1,6 @@
 import os, sys
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/oracle')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'oracle'))
 import numpy as np, torch
 from functools import partial
 from importlib import import_module
