@@ -118,6 +118,7 @@ SIGNATURES = {
     "htrvt_row_ln_f32": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _F, _P]),
     "htrvt_gelu_split": (_I, [_P, _P, _L, _P]),
     "htrvt_attention_f32": (_I, [_P, _I, _I, _I, _I, _F, _P, _P]),
+    "htrvt_attention2_f32": (_I, [_P, _I, _I, _I, _I, _F, _P, _I, _I, _I, _P, _P]),
 }
 
 

@@ -586,7 +586,9 @@ int a2_map3(CUtensorMap* m, const void* ptr, long long cols, long long rows, lon
   return r == CUDA_SUCCESS ? HTRVT_OK : HTRVT_ERR_DRIVER;
 }
 
-int a2_check(int B, int H, int T, int hd, int window, int shift, int Prel, const void* table) {
+}  // namespace
+
+int htrvt::attention2_check(int B, int H, int T, int hd, int window, int shift, int Prel, const void* table) {
   if (hd != kA2Hd || T < 1 || T > 256 || B < 1 || H < 1) return HTRVT_ERR_SHAPE;
   if (window != 0 && window != 16) return HTRVT_ERR_SHAPE;
   if (window == 0 && shift != 0) return HTRVT_ERR_SHAPE;
@@ -595,7 +597,6 @@ int a2_check(int B, int H, int T, int hd, int window, int shift, int Prel, const
   if (!table && Prel != 0 && Prel < T) return HTRVT_ERR_SHAPE;
   return HTRVT_OK;
 }
-}  // namespace
 
 // Attention with relative-position bias, global (window = 0) or 16-token windows over the sequence rolled by
 // -shift (model_window/model/HTR_VT.py:33-62, 114-154).  qkv bf16 token-major [B][T][3*H*128]; out bf16
@@ -603,7 +604,7 @@ int a2_check(int B, int H, int T, int hd, int window, int shift, int Prel, const
 extern "C" int htrvt_attention2_fwd(const void* qkv, int B, int H, int T, int hd, float scale, const float* table,
                                     int Prel, int window, int shift, float drop_p, unsigned long long seed, void* out,
                                     float* lse, cudaStream_t stream) {
-  int r = a2_check(B, H, T, hd, window, shift, Prel, table);
+  int r = attention2_check(B, H, T, hd, window, shift, Prel, table);
   if (r) return r;
   if (!table) Prel = 256;
   const long long ld = 3LL * H * kA2Hd;
@@ -638,7 +639,7 @@ extern "C" int htrvt_attention2_bwd(const void* qkv, const void* out, const void
                                     int T, int hd, float scale, const float* table, int Prel, int window, int shift,
                                     float drop_p, unsigned long long seed, void* dqkv, float* dtable, void* workspace,
                                     size_t workspace_bytes, cudaStream_t stream) {
-  int r = a2_check(B, H, T, hd, window, shift, Prel, table);
+  int r = attention2_check(B, H, T, hd, window, shift, Prel, table);
   if (r) return r;
   if (!lse) return HTRVT_ERR_SHAPE;
   if (!table) { Prel = 256; dtable = nullptr; }

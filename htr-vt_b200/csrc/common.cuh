@@ -372,4 +372,10 @@ __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N, int a_mn, i
          (static_cast<uint32_t>(M >> 4) << 24);
 }
 
+// Argument rules of the windowed variant's attention (attention2.cu), shared by its 16-bit entry and the fp32 one
+// (exact.cu) so both precisions accept the same models and lines: head_dim 128, 1 <= T <= 256, window 0 or 16, shift 0
+// for global blocks and a multiple of 8 below the window otherwise, a bias table of 2 * Prel - 1 <= 511 rows with
+// Prel >= T.  HTRVT_OK or HTRVT_ERR_SHAPE.
+int attention2_check(int B, int H, int T, int hd, int window, int shift, int Prel, const void* table);
+
 }  // namespace htrvt

@@ -193,6 +193,83 @@ __global__ void __launch_bounds__(128) attention_f32_kernel(const float* __restr
   }
 }
 
+// softmax(q k^T * scale + bias) v in fp32 with the windowed variant's semantics (model_window/model/HTR_VT.py:33-62,
+// 114-154; htrvt_attention2_fwd is its 16-bit counterpart).  CTA shape, lane split and arithmetic of
+// attention_f32_kernel; bias = table[(j - i) + Prel - 1][h], the head's column staged in shared memory.
+//   global   (window 0): the CTA's 32 queries scan all T keys in tiles of 32.
+//   windowed (window 16): the sequence is zero-padded to Tp = ceil16(T) and rolled by -shift, so rolled position p
+//     holds token (p + shift) mod Tp.  A CTA takes 32 consecutive rolled positions = two windows, stages their keys
+//     once, and each row reads only the 16 keys of its own window (i, j window-local: the wrap-around window mixes head
+//     and tail tokens, as the reference does).  Keys of padded tokens (>= T) are skipped, i.e. weight exactly 0 as
+//     the reference's finfo.min fill gives; padded query rows are never stored.  A warp's 8 rows share one window,
+//     so the skip is warp-uniform.
+__global__ void __launch_bounds__(128) attention2_f32_kernel(const float* __restrict__ qkv, float* __restrict__ out,
+                                                             const float* __restrict__ table, int B, int H, int T,
+                                                             int Prel, int window, int shift, float scale) {
+  __shared__ float ks[kExKeys][kExHd + 4];
+  __shared__ float vs[kExKeys][kExHd + 4];
+  __shared__ float bias[512];
+  const int Tp = window ? (T + window - 1) / window * window : T;
+  const int qblocks = (Tp + kExRows - 1) / kExRows;
+  const int qb = blockIdx.x % qblocks, bh = blockIdx.x / qblocks;
+  const int h = bh % H, b = bh / H;
+  const int r = threadIdx.x >> 2, part = threadIdx.x & 3;
+  const int pos = qb * kExRows + r;                         // query position (rolled when windowed)
+  auto token = [&](int p) { const int t = p + shift; return t >= Tp ? t - Tp : t; };
+  const long long tok_stride = 3LL * H * kExHd;
+  const float* base = qkv + static_cast<long long>(b) * T * tok_stride + h * kExHd;
+  for (int i = threadIdx.x; i < 512; i += blockDim.x) bias[i] = (table && i < 2 * Prel - 1) ? table[i * H + h] : 0.f;
+  const int tq = token(pos);
+  const bool ok = pos < Tp && tq < T;
+  float q[32], o[32];
+#pragma unroll
+  for (int i = 0; i < 32; ++i) {
+    q[i] = ok ? base[static_cast<long long>(tq) * tok_stride + part * 32 + i] * 1.0f : 0.f;
+    o[i] = 0.f;
+  }
+  float mx = -INFINITY, sum = 0.f;
+  const int ntiles = window ? 1 : (T + kExKeys - 1) / kExKeys;
+  for (int tile = 0; tile < ntiles; ++tile) {
+    const int p0 = window ? qb * kExRows : tile * kExKeys;   // first key position of the tile
+    __syncthreads();                                         // (also publishes `bias` before the first tile)
+    for (int i = threadIdx.x; i < kExKeys * kExHd; i += blockDim.x) {
+      const int kk = i / kExHd, d = i - kk * kExHd;
+      const int tk = token(p0 + kk);
+      const bool kv_ok = p0 + kk < Tp && tk < T;
+      const float* tp = base + static_cast<long long>(tk) * tok_stride;
+      ks[kk][d] = kv_ok ? tp[H * kExHd + d] : 0.f;
+      vs[kk][d] = kv_ok ? tp[2 * H * kExHd + d] : 0.f;
+    }
+    __syncthreads();
+    const int lo = window ? (r & ~15) : 0;
+    const int hi = window ? lo + 16 : min(kExKeys, T - p0);
+    for (int kk = lo; kk < hi; ++kk) {
+      const int p = p0 + kk;
+      if (p >= Tp || token(p) >= T) continue;               // padded key (windowed only)
+      float s = 0.f;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) s = fmaf(q[i], ks[kk][part * 32 + i], s);
+      s += __shfl_xor_sync(0xffffffffu, s, 1);
+      s += __shfl_xor_sync(0xffffffffu, s, 2);
+      // (q k^T) * scale, then + bias: the reference's two roundings.  The clamp only acts on rows that are never
+      // stored (global, pos >= T) and on windowed tables shorter than the window, which the reference cannot build
+      s = __fmul_rn(s, scale) + bias[max(p - pos + Prel - 1, 0)];
+      const float nm = fmaxf(mx, s);
+      const float corr = expf(mx - nm), pr = expf(s - nm);  // first key: mx = -inf -> corr = 0
+      sum = sum * corr + pr;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) o[i] = fmaf(o[i], corr, pr * vs[kk][part * 32 + i]);
+      mx = nm;
+    }
+  }
+  if (ok) {
+    const float inv = 1.0f / sum;
+    float* op = out + (static_cast<long long>(b) * T + tq) * (H * kExHd) + h * kExHd + part * 32;
+#pragma unroll
+    for (int i = 0; i < 32; ++i) op[i] = o[i] * inv;
+  }
+}
+
 }  // namespace htrvt
 
 using namespace htrvt;
@@ -259,6 +336,19 @@ extern "C" int htrvt_attention_f32(const float* qkv, int B, int H, int T, int hd
   if (B <= 0 || H <= 0 || T <= 0 || hd != kExHd || !qkv || !out) return HTRVT_ERR_SHAPE;
   const int qblocks = (T + kExRows - 1) / kExRows;
   attention_f32_kernel<<<B * H * qblocks, 128, 0, stream>>>(qkv, out, B, H, T, scale);
+  HTRVT_LAUNCH_CHECK();
+  return HTRVT_OK;
+}
+
+extern "C" int htrvt_attention2_f32(const float* qkv, int B, int H, int T, int hd, float scale, const float* table,
+                                    int Prel, int window, int shift, float* out, cudaStream_t stream) {
+  const int r = attention2_check(B, H, T, hd, window, shift, Prel, table);
+  if (r) return r;
+  if (!qkv || !out) return HTRVT_ERR_SHAPE;
+  if (!table) Prel = 256;                                   // no table: a zero bias column
+  const int Tp = window ? (T + window - 1) / window * window : T;
+  const int qblocks = (Tp + kExRows - 1) / kExRows;
+  attention2_f32_kernel<<<B * H * qblocks, 128, 0, stream>>>(qkv, out, table, B, H, T, Prel, window, shift, scale);
   HTRVT_LAUNCH_CHECK();
   return HTRVT_OK;
 }

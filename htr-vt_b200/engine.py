@@ -356,10 +356,8 @@ class Engine(object):
 
     def forward_fp32(self, sd, image, mask=None, widths=None, chunk=32):
         """Eval-mode forward with fp32 tensors between kernels and split-bf16 tensor-core contractions (csrc/exact.cu;
-        model_v1/model/HTR_VT.py:222-241, model_v1/model/resnet18.py:73-84 with running statistics).
-        -> logits fp32 [B, T, C].  model_v1 only."""
-        if self.variant != "v1":
-            raise ops.HtrvtError("precision='fp32' is implemented for model_v1 (north_star parity row)")
+        model_v1/model/HTR_VT.py:222-241, model_window/model/HTR_VT.py:320-337, model_v1/model/resnet18.py:73-84 with
+        running statistics).  -> logits fp32 [B, T, C]."""
         if image.shape[0] > chunk:                      # fp32 activations: bound the working set
             return torch.cat([self.forward_fp32(sd, image[i:i + chunk], mask,
                                                 None if widths is None else widths[i:i + chunk], chunk)
@@ -402,7 +400,13 @@ class Engine(object):
             h1p, x1 = ops.row_ln_f32(xs, sd[p + ".norm1.weight"], sd[p + ".norm1.bias"], self.ln_eps, pend)
             qkv = torch.empty((M, 3 * D), dtype=torch.float32, device=dev)
             ops.gemm_tn_split(h1p, wp[p + ".attn.qkv.weight"], qkv, sd[p + ".attn.qkv.bias"])
-            op = ops.split3(ops.attention_f32(qkv, B, self.H, T, self.hd, self.hd ** -0.5))
+            if self.variant == "v1":
+                o = ops.attention_f32(qkv, B, self.H, T, self.hd, self.hd ** -0.5)
+            else:
+                tbl = sd[p + ".attn.relative_position_bias_table"]
+                ws, sh = self.windows[i]
+                o = ops.attention2_f32(qkv, B, self.H, T, self.hd, self.hd ** -0.5, tbl, (tbl.shape[0] + 1) // 2, ws, sh)
+            op = ops.split3(o)
             y1 = torch.empty((M, D), dtype=torch.float32, device=dev)
             ops.gemm_tn_split(op, wp[p + ".attn.proj.weight"], y1, sd[p + ".attn.proj.bias"])
             h2p, x2 = ops.row_ln_f32(x1, sd[p + ".norm2.weight"], sd[p + ".norm2.bias"], self.ln_eps, y1)
@@ -418,6 +422,8 @@ class Engine(object):
         ops.gemm_tn_split(hfp, wp["head.weight"], raw_logits, hb)
         if C8 != C:
             raw_logits = raw_logits[:, :C].contiguous()
+        if self.variant != "v1":                        # the windowed variant has no LayerNorm on the logits
+            return raw_logits.view(B, T, C)
         logits, _, _ = ops.sample_ln_fwd(raw_logits.view(B, T, C), torch.float32, 1e-5)
         return logits
 

@@ -194,7 +194,9 @@ class MaskedAutoencoderViT(nn.Module):
     def set_precision(self, precision):
         """"bf16" (default): 16-bit tensor-core operands, fp32 accumulation - the product path.  "fp32": eval-mode
         parity forward (fp32 tensors, split-bf16 contractions): logits within 1e-4 of the fp32 reference and greedy
-        decode strings identical to it (north_star); forward only, under model.eval() + torch.no_grad()."""
+        decode strings identical to it (north_star); forward only, under model.eval() + torch.no_grad().  Both
+        variants: model_v1 and the windowed model (model_window), whose fp32 attention keeps its relative-position
+        bias, shifted 16-token windows and padded lines."""
         if precision not in ("bf16", "fp32"):
             raise ValueError("precision must be 'bf16' or 'fp32'")
         self.engine.precision = precision

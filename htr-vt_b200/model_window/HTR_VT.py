@@ -6,7 +6,9 @@ attention in the rest, no LayerNorm on the logits, and train-mode Dropout(0.1) /
 DropPath(linspace(0, 0.1, depth)).  Same state_dict keys, shapes and order as the reference (tests/golden/win_*.npz).
 
 As in model.HTR_VT the nn.Modules are parameter containers; the arithmetic runs in the sm_100a kernels
-(csrc/attention2.cu for the attention).  Train-mode randomness: the reference draws its masks from the device
+(csrc/attention2.cu for the attention).  `set_precision("fp32")` selects the eval-mode fp32-parity forward here as
+for model_v1 (csrc/exact.cu, htrvt_attention2_f32 for the attention): use it where an evaluation - greedy decode or the
+LM-rescored beam - must return what the reference returns on the same weights.  Train-mode randomness: the reference draws its masks from the device
 generator, so only the distribution can match - here every mask is a counter-based hash of a seed drawn per
 forward from torch's CPU generator (reproducible under torch.manual_seed), regenerated in the backward.
 """

@@ -899,6 +899,22 @@ def attention_f32(qkv, B, H, T, hd, scale):
     return out
 
 
+def attention2_f32(qkv, B, H, T, hd, scale, table=None, prel=0, window=0, shift=0, out=None):
+    """Windowed-variant attention in fp32 (eval: no dropout): qkv fp32 [B*T, 3*H*hd] -> fp32 [B*T, H*hd] (written
+    into `out` when given).  Relative-position bias table fp32 [2*prel-1, H] (None: no bias), window 0 (global) or 16
+    with shift 0 or 8, as attention2_fwd."""
+    _need_cuda(qkv, table, out)
+    if qkv.dtype != torch.float32 or not qkv.is_contiguous() or (table is not None and table.dtype != torch.float32):
+        raise HtrvtError("attention2_f32 needs contiguous fp32 qkv and an fp32 bias table")
+    if out is None:
+        out = torch.empty((B * T, H * hd), dtype=torch.float32, device=qkv.device)
+    elif out.dtype != torch.float32 or not out.is_contiguous() or out.numel() != B * T * H * hd:
+        raise HtrvtError("attention2_f32: out must be a contiguous fp32 tensor of B*T*H*hd elements")
+    check(lib().htrvt_attention2_f32(_p(qkv), B, H, T, hd, scale, _p(table), prel, window, shift, _p(out), _stream()),
+          "htrvt_attention2_f32")
+    return out
+
+
 def launch_count() -> int:
     """Kernels launched by the library so far (host-side counter in the C library)."""
     fn = lib().htrvt_launch_count
@@ -959,6 +975,19 @@ def _flops(name, a, kw):
         if name == "attention_bwd":
             B, T, _, H, hd = a[0].shape
             return 10.0 * B * H * T * T * hd
+        if name == "conv_fwd_split":                             # six bf16 products
+            xp, wp, ks, sh, sw = a[:5]
+            Ho, Wo = conv_out_hw(xp.shape[2], xp.shape[3], ks, sh, sw)
+            return 6 * 2.0 * xp.shape[1] * Ho * Wo * wp.shape[1] * ks * ks * xp.shape[4]
+        if name == "attention_f32":
+            B, H, T, hd = a[1:5]
+            return 4.0 * B * H * T * T * hd
+        if name == "attention2_f32":
+            B, H, T, hd = a[1:5]
+            window = a[8] if len(a) > 8 else kw.get("window", 0)
+            if window:                                           # every query sees the 16 keys of its window
+                return 4.0 * B * H * ((T + window - 1) // window * window) * window * hd
+            return 4.0 * B * H * T * T * hd
     except Exception:
         pass
     return 0.0
@@ -968,7 +997,7 @@ def _instrument():
     import functools
     g = globals()
     names = ["gemm_tn", "gemm_nn", "linear_wgrad", "conv_fwd", "conv_dgrad", "conv_dgrad_bn", "conv_wgrad", "conv_wgrad_acc", "conv_wgrad_acc_t", "conv_wgrad_acc_w", "unpack_conv_grads", "attention_fwd",
-             "attention_bwd", "attention2_fwd", "attention2_bwd", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
+             "attention_bwd", "attention2_fwd", "attention2_bwd", "attention_f32", "attention2_f32", "split3", "conv_fwd_split", "bn_act_f32", "maxpool_f32", "tokens_f32", "row_ln_f32", "gelu_split", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
              "row_ln_fwd", "row_ln_bwd", "tokens_fwd", "tokens_bwd", "gelu_fwd", "gelu_bwd", "colsum_bf16", "cast_bf16", "cast_colsum_bf16", "dropout_",
              "pack_conv_weight", "pack_weights", "conv1_fwd", "bn_finalize", "bn_act_fwd", "pool_fwd", "pool_bwd", "bn_bwd", "bn_bwd_apply",
              "conv1_wgrad", "stem_head_moments", "stem_head_fwd", "stem_head_bwd"]

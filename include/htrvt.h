@@ -177,7 +177,8 @@ int htrvt_attention_bwd(const void* qkv, const void* out, const void* dout, cons
 
 /* ---- attention of the windowed variant (model_window/model/HTR_VT.py:33-62 Attention.forward with
  * relative_position_bias_table, :114-154 Block._attend: roll by -shift, 16-token windows, roll back), T <= 256.
- * table: fp32 [2*Prel-1][H] or NULL; window: 0 (global) or 16; shift: multiple of 8 (needs T % 128 == 0 when > 0);
+ * table: fp32 [2*Prel-1][H] or NULL; window: 0 (global) or 16; shift: 0, or 8 with window 16 (any T <= 256: the
+ * sequence is zero-padded to a multiple of 16, padded keys masked, padded query rows not stored);
  * drop_p / seed: attention dropout as a counter-based hash of (seed, b, h, query token, key token) - the backward
  * regenerates the mask.  dtable (+=) is accumulated with fp32 atomics.  workspace: partial dQ for global T > 128. */
 int htrvt_attention2_fwd(const void* qkv, int B, int H, int T, int hd, float scale, const float* table, int Prel,
@@ -325,7 +326,8 @@ int htrvt_edit_distance(const int* a, const int* a_off, int a_stride, const int*
  * output: htrvt_gemm_tn with EPI_ACCUM, htrvt_conv_fwd with flags 2048 | 16).  These entry points are the fp32
  * element-wise steps in between; `planes` = bf16 [3][n] (nullable where noted).
  * Reference lines: model_v1/model/HTR_VT.py:27-39 (attention), :68-83 (block), :134-136 / :224 / :236-239 (LayerNorms),
- * model_v1/model/resnet18.py:23-39,73-84 (BatchNorm eval, ReLU, residual, max-pool), timm Mlp (erf GELU). */
+ * model_window/model/HTR_VT.py:33-62, 114-154 (the windowed variant's attention), model_v1/model/resnet18.py:23-39,73-84
+ * (BatchNorm eval, ReLU, residual, max-pool), timm Mlp (erf GELU). */
 int htrvt_split3(const float* src, void* planes_bf16, long long n, void* stream);
 int htrvt_bn_act_f32(const float* raw, const float* scale, const float* shift, const float* res, const float* raw2,
                      const float* scale2, const float* shift2, float* y /*nullable*/, void* planes_bf16 /*nullable*/,
@@ -339,6 +341,12 @@ int htrvt_row_ln_f32(const float* x, const float* addend /*nullable*/, float* x_
 int htrvt_gelu_split(const float* u, void* planes_bf16, long long n, void* stream);
 int htrvt_attention_f32(const float* qkv /*[B,T,3,H,hd]*/, int B, int H, int T, int hd, float scale,
                         float* out /*[B,T,H*hd]*/, void* stream);
+/* softmax(q k^T * scale + bias) v of the windowed variant (model_window/model/HTR_VT.py:33-62 Attention.forward with
+ * relative_position_bias_table, :114-154 Block._attend) in fp32: the semantics of htrvt_attention2_fwd without dropout
+ * or lse.  qkv fp32 [B][T][3][H][128] as the split GEMM writes it, out fp32 [B][T][H*128]; table fp32 [2*Prel-1][H] or
+ * NULL.  Accepts exactly the shapes htrvt_attention2_fwd accepts (same HTRVT_ERR_SHAPE rules). */
+int htrvt_attention2_f32(const float* qkv, int B, int H, int T, int hd, float scale, const float* table, int Prel,
+                         int window, int shift, float* out, void* stream);
 
 #ifdef __cplusplus
 }
