@@ -606,6 +606,7 @@ extern "C" int htrvt_attention2_fwd(const void* qkv, int B, int H, int T, int hd
                                     float* lse, cudaStream_t stream) {
   int r = attention2_check(B, H, T, hd, window, shift, Prel, table);
   if (r) return r;
+  if (!(drop_p >= 0.f && drop_p < 1.f)) return HTRVT_ERR_SHAPE;     // (also refuses NaN)
   if (!table) Prel = 256;
   const long long ld = 3LL * H * kA2Hd;
   const int nblk = (T + 127) / 128;
@@ -641,7 +642,7 @@ extern "C" int htrvt_attention2_bwd(const void* qkv, const void* out, const void
                                     size_t workspace_bytes, cudaStream_t stream) {
   int r = attention2_check(B, H, T, hd, window, shift, Prel, table);
   if (r) return r;
-  if (!lse) return HTRVT_ERR_SHAPE;
+  if (!lse || !(drop_p >= 0.f && drop_p < 1.f)) return HTRVT_ERR_SHAPE;
   if (!table) { Prel = 256; dtable = nullptr; }
   const long long ld = 3LL * H * kA2Hd, ldo = static_cast<long long>(H) * kA2Hd;
   const int nblk = (T + 127) / 128;

@@ -798,7 +798,7 @@ extern "C" int htrvt_pack_weights(int n, const void* const* src, void* const* ds
 // x bf16 [n] in place; per_sample = elements per batch sample (DropPath scale dp[b], nullable); n, per_sample % 8 == 0
 extern "C" int htrvt_dropout_bf16(void* x, long long n, long long per_sample, float p, unsigned long long seed,
                                   unsigned site, const float* dp, cudaStream_t stream) {
-  if (n <= 0 || (n & 7) || per_sample <= 0 || (per_sample & 7) || p < 0.f || p >= 1.f) return HTRVT_ERR_SHAPE;
+  if (n <= 0 || (n & 7) || per_sample <= 0 || (per_sample & 7) || !(p >= 0.f && p < 1.f)) return HTRVT_ERR_SHAPE;
   const long long n8 = n / 8;
   const int blocks = static_cast<int>((n8 + 255) / 256 < 148 * 16 ? (n8 + 255) / 256 : 148 * 16);
   dropout_bf16_kernel<<<blocks, 256, 0, stream>>>(static_cast<__nv_bfloat16*>(x), n8, per_sample / 8, p,

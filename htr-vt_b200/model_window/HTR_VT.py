@@ -89,9 +89,17 @@ class MaskedAutoencoderViT(_BaseViT):
                     nn.init.zeros_(m.bias)
 
     def set_stochastic(self, drop=0.1, attn_drop=0.05, drop_path_rate=0.1):
-        """Override the train-mode regularisation rates (0 everywhere makes train mode deterministic)."""
-        self.drop, self.attn_drop = float(drop), float(attn_drop)
-        self.drop_path = torch.linspace(0, float(drop_path_rate), steps=len(self.blocks)).tolist()
+        """Override the train-mode regularisation rates (0 everywhere makes train mode deterministic).  drop and
+        attn_drop lie in [0, 1); drop_path_rate, the last block's DropPath rate, in [0, 1] (1 drops that block's
+        branches for every sample)."""
+        drop, attn_drop, drop_path_rate = float(drop), float(attn_drop), float(drop_path_rate)
+        for name, v in (("drop", drop), ("attn_drop", attn_drop)):
+            if not 0.0 <= v < 1.0:                  # (also refuses NaN)
+                raise ValueError("%s must lie in [0, 1), got %r" % (name, v))
+        if not 0.0 <= drop_path_rate <= 1.0:
+            raise ValueError("drop_path_rate must lie in [0, 1], got %r" % drop_path_rate)
+        self.drop, self.attn_drop = drop, attn_drop
+        self.drop_path = torch.linspace(0, drop_path_rate, steps=len(self.blocks)).tolist()
         return self
 
     def _train_rng(self, batch, device):
@@ -110,7 +118,10 @@ class MaskedAutoencoderViT(_BaseViT):
             keep = 1.0 - rate
             pair = []
             for _ in range(2):
-                pair.append(((torch.rand(batch, generator=gen) < keep).float() / keep).to(device, non_blocking=True))
+                kept = (torch.rand(batch, generator=gen) < keep).float()
+                if keep > 0:                        # keep = 0 drops every sample: zeros, no 0 / 0 (as timm)
+                    kept = kept / keep
+                pair.append(kept.to(device, non_blocking=True))
             dps.append(tuple(pair))
         return {"seed": seed, "drop": self.drop, "attn_drop": self.attn_drop, "drop_path": dps}
 

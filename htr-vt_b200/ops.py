@@ -551,7 +551,7 @@ def gelu_bwd(da, u):
 
 def dropout_(x, per_sample, p, seed, site, dp=None):
     """In-place inverted dropout of probability p (+ per-sample DropPath scale dp [B] fp32) on a bf16 tensor."""
-    if p <= 0.0 and dp is None:
+    if p == 0.0 and dp is None:                  # (a p outside [0, 1) reaches the kernel entry, which refuses it)
         return x
     check(lib().htrvt_dropout_bf16(_p(x), x.numel(), per_sample, float(p), int(seed), int(site), _p(dp), _stream()),
           "htrvt_dropout_bf16")

@@ -180,7 +180,8 @@ int htrvt_attention_bwd(const void* qkv, const void* out, const void* dout, cons
  * table: fp32 [2*Prel-1][H] or NULL; window: 0 (global) or 16; shift: 0, or 8 with window 16 (any T <= 256: the
  * sequence is zero-padded to a multiple of 16, padded keys masked, padded query rows not stored);
  * drop_p / seed: attention dropout as a counter-based hash of (seed, b, h, query token, key token) - the backward
- * regenerates the mask.  dtable (+=) is accumulated with fp32 atomics.  workspace: partial dQ for global T > 128. */
+ * regenerates the mask; drop_p must lie in [0, 1) (NaN, negative or >= 1: HTRVT_ERR_SHAPE, nothing launched).
+ * dtable (+=) is accumulated with fp32 atomics.  workspace: partial dQ for global T > 128. */
 int htrvt_attention2_fwd(const void* qkv, int B, int H, int T, int hd, float scale, const float* table, int Prel,
                          int window, int shift, float drop_p, unsigned long long seed, void* out, float* lse,
                          void* stream);
@@ -226,7 +227,8 @@ int htrvt_cast_bf16(const float* src, void* dst, long long n, void* stream);
 int htrvt_cast_colsum_bf16(const float* src, void* dst, float* colsum, int M, int N, void* stream);
 /* in-place inverted dropout (+ per-sample DropPath scale dp[b], nullable) on bf16 x[n]; counter-based mask keyed by
  * (seed, site, element index): the same call on the gradient regenerates the mask.  Replaces nn.Dropout / timm
- * DropPath of model_window (model_window/model/HTR_VT.py:21-23, 100-110, 263-273) in train mode. */
+ * DropPath of model_window (model_window/model/HTR_VT.py:21-23, 100-110, 263-273) in train mode.  p must lie in
+ * [0, 1) (NaN, negative or >= 1: HTRVT_ERR_SHAPE, nothing launched). */
 int htrvt_dropout_bf16(void* x, long long n, long long per_sample, float p, unsigned long long seed, unsigned site,
                        const float* dp, void* stream);
 int htrvt_pack_weights(int n, const void* const* src, void* const* dst, const long long* numel, const int* cin,

@@ -190,12 +190,16 @@ def stem_forward(sd, x, training):
     return F.max_pool2d(x, 3, (2, 1), 1)
 
 
-def _attention(sd, p, x, num_heads, window=0, shift=0):
+def _attention(sd, p, x, num_heads, window=0, shift=0, regs=None):
     """Attention.forward (model_v1/model/HTR_VT.py:27-39); with the window variant's relative
-    bias and 1-D window partition (model_window/model/HTR_VT.py:33-62, 114-154)."""
+    bias and 1-D window partition (model_window/model/HTR_VT.py:33-62, 114-154).
+    regs: optional dict of one block's train-mode regularisers (see train_regs): "attn" multiplies the attention
+    probabilities after the softmax (timm attn_drop), "proj" the projection's output (timm proj_drop)."""
     has_bias = (p + ".relative_position_bias_table") in sd
+    ascale = regs.get("attn") if regs is not None else None
+    pscale = regs.get("proj") if regs is not None else None
 
-    def attend(z, key_mask=None):
+    def attend(z, key_mask=None, drop=None):
         Bz, N, C = z.shape
         hd = C // num_heads
         qkv = F.linear(z, sd[p + ".qkv.weight"], sd[p + ".qkv.bias"])
@@ -210,11 +214,14 @@ def _attention(sd, p, x, num_heads, window=0, shift=0):
         attn = attn.softmax(dim=-1)
         if key_mask is not None:
             attn = torch.nan_to_num(attn, nan=0.0)
+        if drop is not None:                           # attention dropout: after the softmax, before @ v
+            attn = attn * drop.to(attn.dtype)
         z = (attn @ v).transpose(1, 2).reshape(Bz, N, C)
         return F.linear(z, sd[p + ".proj.weight"], sd[p + ".proj.bias"])
 
     if window <= 0:
-        return attend(x)
+        x = attend(x, drop=ascale)
+        return x if pscale is None else x * pscale.to(x.dtype)
     # Block._attend (model_window/model/HTR_VT.py:114-154): zero-pad to a multiple of the window, roll tokens and
     # the validity mask by -shift, attend inside consecutive windows with the padded keys masked, undo, strip
     B, N0, C = x.shape
@@ -228,23 +235,52 @@ def _attention(sd, p, x, num_heads, window=0, shift=0):
     if shift > 0:
         x = torch.roll(x, shifts=(-shift,), dims=1)
         valid = torch.roll(valid, shifts=(-shift,), dims=1)
-    x = attend(x.reshape(B * (N // window), window, C), valid.reshape(B * (N // window), window)).reshape(B, N, C)
+    drop = window_attention_scale(ascale, window, shift) if ascale is not None else None
+    x = attend(x.reshape(B * (N // window), window, C), valid.reshape(B * (N // window), window),
+               drop).reshape(B, N, C)
     if shift > 0:
         x = torch.roll(x, shifts=(shift,), dims=1)
-    return x[:, :N0]
+    x = x[:, :N0]
+    return x if pscale is None else x * pscale.to(x.dtype)
 
 
-def _mlp(sd, p, x):
-    """timm 1.0.9 Mlp with nn.GELU (erf form); dropouts are p=0 in model_v1."""
+def window_attention_scale(scale, window, shift):
+    """[B, H, Tp, Tp] attention keep-scale over ORIGINAL token indices (Tp = T padded to a multiple of the window) ->
+    [B * Tp / window, H, window, window] in the layout of Block._attend's windows: rolled position r holds token
+    (r + shift) mod Tp, and only the pairs inside one window are kept."""
+    B, H, Tp, _ = scale.shape
+    nw = Tp // window
+    tok = (torch.arange(Tp, device=scale.device) + shift) % Tp
+    s = scale[:, :, tok][:, :, :, tok].reshape(B, H, nw, window, nw, window)
+    s = torch.diagonal(s, dim1=2, dim2=4)                      # [B, H, window, window, nw]
+    return s.permute(0, 4, 1, 2, 3).reshape(B * nw, H, window, window)
+
+
+def _mlp(sd, p, x, regs=None):
+    """timm 1.0.9 Mlp with nn.GELU (erf form): fc1 -> GELU -> drop1 -> fc2 -> drop2; dropouts are p=0 in model_v1,
+    regs["fc1"] / regs["fc2"] (train_regs) are the keep-scales of drop1 / drop2."""
     h = F.gelu(F.linear(x, sd[p + ".fc1.weight"], sd[p + ".fc1.bias"]))
-    return F.linear(h, sd[p + ".fc2.weight"], sd[p + ".fc2.bias"])
+    if regs is not None and regs.get("fc1") is not None:
+        h = h * regs["fc1"].to(h.dtype)
+    y = F.linear(h, sd[p + ".fc2.weight"], sd[p + ".fc2.bias"])
+    if regs is not None and regs.get("fc2") is not None:
+        y = y * regs["fc2"].to(y.dtype)
+    return y
 
 
-def forward(sd, x, mask=None, training=False, num_heads=6, ln_eps=1e-6, variant="v1"):
+def _drop_path(y, dp):
+    """timm DropPath with a given per-sample scale dp [B] (0 or 1 / keep)."""
+    return y if dp is None else y * dp.to(y.dtype).reshape(-1, 1, 1)
+
+
+def forward(sd, x, mask=None, training=False, num_heads=6, ln_eps=1e-6, variant="v1", regs=None):
     """MaskedAutoencoderViT.forward (model_v1/model/HTR_VT.py:222-241;
     model_window/model/HTR_VT.py:320-337 in eval mode / dropout disabled).
 
     `mask`: optional float [T] (1 keep / 0 masked) as produced by draw_span_mask.
+    `regs`: optional list of per-block train-mode regulariser dicts (train_regs) injected in timm 1.0.9's places
+    (SURVEY.md 13): softmax -> attention dropout -> @ v; proj -> dropout -> DropPath; fc1 -> GELU -> dropout -> fc2 ->
+    dropout -> DropPath.  None: no dropout and no DropPath (the arithmetic is then unchanged).
     In train mode BN running statistics in `sd` are updated in place, as the reference does."""
     D = sd["norm.weight"].shape[0]
     x = F.layer_norm(x, x.shape[1:], None, None, 1e-5)                      # :224
@@ -262,10 +298,13 @@ def forward(sd, x, mask=None, training=False, num_heads=6, ln_eps=1e-6, variant=
         win, shift = (0, 0)
         if variant == "window":
             win, shift = ((16, 0), (16, 8), (0, 0), (0, 0))[i] if i < 4 else (0, 0)
+        blk = regs[i] if regs is not None else None
         h = F.layer_norm(x, (D,), sd[p + ".norm1.weight"], sd[p + ".norm1.bias"], ln_eps)
-        x = x + _attention(sd, p + ".attn", h, num_heads, win, shift)
+        y = _attention(sd, p + ".attn", h, num_heads, win, shift, blk)
+        x = x + (y if blk is None else _drop_path(y, blk.get("dp1")))
         h = F.layer_norm(x, (D,), sd[p + ".norm2.weight"], sd[p + ".norm2.bias"], ln_eps)
-        x = x + _mlp(sd, p + ".mlp", h)
+        y = _mlp(sd, p + ".mlp", h, blk)
+        x = x + (y if blk is None else _drop_path(y, blk.get("dp2")))
     x = F.layer_norm(x, (D,), sd["norm.weight"], sd["norm.bias"], ln_eps)   # :236
     x = F.linear(x, sd["head.weight"], sd["head.bias"])                     # :238
     if variant == "v1":
@@ -588,8 +627,9 @@ def grad_sample_index(name, numel, n=8192):
     return np.sort(rs.choice(numel, size=n, replace=False))
 
 
-def train_step(sd, image, targets, target_lengths, mask, variant="v1", num_heads=6):
-    """compute_loss + backward (model_v1/train.py:21-30,122-123) with an explicit span mask.
+def train_step(sd, image, targets, target_lengths, mask, variant="v1", num_heads=6, regs=None):
+    """compute_loss + backward (model_v1/train.py:21-30,122-123) with an explicit span mask and optional
+    train-mode regularisers (`regs`, see forward / train_regs).
     Returns (loss, {name: grad}) for every floating-point parameter except pos_embed."""
     names = [k for k, v in sd.items() if v.is_floating_point() and "running_" not in k and k != "pos_embed"]
     work = OrderedDict(sd)
@@ -597,7 +637,7 @@ def train_step(sd, image, targets, target_lengths, mask, variant="v1", num_heads
     for k in names:
         leaves[k] = sd[k].detach().clone().requires_grad_(True)
         work[k] = leaves[k]
-    logits = forward(work, image, mask=mask, training=True, num_heads=num_heads, variant=variant)
+    logits = forward(work, image, mask=mask, training=True, num_heads=num_heads, variant=variant, regs=regs)
     B, T = logits.shape[0], logits.shape[1]
     in_len = torch.full((B,), T, dtype=torch.int32)
     loss = ctc_loss_torch(logits, targets, in_len, target_lengths).mean()
@@ -606,3 +646,97 @@ def train_step(sd, image, targets, target_lengths, mask, variant="v1", num_heads
         if "running_" in k or k.endswith("num_batches_tracked"):
             sd[k] = work[k]
     return float(loss.detach()), {k: v.grad for k, v in leaves.items()}, logits.detach()
+
+
+# ----------------------------------------------------------------------------------------------
+# Train-mode regularisers of the windowed variant with the CUDA kernels' own masks.  The kernels draw dropout and
+# attention dropout from counter-based hashes (htr-vt_b200/csrc/norm.cu dropout_bf16_kernel, csrc/attention2.cu
+# attn_keep); the functions below restate that uint32 arithmetic exactly, so a reference can apply the very masks the
+# kernels applied and compare values instead of statistics.
+# ----------------------------------------------------------------------------------------------
+def _mix32(x):
+    """murmur3 finaliser on uint32 arrays (wrap-around arithmetic)."""
+    x = np.asarray(x, dtype=np.uint32)
+    with np.errstate(over="ignore"):
+        x = x ^ (x >> np.uint32(16))
+        x = x * np.uint32(0x85EBCA6B)
+        x = x ^ (x >> np.uint32(13))
+        x = x * np.uint32(0xC2B2AE35)
+    return x ^ (x >> np.uint32(16))
+
+
+def _u32(v):
+    return np.uint32(int(v) & 0xFFFFFFFF)
+
+
+def dropout_keep_scale(n, per_sample, p, seed, site, dp=None, offset=0):
+    """Per-element factor of htrvt_dropout_bf16(x, n, per_sample, p, seed, site, dp) for the flat elements
+    [offset, offset + n): 0 (dropped) or inv_keep * dp[element // per_sample] in float32, inv_keep = 1 / (1 - p).
+    Element e sits in 16-byte group i = e // 8, 32-bit word k = (e // 2) % 4 of it; the word's hash
+    r = mix32(key + uint32(i) * 4 + k) ^ (i >> 30), key = mix32(uint32(seed) ^ site * 0x9e3779b9) ^ (seed >> 32),
+    decides the even element with its low 16 bits and the odd one with its high 16 bits: dropped iff
+    (half << 8) < uint32(float32(p) * 2^24)."""
+    p32 = np.float32(p)
+    thr = np.uint32(int(p32 * np.float32(16777216.0)))
+    inv_keep = np.float32(1.0) / (np.float32(1.0) - p32)
+    key = _mix32(_u32(seed) ^ _u32(int(site) * 0x9E3779B9)) ^ _u32(int(seed) >> 32)
+    e = np.arange(offset, offset + n, dtype=np.int64)
+    w = e >> 1                                                   # 32-bit word index = 4 * i + k
+    with np.errstate(over="ignore"):
+        r = _mix32(key + (w & 0xFFFFFFFF).astype(np.uint32)) ^ ((w >> 2) >> 30).astype(np.uint32)
+    half = np.where((e & 1) == 0, r & np.uint32(0xFFFF), r >> np.uint32(16)).astype(np.uint32)
+    dropped = (half << np.uint32(8)) < thr
+    sc = np.full(n, inv_keep, dtype=np.float32)
+    if dp is not None:
+        dp = np.asarray(dp, dtype=np.float32)
+        sc = inv_keep * dp[e // int(per_sample)]
+    return np.where(dropped, np.float32(0.0), sc).astype(np.float32)
+
+
+def attention_keep(seed, bh, ti, tj, p):
+    """attn_keep of csrc/attention2.cu as a bool (True = kept) for broadcastable integer arrays bh (= b * H + h),
+    ti (query token), tj (key token): a = mix32(uint32(seed) ^ bh * 0x9e3779b9),
+    v = mix32(a ^ mix32((seed >> 32) + ti * 65537 + tj)), dropped iff float32(v >> 8) * 2^-24 < float32(p)."""
+    bh, ti, tj = (np.asarray(v, dtype=np.int64) for v in (bh, ti, tj))
+    with np.errstate(over="ignore"):
+        a = _mix32(_u32(seed) ^ ((bh & 0xFFFFFFFF).astype(np.uint32) * np.uint32(0x9E3779B9)))
+        c = _u32(int(seed) >> 32) + (ti & 0xFFFFFFFF).astype(np.uint32) * np.uint32(65537) + \
+            (tj & 0xFFFFFFFF).astype(np.uint32)
+    v = _mix32(a ^ _mix32(c))
+    u = (v >> np.uint32(8)).astype(np.float32) * np.float32(1.0 / 16777216.0)
+    return ~(u < np.float32(p))
+
+
+def window_blocks(depth):
+    """(window, shift) per block of the windowed variant: 16-token windows in block 0, shifted by 8 in block 1,
+    global attention in the rest (as forward above and the model's engine use them)."""
+    return [((16, 0) if i == 0 else ((16, 8) if i == 1 else (0, 0))) for i in range(depth)]
+
+
+def train_regs(seed, drop, attn_drop, drop_path, B, T, D, hidden, num_heads):
+    """The per-block `regs` of forward / train_step for one train-mode step of the windowed variant's engine
+    (htr-vt_b200/engine.py), from the draw the model made for it (model_window HTR_VT._train_rng: seed, rates, and
+    drop_path = [(dp1, dp2) per block], tensors [B] or None).  Block i uses attention seed seed + 16 i and dropout
+    sites 8 i + 1 (proj, DropPath dp1), 8 i + 2 (fc1 activation), 8 i + 3 (fc2, DropPath dp2) over the token-major
+    [B, T, features] tensors.  Entries: "attn" [B, H, Tp, Tp] keep-scale over token indices (Tp = T padded to the
+    window in windowed blocks), "proj" / "fc2" [B, T, D], "fc1" [B, T, hidden] (DropPath folded out: the dropout
+    factors alone), "dp1" / "dp2" [B] - each None where that regulariser is off."""
+    regs = []
+    for i, (window, shift) in enumerate(window_blocks(len(drop_path))):
+        blk = {"attn": None, "proj": None, "fc1": None, "fc2": None}
+        if attn_drop > 0:
+            Tp = -(-T // window) * window if window else T
+            bh = np.arange(B * num_heads).reshape(B, num_heads, 1, 1)
+            t = np.arange(Tp)
+            keep = attention_keep(seed + 16 * i, bh, t.reshape(1, 1, Tp, 1), t.reshape(1, 1, 1, Tp), attn_drop)
+            inv = np.float32(1.0) / (np.float32(1.0) - np.float32(attn_drop))
+            blk["attn"] = torch.from_numpy(np.where(keep, inv, np.float32(0.0)).astype(np.float32))
+        if drop > 0:
+            for name, site, width in (("proj", 8 * i + 1, D), ("fc1", 8 * i + 2, hidden), ("fc2", 8 * i + 3, D)):
+                blk[name] = torch.from_numpy(
+                    dropout_keep_scale(B * T * width, T * width, drop, seed, site).reshape(B, T, width))
+        dp1, dp2 = drop_path[i]
+        blk["dp1"] = None if dp1 is None else torch.as_tensor(dp1).detach().float().cpu()
+        blk["dp2"] = None if dp2 is None else torch.as_tensor(dp2).detach().float().cpu()
+        regs.append(blk)
+    return regs

@@ -307,12 +307,15 @@ def test_end_to_end_decode_strings():
 # ------------------------------------------------------------------------------------------------
 # windowed variant (model_window): relative-position bias, 16-token shifted windows, T up to 256
 # ------------------------------------------------------------------------------------------------
-def _build_window(nb_cls, W, D, depth, heads, seed):
+def _build_window(nb_cls, W, D, depth, heads, seed, table_size_from_w=False):
+    """table_size_from_w: size the bias table for exactly W / 4 tokens (img_size = [W, 64], the convention of
+    create_model), which a line whose token count is not a multiple of 16 needs to load init_state_dict's weights."""
     import htrvt_b200  # noqa: F401
     from functools import partial
     Wm = import_module("htr-vt_b200.model_window.HTR_VT")
-    m = Wm.MaskedAutoencoderViT(nb_cls, img_size=[64, W], patch_size=(4, 64), embed_dim=D, depth=depth,
-                                num_heads=heads, mlp_ratio=4, norm_layer=partial(torch.nn.LayerNorm, eps=1e-6))
+    m = Wm.MaskedAutoencoderViT(nb_cls, img_size=[W, 64] if table_size_from_w else [64, W], patch_size=(4, 64),
+                                embed_dim=D, depth=depth, num_heads=heads, mlp_ratio=4,
+                                norm_layer=partial(torch.nn.LayerNorm, eps=1e-6))
     sd = O.init_state_dict(nb_cls, [64, W], seed=seed, embed_dim=D, depth=depth, num_heads=heads, variant="window")
     m.load_state_dict(sd, strict=True)
     return m.cuda(), sd
@@ -374,25 +377,88 @@ def test_window_ragged_widths_match_reference_golden(tag):
     assert not bad, bad
 
 
-@pytest.mark.parametrize("cfg", [dict(nb_cls=20, W=512, D=256, depth=4, heads=2, B=3, seed=9),
-                                 dict(nb_cls=90, W=1024, D=768, depth=4, heads=6, B=2, seed=321)])
+def _capture_draws(m):
+    """Record every train-mode draw (seed, rates, DropPath scales) the model makes, by wrapping its _train_rng."""
+    draws = []
+    orig = m._train_rng
+
+    def capture(batch, device):
+        rng = orig(batch, device)
+        draws.append(rng)
+        return rng
+
+    m._train_rng = capture
+    return draws
+
+
+def _regs_of(draw, B, T, D, heads):
+    """Oracle regs (htrvt_oracle.train_regs) for the masks the engine applied in the step that made `draw`."""
+    if draw is None:
+        return None
+    return O.train_regs(draw["seed"], draw["drop"], draw["attn_drop"], draw["drop_path"], B, T, D, 4 * D, heads)
+
+
+@pytest.mark.parametrize("cfg", [
+    dict(nb_cls=20, W=512, D=256, depth=4, heads=2, B=3, seed=9),
+    dict(nb_cls=90, W=1024, D=768, depth=4, heads=6, B=2, seed=321),
+    # train-mode regularisers on (rates = drop, attn_drop, drop_path_rate), compared with the oracle applying the masks
+    # the kernels applied; depth 4 covers blocks 0 (window 16, shift 0), 1 (16, 8) and 2-3 (global)
+    pytest.param(dict(nb_cls=90, W=1024, D=768, depth=4, heads=6, B=2, seed=321, rates=(0.1, 0.05, 0.1)),
+                 id="defaults"),
+    pytest.param(dict(nb_cls=20, W=512, D=256, depth=4, heads=2, B=3, seed=9, rates=(0.1, 0.0, 0.0)),
+                 id="drop_only"),
+    pytest.param(dict(nb_cls=20, W=512, D=256, depth=4, heads=2, B=3, seed=9, rates=(0.0, 0.05, 0.0)),
+                 id="attn_drop_only"),
+    pytest.param(dict(nb_cls=20, W=512, D=256, depth=4, heads=2, B=4, seed=9, rates=(0.0, 0.0, 0.5)),
+                 id="drop_path_only"),
+    pytest.param(dict(nb_cls=40, W=1000, D=256, depth=4, heads=2, B=3, seed=19, rates=(0.1, 0.05, 0.1)),
+                 id="ragged_w1000_defaults"),
+])
 def test_window_train_step_matches_oracle(cfg):
-    """Train-mode forward/backward with the stochastic regularisers switched off (the reference draws them from the
-    device generator: only eval / p = 0 can be compared value by value, SURVEY.md 9.13)."""
+    """Train-mode forward/backward against the oracle.  With the regularisers off (the first two configs) the step is
+    deterministic.  With them on, the reference draws its masks from the device generator, so only the distribution
+    could match it (SURVEY.md 9.13); here the oracle applies the kernels' own masks (train_regs: the same seed, sites
+    and DropPath draw), which makes the comparison value by value again."""
     import htrvt_b200 as h
-    m, sd = _build_window(cfg["nb_cls"], cfg["W"], cfg["D"], cfg["depth"], cfg["heads"], cfg["seed"])
-    m.train().set_stochastic(0.0, 0.0, 0.0)
-    B, W = cfg["B"], cfg["W"]
+    rates = cfg.get("rates", (0.0, 0.0, 0.0))
+    B, W, D, heads = cfg["B"], cfg["W"], cfg["D"], cfg["heads"]
+    T = W // 4
+    m, sd = _build_window(cfg["nb_cls"], W, D, cfg["depth"], heads, cfg["seed"], table_size_from_w=T % 16 != 0)
+    m.train().set_stochastic(*rates)
+    draws = _capture_draws(m)
     x = _images(cfg["seed"] + 1, B, W)
     tg, tl = _labels(cfg["seed"] + 2, B, cfg["nb_cls"], 4, 40)
     torch.manual_seed(7)
     preds = m(x.cuda(), 0.4, 8, use_masking=True)
     loss = h.ctc_loss_from_logits(preds.float(), tg.cuda(), tl).mean()
     loss.backward()
+    assert len(draws) == 1
+    regs = _regs_of(draws[0], B, T, D, heads)
+    drop, attn_drop, dpr = rates
+    if regs is None:
+        assert rates == (0.0, 0.0, 0.0)
+    else:
+        # the draw exercises what the config targets
+        assert draws[0]["drop"] == drop and draws[0]["attn_drop"] == attn_drop
+        for blk in regs:
+            for name in ("proj", "fc1", "fc2"):
+                assert (blk[name] is not None) == (drop > 0)
+                if drop > 0:
+                    assert (blk[name] == 0).any() and (blk[name] > 1).any()
+            assert (blk["attn"] is not None) == (attn_drop > 0)
+            if attn_drop > 0:
+                assert (blk["attn"] == 0).any()
+        if dpr > 0:
+            dps = [d for blk in regs for d in (blk["dp1"], blk["dp2"]) if d is not None]
+            assert len(dps) == 2 * (cfg["depth"] - 1)
+            assert any((d == 0).any() for d in dps)                         # some sample loses a branch
+        if dpr >= 0.5:
+            assert any(not torch.equal(blk["dp1"], blk["dp2"]) for blk in regs if blk["dp1"] is not None)
     torch.manual_seed(7)
-    mask = O.draw_span_mask(W // 4, 0.4, 8)
+    mask = O.draw_span_mask(T, 0.4, 8)
     sd_ref = {k: v.clone() for k, v in sd.items()}
-    ref_loss, ref_grads, ref_logits = O.train_step(sd_ref, x, tg, tl, mask, variant="window", num_heads=cfg["heads"])
+    ref_loss, ref_grads, ref_logits = O.train_step(sd_ref, x, tg, tl, mask, variant="window", num_heads=heads,
+                                                   regs=regs)
     err = _relerr(preds.detach().cpu().numpy(), ref_logits.numpy())
     assert err < 2e-2, err
     assert abs(loss.item() - ref_loss) < 2e-2 * abs(ref_loss)
@@ -401,6 +467,10 @@ def test_window_train_step_matches_oracle(cfg):
         assert p.grad is not None, name
         a = p.grad.detach().float().cpu().double().reshape(-1)
         b = ref_grads[name].double().reshape(-1)
+        if float(b.norm()) == 0.0:           # a branch DropPath removed for every sample: no gradient at all
+            if float(a.abs().max()) != 0.0:
+                bad.append((name, "want 0", float(a.abs().max())))
+            continue
         cos = float((a @ b) / (a.norm() * b.norm() + 1e-30))
         ratio = float(a.norm() / (b.norm() + 1e-30))
         # tiny batches (B = 2 / 3): batch statistics amplify bf16 noise in the stem, so the stem bound is looser here;
@@ -409,6 +479,35 @@ def test_window_train_step_matches_oracle(cfg):
         if not (cos > lo_cos and abs(ratio - 1.0) < tol):
             bad.append((name, round(cos, 4), round(ratio, 4)))
     assert not bad, bad
+
+
+def test_window_drop_path_rate_one_removes_the_last_block():
+    """set_stochastic(drop_path_rate=1.0): the last block's DropPath keeps no sample.  Its scales are 0 (as timm's
+    DropPath, which skips the division by keep = 0), so the logits stay finite, the block's parameters get exactly
+    zero gradient, and the step matches the oracle with the captured DropPath draw."""
+    import htrvt_b200 as h
+    nb_cls, W, D, heads, B = 20, 512, 256, 2, 3
+    m, sd = _build_window(nb_cls, W, D, 4, heads, 9)
+    m.train().set_stochastic(0.0, 0.0, 1.0)
+    draws = _capture_draws(m)
+    x = _images(10, B, W)
+    tg, tl = _labels(11, B, nb_cls, 4, 40)
+    torch.manual_seed(7)
+    preds = m(x.cuda(), 0.4, 8, use_masking=True)
+    assert torch.isfinite(preds).all()
+    h.ctc_loss_from_logits(preds.float(), tg.cuda(), tl).mean().backward()
+    dp1, dp2 = draws[0]["drop_path"][-1]
+    assert not dp1.any() and not dp2.any()
+    for name, p in m.named_parameters():
+        if name.startswith("blocks.3."):
+            assert not p.grad.any(), name
+    assert m.head.weight.grad.abs().max() > 0 and m.blocks[0].mlp.fc1.weight.grad.abs().max() > 0
+    torch.manual_seed(7)
+    mask = O.draw_span_mask(W // 4, 0.4, 8)
+    regs = _regs_of(draws[0], B, W // 4, D, heads)
+    _, _, ref_logits = O.train_step({k: v.clone() for k, v in sd.items()}, x, tg, tl, mask, variant="window",
+                                    num_heads=heads, regs=regs)
+    assert _relerr(preds.detach().cpu().numpy(), ref_logits.numpy()) < 2e-2
 
 
 def test_window_train_mode_is_stochastic_and_seeded():
