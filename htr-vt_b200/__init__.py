@@ -13,10 +13,13 @@ from . import _lib  # noqa: F401
 from .ctc import CTCLoss, ctc_loss_from_logits, greedy_decode  # noqa: F401
 from .converter import CTCLabelConverter  # noqa: F401
 from .metrics import ErrorRateMeter, cer_from_ids, edit_distances, format_string_for_wer  # noqa: F401
-from .beam import beam_search_with_lm_batch, kbest_candidates, simple_ctc_beam_search_with_lm  # noqa: F401
+from .beam import (beam_search_with_lm_batch, ctc_lm_decode, kbest_candidates,  # noqa: F401
+                   simple_ctc_beam_search_with_lm)
+from .lm import CharNGramLM  # noqa: F401
 from .prefetch import HostPrefetcher, RunningLoss  # noqa: F401
 from .augment import SameTrCollate, augment_lines, draw_collate_params  # noqa: F401
 
 __all__ = ["CTCLoss", "ctc_loss_from_logits", "greedy_decode", "CTCLabelConverter", "ErrorRateMeter", "cer_from_ids",
            "edit_distances", "format_string_for_wer", "simple_ctc_beam_search_with_lm", "beam_search_with_lm_batch",
-           "kbest_candidates", "HostPrefetcher", "RunningLoss", "SameTrCollate", "augment_lines", "draw_collate_params"]
+           "kbest_candidates", "ctc_lm_decode", "CharNGramLM", "HostPrefetcher", "RunningLoss", "SameTrCollate",
+           "augment_lines", "draw_collate_params"]

@@ -11,6 +11,11 @@ the reference; any object with a `.score(str) -> float` method).
 (csrc/prefix_beam.cu, SURVEY.md 8(f) row 4): the K candidates are the K most probable LABELLINGS, each scored with the
 summed probability of all its alignments, instead of the K best single alignment paths (which usually collapse to two
 or three distinct strings).  The default `search="paths"` is the reference's behaviour, bit for bit.
+
+`kbest_candidates(..., search="prefix", lm=CharNGramLM, alpha=, beta=)` and `ctc_lm_decode` put a character n-gram LM
+inside the prefix search (lm.py, csrc/prefix_beam.cu): every extension is ranked by CTC log-prob + alpha * ln(10) *
+log10 p(char | context) + beta, and the line's end adds the </s> term, so the LM shapes which labellings survive
+instead of only picking among the K the acoustic model kept.
 """
 import numpy as np
 import torch
@@ -39,14 +44,24 @@ def _candidate_strings(ids, lens, converter, merge_repeats=True):
     return ["".join(table[i] for i in kept[e - c:e]) for c, e in zip(counts.tolist(), ends.tolist())]
 
 
-def kbest_candidates(log_probs, converter, beam_size=5, lengths=None, layout="tbc", search="paths"):
+def kbest_candidates(log_probs, converter, beam_size=5, lengths=None, layout="tbc", search="paths", lm=None,
+                     alpha=None, beta=0.0):
     """-> per line: list of (string, score) for the surviving beams with a non-empty string, in the reference's
     order (test_with_kenlm.py:42-53).  search: "paths" (the reference's per-frame path beam; score = path log-prob)
-    or "prefix" (CTC prefix beam search; score = log-probability of the labelling)."""
+    or "prefix" (CTC prefix beam search; score = log-probability of the labelling).  lm (a CharNGramLM, prefix search
+    only) with weight alpha and per-character bonus beta: the candidates come from the LM-fused search, in its order,
+    and score = CTC log-prob + alpha * ln(10) * log10 P(string </s>) + beta * len."""
     if search not in ("paths", "prefix"):
         raise ValueError("search must be 'paths' or 'prefix'")
-    fn = ops.ctc_kbest_paths if search == "paths" else ops.ctc_prefix_beam
-    ids, lens, scores = fn(log_probs, beam_size, lengths, layout)
+    if lm is not None:
+        if search != "prefix":
+            raise ValueError("lm= needs search='prefix' (the path beam has no LM term)")
+        if alpha is None:
+            raise ValueError("lm= needs its weight alpha")
+        ids, lens, scores, _ = ops.ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta, lengths, layout)
+    else:
+        fn = ops.ctc_kbest_paths if search == "paths" else ops.ctc_prefix_beam
+        ids, lens, scores = fn(log_probs, beam_size, lengths, layout)
     ids, lens, scores = ids.cpu().numpy(), lens.cpu().numpy(), scores.cpu().numpy()
     B, K, T = ids.shape
     strings = _candidate_strings(ids.reshape(B * K, T), np.maximum(lens.reshape(-1), 0), converter,
@@ -79,3 +94,17 @@ def beam_search_with_lm_batch(preds_log, converter, lm_scorer, beam_size=5, leng
     if lp.stride(-1) != 1:
         lp = lp.contiguous()
     return [_pick(c, lm_scorer) for c in kbest_candidates(lp, converter, beam_size, lengths, search=search)]
+
+
+def ctc_lm_decode(preds_log, converter, lm, alpha, beta=0.0, beam_size=8, lengths=None):
+    """preds_log [T, B, C] (validation_with_kenlm's layout) -> B strings: the best-ranked labelling of the LM-fused CTC
+    prefix beam search per line ("" when that is the empty labelling).  lm: CharNGramLM on the same device."""
+    if not preds_log.is_cuda:
+        raise ops.HtrvtError("ctc_lm_decode needs a CUDA tensor (no CPU fallback)")
+    lp = preds_log.float()
+    if lp.stride(-1) != 1:
+        lp = lp.contiguous()
+    ids, lens, _, _ = ops.ctc_prefix_beam_lm(lp, beam_size, lm, alpha, beta, lengths, "tbc")
+    best_ids = ids[:, 0].cpu().numpy()
+    best_lens = np.maximum(lens[:, 0].cpu().numpy(), 0)
+    return _candidate_strings(best_ids, best_lens, converter, merge_repeats=False)

@@ -20,6 +20,12 @@
 // float64 in log space.  Selection = K rounds of a warp arg-max over the nb * (C - 1) + nb candidates in the strict
 // total order (score desc, candidate number asc); a round looks for the best candidate that comes AFTER the previous
 // winner in that order, so nothing has to be marked as taken.
+//
+// The LM-fused instantiation (LM = true, htrvt_ctc_prefix_beam_lm) ranks by lae(pb', pnb') + lm' instead, where lm is
+// an entry's float64 sum of alpha * ln10 * log10 p(label | context) + beta over its labels (character n-gram, ARPA
+// backoff).  The LM term of an extension depends only on (entry, label), so it is computed once, when the entry is
+// created: the 32 lanes fill the entry's row of lm + term(c) for every class (and its </s> term) in a per-warp row pool
+// of 2K rows; an entry that stays keeps its row.  The CTC masses (pb, pnb) are exactly those of the plain search.
 #include "common.cuh"
 #include <climits>
 
@@ -27,6 +33,37 @@ namespace htrvt {
 
 constexpr int kPbMaxK = 16;         // beam entries
 constexpr int kPbCpl = 8;           // classes per lane held in registers: C <= 256
+constexpr int kLmMaxOrder = 8;      // n-gram order: contexts of up to 7 tokens, keys of up to 8 16-bit fields
+constexpr double kLn10 = 2.302585092994046;
+constexpr int kLmUnk = 0, kLmBos = 1, kLmEos = 2;   // token ids of <unk>, <s>, </s>
+
+// One slot of the LM's open-addressing table (32 bytes, one sector).  Key = the n-gram's tokens, LAST token first, as
+// 16-bit fields (token + 1; 0 = no token) in lo (fields 0-3) and hi (fields 4-7); lo == 0 marks an empty slot.  Keys
+// are compared in full, so a hash collision never matches.  Linear probing from lm_hash(lo, hi) & (slots - 1).
+struct PbLmSlot {
+  unsigned long long lo, hi;
+  float p, b;                        // log10 probability, log10 backoff
+  unsigned long long pad;
+};
+struct PbLmArgs {
+  const PbLmSlot* table;
+  unsigned long long mask;           // slots - 1
+  int order;
+  const int* tok_map;                // class id -> token id (ids >= n_map: <unk>)
+  int n_map;
+  double alpha, beta;
+  double* ctc_scores;
+};
+struct PbLmWarp {                   // LM state of one line; per pool row (2K rows), except row[] / skey[]
+  double lm[2 * kPbMaxK];                                   // the row's entry: sum of its labels' LM terms
+  double eos[2 * kPbMaxK];                                  // alpha ln10 log10 p(</s> | context)
+  double skey[kPbMaxK];                                     // ranking key of every entry's stay candidate
+  unsigned long long clo[2 * kPbMaxK], chi[2 * kPbMaxK];    // context, most recent token first, key-field layout
+  int clen[2 * kPbMaxK];
+  int row[2][kPbMaxK];                                      // pool row of entry j of generation g
+  int nrow[kPbMaxK];                                        // rows created this frame
+  float bow[kPbMaxK][kLmMaxOrder];                          // log10 bow of their contexts' suffixes (0: unlisted)
+};
 
 struct PbGen {                      // one beam generation of one line
   double pb[kPbMaxK], pnb[kPbMaxK], tot[kPbMaxK];
@@ -65,17 +102,138 @@ __device__ __forceinline__ bool pb_before(long long k, int n, long long bk, int 
   return k > bk || (k == bk && n < bn);
 }
 
-template <int CPL>                  // class slots per lane: C <= 32 * CPL
+// ---- character n-gram LM ------------------------------------------------------------------------------------------
+// (mirrored bit for bit by htr-vt_b200/lm.py::lm_hash, which packs the table)
+__device__ __forceinline__ unsigned long long lm_hash(unsigned long long lo, unsigned long long hi) {
+  unsigned long long h = lo * 0x9e3779b97f4a7c15ull + hi * 0xc2b2ae3d27d4eb4full;
+  h ^= h >> 31;
+  h *= 0xbf58476d1ce4e5b9ull;
+  return h ^ (h >> 29);
+}
+__device__ __forceinline__ ulonglong2 lm_key_at(const PbLmSlot* t, unsigned long long i) {
+  return __ldg(reinterpret_cast<const ulonglong2*>(t + i));
+}
+__device__ __forceinline__ float2 lm_val_at(const PbLmSlot* t, unsigned long long i) {
+  return __ldg(reinterpret_cast<const float2*>(t + i) + 2);
+}
+// the rest of a probe whose first slot (i, s) is already loaded: the slot holding (lo, hi), or -1
+__device__ __forceinline__ long long lm_walk(const PbLmSlot* t, unsigned long long mask, unsigned long long lo,
+                                             unsigned long long hi, unsigned long long i, ulonglong2 s) {
+  for (unsigned long long n = 0; n <= mask; ++n) {
+    if (s.x == lo && s.y == hi) return static_cast<long long>(i);
+    if (s.x == 0ull) return -1;
+    i = (i + 1) & mask;
+    s = lm_key_at(t, i);
+  }
+  return -1;
+}
+// the first m fields of a context (key-field layout)
+__device__ __forceinline__ void lm_ctx_prefix(unsigned long long clo, unsigned long long chi, int m,
+                                              unsigned long long& lo, unsigned long long& hi) {
+  if (m >= 4) {
+    lo = clo;
+    hi = chi & ((1ull << (16 * (m - 4))) - 1ull);
+  } else {
+    lo = clo & ((1ull << (16 * m)) - 1ull);
+    hi = 0ull;
+  }
+}
+__device__ __forceinline__ int lm_tok(const PbLmArgs& a, int c) { return c < a.n_map ? __ldg(a.tok_map + c) : kLmUnk; }
+
+// Fill the rows L->nrow[0 .. nE) (their lm / context already set): row[c] = lm + alpha ln10 S(c) + beta for every label
+// c, eos = alpha ln10 S(</s>), with S(w) = log10 p(w | context) by ARPA backoff: the listed prob of the longest
+// (context suffix, w), plus the bows of the longer context suffixes, summed in float64 longest-context bow first and the
+// found prob last (the unigram level falls back to <unk>'s prob).  All 32 lanes, (row, class) pairs spread over lanes;
+// a lane issues the first-slot loads of every level of its query before it looks at any of them.
+__device__ __forceinline__ void lm_fill_rows(const PbLmArgs& a, PbLmWarp* L, double* rows, int nE, int C, float unk,
+                                          int lane) {
+  const int M1 = a.order - 1;
+  for (int idx = lane; idx < nE * M1; idx += 32) {            // context bows: (row, suffix length k = 1 .. clen)
+    const int e = idx / M1, k = idx - e * M1 + 1;
+    const int r = L->nrow[e];
+    float bw = 0.f;
+    if (k <= L->clen[r]) {
+      unsigned long long lo, hi;
+      lm_ctx_prefix(L->clo[r], L->chi[r], k, lo, hi);
+      const unsigned long long i = lm_hash(lo, hi) & a.mask;
+      const long long f = lm_walk(a.table, a.mask, lo, hi, i, lm_key_at(a.table, i));
+      if (f >= 0) bw = lm_val_at(a.table, static_cast<unsigned long long>(f)).y;
+    }
+    L->bow[e][k - 1] = bw;
+  }
+  __syncwarp();
+  const int Cm = C - 1;
+  for (int idx = lane; idx < nE * C; idx += 32) {             // nE * (C - 1) labels, then nE </s> queries
+    int e, c, tok;
+    if (idx < nE * Cm) {
+      e = idx / Cm;
+      c = idx - e * Cm + 1;
+      tok = lm_tok(a, c);
+    } else {
+      e = idx - nE * Cm;
+      c = -1;
+      tok = kLmEos;
+    }
+    const int r = L->nrow[e];
+    const int M = L->clen[r];
+    const unsigned long long clo = L->clo[r], chi = L->chi[r];
+    unsigned long long klo[kLmMaxOrder], khi[kLmMaxOrder], ix[kLmMaxOrder];
+    ulonglong2 s[kLmMaxOrder];
+    float p[kLmMaxOrder];
+#pragma unroll
+    for (int m = 0; m < kLmMaxOrder; ++m) {                   // key of (last m context tokens, w): w first
+      if (m <= M) {
+        unsigned long long lo, hi;
+        lm_ctx_prefix(clo, chi, m, lo, hi);
+        klo[m] = (lo << 16) | static_cast<unsigned long long>(tok + 1);
+        khi[m] = (hi << 16) | (lo >> 48);
+        ix[m] = lm_hash(klo[m], khi[m]) & a.mask;
+        s[m] = lm_key_at(a.table, ix[m]);
+        p[m] = lm_val_at(a.table, ix[m]).x;
+      }
+    }
+    double S = 0.0;
+    bool found = false;
+#pragma unroll
+    for (int m = kLmMaxOrder - 1; m >= 0; --m) {
+      if (m <= M && !found) {
+        if (s[m].x == klo[m] && s[m].y == khi[m]) {
+          S += static_cast<double>(p[m]);
+          found = true;
+        } else {
+          const long long f = s[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, klo[m], khi[m], ix[m], s[m]);
+          if (f >= 0) {
+            S += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(f)).x);
+            found = true;
+          } else if (m > 0) {
+            S += static_cast<double>(L->bow[e][m - 1]);
+          }
+        }
+      }
+    }
+    if (!found) S += static_cast<double>(unk);
+    const double t = __dmul_rn(a.alpha, __dmul_rn(kLn10, S));   // no contraction: the oracle's arithmetic
+    if (c < 0) L->eos[r] = t;
+    else rows[r * C + c] = __dadd_rn(L->lm[r], __dadd_rn(t, a.beta));
+  }
+  __syncwarp();
+}
+
+template <int CPL, bool LM>         // class slots per lane: C <= 32 * CPL; LM: fused character n-gram LM
 __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __restrict__ x, long long sb, long long st,
                                                               const int* __restrict__ lengths, int B, int T, int C,
                                                               int K, int* __restrict__ ids, int* __restrict__ lens,
-                                                              double* __restrict__ scores) {
+                                                              double* __restrict__ scores, PbLmArgs la) {
   extern __shared__ __align__(16) uint8_t pb_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
   const int b = blockIdx.x * warps + warp;
   if (b >= B) return;
   PbWarp* W = reinterpret_cast<PbWarp*>(pb_smem) + warp;
-  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + sizeof(PbWarp) * warps) +
+  const size_t lm_bytes = LM ? sizeof(PbLmWarp) + sizeof(double) * 2 * K * C : 0;
+  PbLmWarp* L = reinterpret_cast<PbLmWarp*>(pb_smem + sizeof(PbWarp) * warps) + warp;
+  double* rows = reinterpret_cast<double*>(pb_smem + (sizeof(PbWarp) + sizeof(PbLmWarp)) * warps) +
+                 static_cast<size_t>(warp) * 2 * K * C;
+  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + (sizeof(PbWarp) + lm_bytes) * warps) +
                     static_cast<size_t>(warp) * (static_cast<size_t>(T) * K + 1);
   int Tb = lengths ? lengths[b] : T;
   Tb = min(max(Tb, 0), T);
@@ -88,6 +246,21 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
     g.hash[0] = 0x243f6a8885a308d3ull; g.phash[0] = 0ull;
     g.last[0] = -1; g.len[0] = 0; g.node[0] = 0;
     nodes[0] = 0u;
+  }
+  unsigned used = 1u;                 // LM: pool rows held by the current generation
+  float unk = -100.f;                 // LM: log10 p(<unk>) (-100 when the LM does not list it)
+  if constexpr (LM) {
+    const ulonglong2 s = lm_key_at(la.table, lm_hash(kLmUnk + 1, 0ull) & la.mask);
+    const long long f = lm_walk(la.table, la.mask, kLmUnk + 1, 0ull, lm_hash(kLmUnk + 1, 0ull) & la.mask, s);
+    if (f >= 0) unk = lm_val_at(la.table, static_cast<unsigned long long>(f)).x;
+    if (lane == 0) {                                     // the empty prefix: context <s>, row 0
+      L->row[0][0] = 0; L->nrow[0] = 0; L->lm[0] = 0.0;
+      L->clen[0] = min(1, la.order - 1);
+      L->clo[0] = la.order > 1 ? static_cast<unsigned long long>(kLmBos + 1) : 0ull;
+      L->chi[0] = 0ull;
+    }
+    __syncwarp();
+    lm_fill_rows(la, L, rows, 1, C, unk, lane);
   }
   float v[CPL], vn[CPL];
 #pragma unroll
@@ -135,6 +308,7 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
       W->spb[j] = npb;
       W->spnb[j] = npnb;
       W->stot[j] = lae(npb, npnb);
+      if constexpr (LM) L->skey[j] = W->stot[j] + L->lm[L->row[cur][j]];
     }
     __syncwarp();
     unsigned excl[CPL];                                   // bit i of excl[u]: extension (i, lane + 32 u) was folded
@@ -166,17 +340,20 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
       int bnu[CPL];
 #pragma unroll
       for (int u = 0; u < CPL; ++u) { bku[u] = LLONG_MIN; bnu[u] = 0x7fffffff; }
-      if (lane < nb) { bku[0] = pb_key(W->stot[lane]); bnu[0] = lane; }
+      if (lane < nb) { bku[0] = pb_key(LM ? L->skey[lane] : W->stot[lane]); bnu[0] = lane; }
 #pragma unroll 4
       for (int i = 0; i < nb; ++i) {
         const double ti = g.tot[i], pbi = g.pb[i];
         const int li = g.len[i] > 0 ? g.last[i] : -1;
         const int n0 = K + i * C;
+        const double* rw = LM ? rows + L->row[cur][i] * C : nullptr;
 #pragma unroll
         for (int u = 0; u < CPL; ++u) {
           const int c = lane + 32 * u;
           if (!((excl[u] >> i) & 1u)) {
-            const long long k = pb_key((c == li ? pbi : ti) + static_cast<double>(v[u]));
+            double s = (c == li ? pbi : ti) + static_cast<double>(v[u]);
+            if constexpr (LM) s = s + rw[c];
+            const long long k = pb_key(s);
             if (pb_before(k, n0 + c, bku[u], bnu[u])) { bku[u] = k; bnu[u] = n0 + c; }
           }
         }
@@ -214,7 +391,7 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
         bool ok;
         if (idx == M) {                                       // the owner's stay candidate
           ok = own < nb;
-          k = ok ? pb_key(W->stot[own]) : LLONG_MIN;
+          k = ok ? pb_key(LM ? L->skey[own] : W->stot[own]) : LLONG_MIN;
           n = own;
         } else {
           const int i = idx / CPL, u = idx - i * CPL;
@@ -225,7 +402,13 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
             if (q == u) ex = oex[q];
           ok = !((ex >> i) & 1u);                             // (invalid classes carry an all-ones mask)
           const int li = g.len[i] > 0 ? g.last[i] : -1;
-          k = ok ? pb_key((c == li ? g.pb[i] : g.tot[i]) + static_cast<double>(W->lp[c])) : LLONG_MIN;
+          if (ok) {
+            double s = (c == li ? g.pb[i] : g.tot[i]) + static_cast<double>(W->lp[c]);
+            if constexpr (LM) s = s + rows[L->row[cur][i] * C + c];
+            k = pb_key(s);
+          } else {
+            k = LLONG_MIN;
+          }
           n = K + i * C + c;
         }
         if (ok && pb_before(bk, bn, k, n) && pb_before(k, n, ck, cn)) { ck = k; cn = n; }
@@ -249,31 +432,81 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
       if (ext) { pi = (n - K) / C; c = (n - K) - pi * C; }
     }
     const unsigned em = __ballot_sync(0xffffffffu, ext);
+    int nr = 0;                                               // LM: the entry's pool row
     if (lane < nnew) {
+      // (win_s is the ranking key; with the LM it is not the CTC mass, which is then recomputed: + 0.0 folds -0.0
+      // onto +0.0 as the integer image of win_s does, so that alpha = beta = 0 reproduces the plain search bit for bit)
       if (!ext) {
-        gn.pb[lane] = W->spb[n]; gn.pnb[lane] = W->spnb[n]; gn.tot[lane] = W->win_s[lane];
+        gn.pb[lane] = W->spb[n]; gn.pnb[lane] = W->spnb[n]; gn.tot[lane] = LM ? W->stot[n] + 0.0 : W->win_s[lane];
         gn.hash[lane] = g.hash[n]; gn.phash[lane] = g.phash[n];
         gn.last[lane] = g.last[n]; gn.len[lane] = g.len[n]; gn.node[lane] = g.node[n];
+        if constexpr (LM) { nr = L->row[cur][n]; L->row[cur ^ 1][lane] = nr; }
       } else {
-        const int nd = nnodes + __popc(em & ((1u << lane) - 1u));
+        const int q = __popc(em & ((1u << lane) - 1u));
+        const int nd = nnodes + q;
         nodes[nd] = (static_cast<uint32_t>(g.node[pi]) << 16) | static_cast<uint32_t>(c);
-        gn.pb[lane] = -INFINITY; gn.pnb[lane] = W->win_s[lane]; gn.tot[lane] = W->win_s[lane];
+        double s = W->win_s[lane];
+        if constexpr (LM) {
+          const int li = g.len[pi] > 0 ? g.last[pi] : -1;
+          s = ((c == li ? g.pb[pi] : g.tot[pi]) + static_cast<double>(W->lp[c])) + 0.0;
+        }
+        gn.pb[lane] = -INFINITY; gn.pnb[lane] = s; gn.tot[lane] = s;
         gn.hash[lane] = pb_hash(g.hash[pi], c); gn.phash[lane] = g.hash[pi];
         gn.last[lane] = c; gn.len[lane] = g.len[pi] + 1; gn.node[lane] = nd;
+        if constexpr (LM) {                                   // a free row (not held by generation cur), q-th of them
+          unsigned fr = ~used & (K == 16 ? 0xffffffffu : (1u << (2 * K)) - 1u);
+          for (int z = 0; z < q; ++z) fr &= fr - 1u;
+          nr = __ffs(fr) - 1;
+          const int pr = L->row[cur][pi];
+          L->lm[nr] = rows[pr * C + c];
+          const int M = L->clen[pr];
+          const int M1 = la.order - 1;
+          unsigned long long lo = (L->clo[pr] << 16) | static_cast<unsigned long long>(lm_tok(la, c) + 1);
+          unsigned long long hi = (L->chi[pr] << 16) | (L->clo[pr] >> 48);
+          lm_ctx_prefix(lo, hi, M1, lo, hi);
+          L->clo[nr] = lo; L->chi[nr] = hi; L->clen[nr] = min(M + 1, M1);
+          L->nrow[q] = nr;
+          L->row[cur ^ 1][lane] = nr;
+        }
       }
     }
     nnodes += __popc(em);
     nb = nnew;
     cur ^= 1;
+    if constexpr (LM) {
+      used = __reduce_or_sync(0xffffffffu, lane < nnew ? 1u << nr : 0u);
+      if (em) {
+        __syncwarp();
+        lm_fill_rows(la, L, rows, __popc(em), C, unk, lane);
+      }
+    }
 #pragma unroll
     for (int u = 0; u < CPL; ++u) v[u] = vn[u];
     __syncwarp();
   }
 
   // ---- spell the surviving prefixes --------------------------------------------------------------------------
+  // LM: the key gains the </s> term and the survivors are re-ranked by it, stably (ties keep beam rank)
+  int slot = lane;
+  double fused = 0.0;
+  if constexpr (LM) {
+    const PbGen& g = W->gen[cur];
+    long long mk = LLONG_MIN;
+    if (lane < nb) {
+      const int r = L->row[cur][lane];
+      fused = (g.tot[lane] + L->lm[r]) + L->eos[r];
+      mk = pb_key(fused);
+    }
+    int rank = 0;
+    for (int j = 0; j < nb; ++j) {
+      const long long kj = __shfl_sync(0xffffffffu, mk, j);
+      if (kj > mk || (kj == mk && j < lane)) ++rank;
+    }
+    if (lane < nb) slot = rank;
+  }
   if (lane < K) {
     const PbGen& g = W->gen[cur];
-    int* out = ids + (static_cast<long long>(b) * K + lane) * T;
+    int* out = ids + (static_cast<long long>(b) * K + slot) * T;
     const bool live = lane < nb;
     int n = 0;
     if (live) {
@@ -286,9 +519,47 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
       }
     }
     for (int p = n; p < T; ++p) out[p] = 0;
-    lens[b * K + lane] = live ? n : -1;
-    scores[b * K + lane] = live ? g.tot[lane] : -INFINITY;
+    lens[b * K + slot] = live ? n : -1;
+    if constexpr (LM) {
+      scores[b * K + slot] = live ? fused : -INFINITY;
+      la.ctc_scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
+    } else {
+      scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
+    }
   }
+}
+
+// Shared launcher: shared memory = per warp the beam state, the LM state + row pool (LM only) and the node array;
+// fewer warps per CTA above 200 KB.
+template <bool LM>
+static int pb_launch(const float* log_probs, long long stride_b, long long stride_t, const int* lengths, int B, int T,
+                     int C, int K, int* ids, int* lens, double* scores, const PbLmArgs& la, cudaStream_t stream) {
+  if (B <= 0 || T <= 0 || C <= 0 || !log_probs || !ids || !lens || !scores) return HTRVT_ERR_SHAPE;
+  if (K < 1 || K > kPbMaxK || C > 32 * kPbCpl || static_cast<long long>(T) * K >= 65535) return HTRVT_ERR_SHAPE;
+  int warps = 4;
+  const size_t lm_bytes = LM ? sizeof(PbLmWarp) + sizeof(double) * 2 * K * C : 0;
+  auto need = [&](int w) {
+    return static_cast<size_t>(w) * (sizeof(PbWarp) + lm_bytes + (static_cast<size_t>(T) * K + 1) * 4);
+  };
+  while (warps > 1 && need(warps) > 200 * 1024) warps >>= 1;
+  const size_t smem = need(warps);
+  if (smem > 227 * 1024) return HTRVT_ERR_SHAPE;
+  const dim3 grid((B + warps - 1) / warps), block(warps * 32);
+#define PB_LAUNCH(CPL)                                                                                         \
+  do {                                                                                                         \
+    if (smem > 48 * 1024 && !HTRVT_ENSURE_SMEM((ctc_prefix_beam_kernel<CPL, LM>), 227 * 1024))                \
+      return HTRVT_ERR_LAUNCH;                                                                                 \
+    ctc_prefix_beam_kernel<CPL, LM><<<grid, block, smem, stream>>>(log_probs, stride_b, stride_t, lengths, B, T, \
+                                                                   C, K, ids, lens, scores, la);               \
+  } while (0)
+  if (C <= 32) PB_LAUNCH(1);
+  else if (C <= 64) PB_LAUNCH(2);
+  else if (C <= 96) PB_LAUNCH(3);
+  else if (C <= 128) PB_LAUNCH(4);
+  else PB_LAUNCH(8);
+#undef PB_LAUNCH
+  HTRVT_LAUNCH_CHECK();
+  return HTRVT_OK;
 }
 
 }  // namespace htrvt
@@ -301,26 +572,30 @@ using namespace htrvt;
 extern "C" int htrvt_ctc_prefix_beam(const float* log_probs, long long stride_b, long long stride_t,
                                      const int* lengths, int B, int T, int C, int K, int* ids, int* lens,
                                      double* scores, cudaStream_t stream) {
-  if (B <= 0 || T <= 0 || C <= 0 || !log_probs || !ids || !lens || !scores) return HTRVT_ERR_SHAPE;
-  if (K < 1 || K > kPbMaxK || C > 32 * kPbCpl || static_cast<long long>(T) * K >= 65535) return HTRVT_ERR_SHAPE;
-  int warps = 4;
-  auto need = [&](int w) { return static_cast<size_t>(w) * (sizeof(PbWarp) + (static_cast<size_t>(T) * K + 1) * 4); };
-  while (warps > 1 && need(warps) > 200 * 1024) warps >>= 1;
-  const size_t smem = need(warps);
-  if (smem > 227 * 1024) return HTRVT_ERR_SHAPE;
-  const dim3 grid((B + warps - 1) / warps), block(warps * 32);
-#define PB_LAUNCH(CPL)                                                                                         \
-  do {                                                                                                         \
-    if (smem > 48 * 1024 && !HTRVT_ENSURE_SMEM(ctc_prefix_beam_kernel<CPL>, 227 * 1024)) return HTRVT_ERR_LAUNCH; \
-    ctc_prefix_beam_kernel<CPL><<<grid, block, smem, stream>>>(log_probs, stride_b, stride_t, lengths, B, T, C, K, \
-                                                               ids, lens, scores);                             \
-  } while (0)
-  if (C <= 32) PB_LAUNCH(1);
-  else if (C <= 64) PB_LAUNCH(2);
-  else if (C <= 96) PB_LAUNCH(3);
-  else if (C <= 128) PB_LAUNCH(4);
-  else PB_LAUNCH(8);
-#undef PB_LAUNCH
-  HTRVT_LAUNCH_CHECK();
-  return HTRVT_OK;
+  return pb_launch<false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, PbLmArgs{}, stream);
+}
+
+// The same search with a character n-gram LM fused into the ranking (header: include/htrvt.h).  lm_table: lm_slots
+// (a power of two) PbLmSlot records with at least one empty slot; token ids <unk> = 0, <s> = 1, </s> = 2; tok_map:
+// class id -> token id for ids < n_tok_map, <unk> beyond.  scores = fused score with the </s> term, ctc_scores =
+// log P(labelling's alignments), both float64 [B, K], entries in fused order.
+extern "C" int htrvt_ctc_prefix_beam_lm(const float* log_probs, long long stride_b, long long stride_t,
+                                        const int* lengths, int B, int T, int C, int K, const void* lm_table,
+                                        long long lm_slots, int lm_order, const int* tok_map, int n_tok_map,
+                                        double alpha, double beta, int* ids, int* lens, double* scores,
+                                        double* ctc_scores, cudaStream_t stream) {
+  if (!lm_table || !ctc_scores || lm_slots < 2 || (lm_slots & (lm_slots - 1)) != 0) return HTRVT_ERR_SHAPE;
+  if (lm_order < 1 || lm_order > kLmMaxOrder || n_tok_map < 0 || (n_tok_map > 0 && !tok_map)) return HTRVT_ERR_SHAPE;
+  if (!isfinite(alpha) || !isfinite(beta)) return HTRVT_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(lm_table) & 31) != 0) return HTRVT_ERR_ALIGN;
+  PbLmArgs la;
+  la.table = static_cast<const PbLmSlot*>(lm_table);
+  la.mask = static_cast<unsigned long long>(lm_slots - 1);
+  la.order = lm_order;
+  la.tok_map = tok_map;
+  la.n_map = n_tok_map;
+  la.alpha = alpha;
+  la.beta = beta;
+  la.ctc_scores = ctc_scores;
+  return pb_launch<true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, stream);
 }

@@ -393,6 +393,36 @@ def ctc_prefix_beam(log_probs, beam_size, lengths=None, layout="tbc"):
     return ids, lens, scores
 
 
+def ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta=0.0, lengths=None, layout="tbc"):
+    """ctc_prefix_beam with a character n-gram LM (lm.py::CharNGramLM) fused into the search: candidates rank by
+    CTC log-prob + sum of (alpha * ln10 * log10 p(label | context) + beta), survivors by that plus the </s> term.
+    Returns (ids [B,K,T] int32, lens [B,K] int32, scores [B,K] float64 (fused), ctc_scores [B,K] float64), in fused
+    order.  alpha = beta = 0 reproduces ctc_prefix_beam's ids, lens and scores bit for bit."""
+    _need_cuda(log_probs)
+    if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
+        raise HtrvtError("ctc_prefix_beam_lm expects fp32 log-probs with a contiguous class axis")
+    if lm.table.device != log_probs.device:
+        raise HtrvtError("ctc_prefix_beam_lm: the LM table lives on %s, the log-probs on %s"
+                         % (lm.table.device, log_probs.device))
+    if layout == "btc":
+        B, T, C = log_probs.shape
+        sb, st = log_probs.stride(0), log_probs.stride(1)
+    else:
+        T, B, C = log_probs.shape
+        sb, st = log_probs.stride(1), log_probs.stride(0)
+    dev = log_probs.device
+    K = int(beam_size)
+    ids = torch.empty((B, K, T), dtype=torch.int32, device=dev)
+    lens = torch.empty((B, K), dtype=torch.int32, device=dev)
+    scores = torch.empty((B, K), dtype=torch.float64, device=dev)
+    ctc_scores = torch.empty((B, K), dtype=torch.float64, device=dev)
+    ln = None if lengths is None else lengths.to(device=dev, dtype=torch.int32).contiguous()
+    check(lib().htrvt_ctc_prefix_beam_lm(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(lm.table), lm.slots, lm.order,
+                                         _p(lm.token_map), lm.token_map.numel(), float(alpha), float(beta), _p(ids),
+                                         _p(lens), _p(scores), _p(ctc_scores), _stream()), "htrvt_ctc_prefix_beam_lm")
+    return ids, lens, scores, ctc_scores
+
+
 def augment_lines(img_u8, records, morph):
     """SameTrCollate's pixel work on a uint8 batch (csrc/augment.cu; model_v1/data/dataset.py:13-45).
     img_u8: CUDA uint8 [B, H, W] with contiguous rows; records: uint8 [B, 128] (CPU or CUDA; augment.py::pack_params);
@@ -997,7 +1027,7 @@ def _instrument():
     import functools
     g = globals()
     names = ["gemm_tn", "gemm_nn", "linear_wgrad", "conv_fwd", "conv_dgrad", "conv_dgrad_bn", "conv_wgrad", "conv_wgrad_acc", "conv_wgrad_acc_t", "conv_wgrad_acc_w", "unpack_conv_grads", "attention_fwd",
-             "attention_bwd", "attention2_fwd", "attention2_bwd", "attention_f32", "attention2_f32", "split3", "conv_fwd_split", "bn_act_f32", "maxpool_f32", "tokens_f32", "row_ln_f32", "gelu_split", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
+             "attention_bwd", "attention2_fwd", "attention2_bwd", "attention_f32", "attention2_f32", "split3", "conv_fwd_split", "bn_act_f32", "maxpool_f32", "tokens_f32", "row_ln_f32", "gelu_split", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "ctc_prefix_beam_lm", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
              "row_ln_fwd", "row_ln_bwd", "tokens_fwd", "tokens_bwd", "gelu_fwd", "gelu_bwd", "colsum_bf16", "cast_bf16", "cast_colsum_bf16", "dropout_",
              "pack_conv_weight", "pack_weights", "conv1_fwd", "bn_finalize", "bn_act_fwd", "pool_fwd", "pool_bwd", "bn_bwd", "bn_bwd_apply",
              "conv1_wgrad", "stem_head_moments", "stem_head_fwd", "stem_head_bwd"]

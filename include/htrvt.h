@@ -85,6 +85,30 @@ int htrvt_ctc_kbest_paths(const float* log_probs, long long stride_b, long long 
 int htrvt_ctc_prefix_beam(const float* log_probs, long long stride_b, long long stride_t, const int* lengths, int B,
                           int T, int C, int K, int* ids, int* lens, double* scores, void* stream);
 
+/* ---- CTC prefix beam search with a fused character n-gram LM ----------------------------------------------------
+ * htrvt_ctc_prefix_beam_lm is htrvt_ctc_prefix_beam with the language-model term inside the search (Hannun et al.
+ * 2014, "First-Pass Large Vocabulary Continuous Speech Recognition using Bi-Directional Recurrent DNNs", algorithm 1),
+ * extending the LM evaluation of model_window/test_with_kenlm.py:25-59, where the LM only picks among K finished
+ * candidates.  Every beam entry keeps its CTC masses (pb, pnb) exactly as the plain search and a float64 lm = sum over
+ * its labels of alpha * ln10 * S + beta, S = log10 p(label | previous order-1 tokens, starting from <s>) by ARPA
+ * backoff: the listed prob of (context, w), else bow(context) (0 if unlisted) + log10 p(w | context minus its oldest
+ * token), with <unk>'s unigram prob when w has none; S is the float64 sum of the float32 table values, longest
+ * context's bow first, found prob last.  Candidates rank by lae(pb', pnb') + lm' (ties as in the plain search); an
+ * extension that spells an entry merges its CTC mass into it (lm unchanged).  At the end each survivor's key gains
+ * alpha * ln10 * log10 p(</s> | context) (KenLM's score(bos=True, eos=True)) and the survivors are re-ranked stably.
+ * alpha = beta = 0 gives the ids, lens and scores of htrvt_ctc_prefix_beam bit for bit.
+ * lm_table: lm_slots (a power of two) 32-byte slots {u64 lo, hi; float log10 p, log10 bow; u64 pad}, 32-byte aligned,
+ * open addressing with linear probing and at least one empty slot (the layout htr-vt_b200/lm.py packs); lm_order 1..8;
+ * token ids <unk> = 0, <s> = 1, </s> = 2; tok_map int32 [n_tok_map]: class id -> token id (ids beyond: <unk>).
+ * scores float64 [B, K] = the fused score with the </s> term, ctc_scores float64 [B, K] = lae(pb, pnb), entries in
+ * fused order; ids / lens as htrvt_ctc_prefix_beam.  HTRVT_ERR_SHAPE: non-finite alpha or beta, lm_order outside
+ * 1..8, a slot count that is not a power of two, or the limits of htrvt_ctc_prefix_beam (K <= 16, C <= 256,
+ * T * K < 65535). */
+int htrvt_ctc_prefix_beam_lm(const float* log_probs, long long stride_b, long long stride_t, const int* lengths, int B,
+                             int T, int C, int K, const void* lm_table, long long lm_slots, int lm_order,
+                             const int* tok_map, int n_tok_map, double alpha, double beta, int* ids, int* lens,
+                             double* scores, double* ctc_scores, void* stream);
+
 /* ---- training-time augmentation of a uint8 batch of line images (SURVEY.md 8(f) row 2) ----------------------
  * htrvt_augment_lines replaces the per-image PIL / OpenCV / scikit-image work of `SameTrCollate`
  * (model_v1/data/dataset.py:13-45): RandomTransform's projective warp + resize (model_v1/data/transform.py:164-230),
