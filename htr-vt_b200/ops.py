@@ -2,6 +2,7 @@
 
 PyTorch is used here for device memory and streams only; all arithmetic runs in csrc/*.cu.
 """
+import collections
 import ctypes
 
 import torch
@@ -421,6 +422,61 @@ def ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta=0.0, lengths=None, 
                                          _p(lm.token_map), lm.token_map.numel(), float(alpha), float(beta), _p(ids),
                                          _p(lens), _p(scores), _p(ctc_scores), _stream()), "htrvt_ctc_prefix_beam_lm")
     return ids, lens, scores, ctc_scores
+
+
+CtcAlignment = collections.namedtuple("CtcAlignment", "path frame_scores spans token_scores score status")
+
+
+def ctc_align(x, targets, target_lengths, input_lengths=None, layout="tbc", is_logprob=True):
+    """Best CTC alignment of known labels per line (csrc/ctc_align.cu, blank = 0).
+    x: fp32 log-probs (or raw logits with is_logprob=False) [T,B,C] ("tbc") or [B,T,C] ("btc"), class axis contiguous;
+    targets int32 concatenated [sum L] or padded [B, Lpad]; lengths [B].  Lengths and targets may live on the host; the
+    longest label is then the kernel's hint, else a device-side max is read back to size `spans`.
+    Returns CtcAlignment of device tensors: path int32 [B,T] (-1 beyond a line's frames), frame_scores fp32 [B,T],
+    spans int32 [B,Lmax,2] ([start, end) frames of each label), token_scores fp32 [B,Lmax], score float64 [B],
+    status int32 [B] (0 aligned, 1 infeasible, 2 invalid line data)."""
+    _need_cuda(x)
+    if x.dtype != torch.float32 or x.stride(-1) != 1:
+        raise HtrvtError("ctc_align expects fp32 input with a contiguous class axis")
+    if layout == "btc":
+        B, T, C = x.shape
+        sb, st = x.stride(0), x.stride(1)
+    elif layout == "tbc":
+        T, B, C = x.shape
+        sb, st = x.stride(1), x.stride(0)
+    else:
+        raise ValueError("layout must be 'tbc' or 'btc', got %r" % (layout,))
+    dev = x.device
+    if not torch.is_tensor(target_lengths):
+        target_lengths = torch.as_tensor(target_lengths, dtype=torch.int32)
+    if target_lengths.device.type == "cpu":
+        hint = max(int(target_lengths.max()), 0) if target_lengths.numel() else 0
+        lmax = hint
+    else:
+        hint = -1
+        lmax = max(int(target_lengths.max()), 0) if target_lengths.numel() else 0
+    tg = torch.as_tensor(targets).to(device=dev, dtype=torch.int32)
+    tgt_stride = 0
+    if tg.dim() == 2:
+        tg = tg.contiguous()
+        tgt_stride = tg.size(1)
+    else:
+        tg = tg.reshape(-1).contiguous()
+    tl = target_lengths.to(device=dev, dtype=torch.int32).contiguous()
+    il = None if input_lengths is None else torch.as_tensor(input_lengths).to(device=dev, dtype=torch.int32).contiguous()
+    path = torch.empty((B, T), dtype=torch.int32, device=dev)
+    frame_scores = torch.empty((B, T), dtype=torch.float32, device=dev)
+    spans = torch.empty((B, lmax, 2), dtype=torch.int32, device=dev)
+    token_scores = torch.empty((B, lmax), dtype=torch.float32, device=dev)
+    score = torch.empty(B, dtype=torch.float64, device=dev)
+    status = torch.empty(B, dtype=torch.int32, device=dev)
+    nbytes = lib().htrvt_ctc_align_workspace_bytes(B, T, hint)
+    ws = workspace(nbytes, dev) if nbytes else None
+    check(lib().htrvt_ctc_align(_p(x), sb, st, int(bool(is_logprob)), _p(tg) if tg.numel() else None, tgt_stride,
+                                _p(il), _p(tl), B, T, C, hint, _p(path), _p(frame_scores), _p(spans) if lmax else None,
+                                lmax, _p(token_scores) if lmax else None, _p(score), _p(status), _p(ws),
+                                ws.numel() if ws is not None else 0, _stream()), "htrvt_ctc_align")
+    return CtcAlignment(path, frame_scores, spans, token_scores, score, status)
 
 
 def augment_lines(img_u8, records, morph):
@@ -1027,7 +1083,7 @@ def _instrument():
     import functools
     g = globals()
     names = ["gemm_tn", "gemm_nn", "linear_wgrad", "conv_fwd", "conv_dgrad", "conv_dgrad_bn", "conv_wgrad", "conv_wgrad_acc", "conv_wgrad_acc_t", "conv_wgrad_acc_w", "unpack_conv_grads", "attention_fwd",
-             "attention_bwd", "attention2_fwd", "attention2_bwd", "attention_f32", "attention2_f32", "split3", "conv_fwd_split", "bn_act_f32", "maxpool_f32", "tokens_f32", "row_ln_f32", "gelu_split", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "ctc_prefix_beam_lm", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
+             "attention_bwd", "attention2_fwd", "attention2_bwd", "attention_f32", "attention2_f32", "split3", "conv_fwd_split", "bn_act_f32", "maxpool_f32", "tokens_f32", "row_ln_f32", "gelu_split", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "ctc_prefix_beam_lm", "ctc_align", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
              "row_ln_fwd", "row_ln_bwd", "tokens_fwd", "tokens_bwd", "gelu_fwd", "gelu_bwd", "colsum_bf16", "cast_bf16", "cast_colsum_bf16", "dropout_",
              "pack_conv_weight", "pack_weights", "conv1_fwd", "bn_finalize", "bn_act_fwd", "pool_fwd", "pool_bwd", "bn_bwd", "bn_bwd_apply",
              "conv1_wgrad", "stem_head_moments", "stem_head_fwd", "stem_head_bwd"]

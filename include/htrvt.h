@@ -109,6 +109,39 @@ int htrvt_ctc_prefix_beam_lm(const float* log_probs, long long stride_b, long lo
                              const int* tok_map, int n_tok_map, double alpha, double beta, int* ids, int* lens,
                              double* scores, double* ctc_scores, void* stream);
 
+/* ---- CTC forced alignment of a known transcription -----------------------------------------------------------
+ * htrvt_ctc_align: the single best path (Viterbi) through the CTC trellis of each line's labels, blank = 0, with the
+ * frames each label occupies: the alignment torchaudio.functional.forced_align computes one line at a time on the host.
+ * States S = 2L + 1, ext[2k] = 0, ext[2k+1] = label[k]; d_0(0) = lp(0, 0), d_0(1) = lp(0, label[0]), others -inf;
+ * d_t(s) = max(c0, c1, c2) + lp(t, ext[s]) over c0 = d_{t-1}(s), c1 = d_{t-1}(s-1), c2 = d_{t-1}(s-2) (only when
+ * ext[s] != 0 and ext[s] != ext[s-2]); on a tie the FIRST of c0, c1, c2 wins (stay, previous, skip).  d is float64:
+ * each fp32 input is widened, one float64 add per state per frame after the max.  The path ends in S-1 if
+ * d(S-1) > d(S-2), else in S-2 (a tie ends on the last label); L = 0 gives an all-blank path.
+ * x: fp32 log-probs, or raw logits with is_logprob = 0 (the path is the same; the scores below subtract each frame's
+ * float64 log-sum-exp over the full row), class axis contiguous, element strides for the batch and time axes.
+ * targets / tgt_stride / input_lengths / target_lengths as htrvt_ctc_loss_grad (concatenated: line b's labels start at
+ * the sum of the earlier lines' lengths, negative ones counted as 0; input_lengths NULL = T for every line).
+ * Outputs for line b with T_b frames:
+ *   path int32 [B, T]: the class of every frame t < T_b, -1 beyond;  frame_scores fp32 [B, T]: log-prob of that class at
+ *   that frame, 0 beyond;  spans int32 [B, span_stride, 2]: [start, end) frames of label k (the frames spent in state
+ *   2k+1), -1 for k >= L;  token_scores fp32 [B, span_stride]: float64 sum of the span's frame scores in frame order,
+ *   0 for k >= L;  score float64 [B]: the Viterbi log-prob;  status int32 [B]:
+ *     0 aligned (T_b = 0 with L = 0: score 0);
+ *     1 infeasible, T_b < L + number of adjacent equal labels: score -inf, path and spans -1;
+ *     2 invalid line data: a label outside [1, C), a negative length, T_b > T, L > 256, L > max_target_len (when given)
+ *       or L > span_stride, or L > 0 with targets NULL: score -inf, path and spans -1.  Nothing outside the line is read.
+ * max_target_len: host-side hint (longest label) or -1 = unknown (worst case, 256); it picks the states per lane and
+ * the workspace.  Limits: L <= 256, T <= 2^20.  workspace: htrvt_ctc_align_workspace_bytes(B, T, max_target_len) bytes,
+ * 16-byte aligned (back-pointers, B * T * 128 bytes, twice that for a hint above 255 or -1).  spans / token_scores may be
+ * NULL when span_stride = 0.  HTRVT_ERR_SHAPE: B <= 0, T <= 0 or above the limit, C < 2, negative strides,
+ * max_target_len > 256, a missing output; HTRVT_ERR_WORKSPACE; HTRVT_ERR_ALIGN.  Deterministic, no atomics. */
+size_t htrvt_ctc_align_workspace_bytes(int B, int T, int max_target_len);
+int htrvt_ctc_align(const float* x, long long stride_b, long long stride_t, int is_logprob, const int* targets,
+                    int tgt_stride, const int* input_lengths, const int* target_lengths, int B, int T, int C,
+                    int max_target_len, int* path, float* frame_scores, int* spans, int span_stride,
+                    float* token_scores, double* score, int* status, void* workspace, size_t workspace_bytes,
+                    void* stream);
+
 /* ---- training-time augmentation of a uint8 batch of line images (SURVEY.md 8(f) row 2) ----------------------
  * htrvt_augment_lines replaces the per-image PIL / OpenCV / scikit-image work of `SameTrCollate`
  * (model_v1/data/dataset.py:13-45): RandomTransform's projective warp + resize (model_v1/data/transform.py:164-230),
