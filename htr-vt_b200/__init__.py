@@ -13,8 +13,9 @@ from . import _lib  # noqa: F401
 from .ctc import CTCLoss, ctc_loss_from_logits, greedy_decode  # noqa: F401
 from .converter import CTCLabelConverter  # noqa: F401
 from .metrics import ErrorRateMeter, cer_from_ids, edit_distances, format_string_for_wer  # noqa: F401
-from .beam import (beam_search_with_lm_batch, ctc_lm_decode, kbest_candidates,  # noqa: F401
+from .beam import (beam_search_with_lm_batch, ctc_lexicon_decode, ctc_lm_decode, kbest_candidates,  # noqa: F401
                    simple_ctc_beam_search_with_lm)
+from .lexicon import Lexicon  # noqa: F401
 from .lm import CharNGramLM  # noqa: F401
 from .prefetch import HostPrefetcher, RunningLoss  # noqa: F401
 from .augment import SameTrCollate, augment_lines, draw_collate_params  # noqa: F401
@@ -22,5 +23,6 @@ from .align import align_text, ctc_align, forced_align  # noqa: F401
 
 __all__ = ["CTCLoss", "ctc_loss_from_logits", "greedy_decode", "CTCLabelConverter", "ErrorRateMeter", "cer_from_ids",
            "edit_distances", "format_string_for_wer", "simple_ctc_beam_search_with_lm", "beam_search_with_lm_batch",
-           "kbest_candidates", "ctc_lm_decode", "CharNGramLM", "HostPrefetcher", "RunningLoss", "SameTrCollate",
+           "kbest_candidates", "ctc_lm_decode", "CharNGramLM", "ctc_lexicon_decode", "Lexicon", "HostPrefetcher",
+           "RunningLoss", "SameTrCollate",
            "augment_lines", "draw_collate_params", "ctc_align", "forced_align", "align_text"]

@@ -16,6 +16,9 @@ or three distinct strings).  The default `search="paths"` is the reference's beh
 inside the prefix search (lm.py, csrc/prefix_beam.cu): every extension is ranked by CTC log-prob + alpha * ln(10) *
 log10 p(char | context) + beta, and the line's end adds the </s> term, so the LM shapes which labellings survive
 instead of only picking among the K the acoustic model kept.
+
+`kbest_candidates(..., search="prefix", lexicon=Lexicon)` and `ctc_lexicon_decode` constrain that search to a word
+lexicon (lexicon.py, csrc/prefix_beam.cu): every word of a candidate comes from the list, with or without the LM.
 """
 import numpy as np
 import torch
@@ -45,15 +48,24 @@ def _candidate_strings(ids, lens, converter, merge_repeats=True):
 
 
 def kbest_candidates(log_probs, converter, beam_size=5, lengths=None, layout="tbc", search="paths", lm=None,
-                     alpha=None, beta=0.0):
+                     alpha=None, beta=0.0, lexicon=None):
     """-> per line: list of (string, score) for the surviving beams with a non-empty string, in the reference's
     order (test_with_kenlm.py:42-53).  search: "paths" (the reference's per-frame path beam; score = path log-prob)
     or "prefix" (CTC prefix beam search; score = log-probability of the labelling).  lm (a CharNGramLM, prefix search
     only) with weight alpha and per-character bonus beta: the candidates come from the LM-fused search, in its order,
-    and score = CTC log-prob + alpha * ln(10) * log10 P(string </s>) + beta * len."""
+    and score = CTC log-prob + alpha * ln(10) * log10 P(string </s>) + beta * len.  lexicon (a Lexicon, prefix search
+    only, with or without lm): only labellings whose every word is in the lexicon, ranked and scored as without it."""
     if search not in ("paths", "prefix"):
         raise ValueError("search must be 'paths' or 'prefix'")
-    if lm is not None:
+    if lexicon is not None:
+        if search != "prefix":
+            raise ValueError("lexicon= needs search='prefix' (the path beam has no lexicon constraint)")
+        if lm is not None and alpha is None:
+            raise ValueError("lm= needs its weight alpha")
+        if lm is None:
+            alpha, beta = 0.0, 0.0
+        ids, lens, scores, _ = ops.ctc_prefix_beam_lex(log_probs, beam_size, lexicon, lm, alpha, beta, lengths, layout)
+    elif lm is not None:
         if search != "prefix":
             raise ValueError("lm= needs search='prefix' (the path beam has no LM term)")
         if alpha is None:
@@ -105,6 +117,21 @@ def ctc_lm_decode(preds_log, converter, lm, alpha, beta=0.0, beam_size=8, length
     if lp.stride(-1) != 1:
         lp = lp.contiguous()
     ids, lens, _, _ = ops.ctc_prefix_beam_lm(lp, beam_size, lm, alpha, beta, lengths, "tbc")
+    best_ids = ids[:, 0].cpu().numpy()
+    best_lens = np.maximum(lens[:, 0].cpu().numpy(), 0)
+    return _candidate_strings(best_ids, best_lens, converter, merge_repeats=False)
+
+
+def ctc_lexicon_decode(preds_log, converter, lexicon, beam_size=8, lengths=None, lm=None, alpha=0.0, beta=0.0):
+    """preds_log [T, B, C] (validation_with_kenlm's layout) -> B strings: the best-ranked labelling per line of the CTC
+    prefix beam search constrained to lexicon (a Lexicon on the same device), with the character LM lm (weights alpha,
+    beta) fused in when given ("" for the empty labelling, and for a line with no accepted labelling)."""
+    if not preds_log.is_cuda:
+        raise ops.HtrvtError("ctc_lexicon_decode needs a CUDA tensor (no CPU fallback)")
+    lp = preds_log.float()
+    if lp.stride(-1) != 1:
+        lp = lp.contiguous()
+    ids, lens, _, _ = ops.ctc_prefix_beam_lex(lp, beam_size, lexicon, lm, alpha, beta, lengths, "tbc")
     best_ids = ids[:, 0].cpu().numpy()
     best_lens = np.maximum(lens[:, 0].cpu().numpy(), 0)
     return _candidate_strings(best_ids, best_lens, converter, merge_repeats=False)

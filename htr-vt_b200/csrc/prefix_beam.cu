@@ -26,6 +26,16 @@
 // backoff).  The LM term of an extension depends only on (entry, label), so it is computed once, when the entry is
 // created: the 32 lanes fill the entry's row of lm + term(c) for every class (and its </s> term) in a per-warp row pool
 // of 2K rows; an entry that stays keeps its row.  The CTC masses (pb, pnb) are exactly those of the plain search.
+//
+// The lexicon-constrained instantiation (LEX = true, htrvt_ctc_prefix_beam_lex; with or without the LM) only accepts
+// labellings whose every maximal run of word characters is a lexicon word (Scheidl et al. 2018, "Words" mode).  Each
+// entry carries a trie node (0: between words) that its prefix alone determines, so the merge test stays valid.  Its
+// pool row (the LM's bookkeeping, kept when LEX is on without the LM) holds two class bitmasks filled by the warp when
+// the entry is created: `allow` (the classes the state machine permits from that node) and `allow_last` (those whose
+// target state is between words or a word end).  The disallowed (entry, class) pairs are ORed into the fold mask
+// `excl`, so the selection rounds skip them; in the line's last frame `allow_last` is used and an entry left inside an
+// unfinished word cannot stay.  Ranking and scores are otherwise those of the plain / LM search: the lexicon only
+// removes candidates.
 #include "common.cuh"
 #include <climits>
 
@@ -63,6 +73,24 @@ struct PbLmWarp {                   // LM state of one line; per pool row (2K ro
   int row[2][kPbMaxK];                                      // pool row of entry j of generation g
   int nrow[kPbMaxK];                                        // rows created this frame
   float bow[kPbMaxK][kLmMaxOrder];                          // log10 bow of their contexts' suffixes (0: unlisted)
+};
+
+// Word lexicon as a trie in CSR form (htr-vt_b200/lexicon.py packs it): node 0 = root; the edges of node n are
+// first[n] .. first[n + 1] - 1, sorted by label; is_word: class id -> word character (ids >= n_map: free).
+struct PbLexArgs {
+  const int* first;
+  const int* label;
+  const int* child;
+  const unsigned char* word_end;
+  const unsigned char* is_word;
+  int n_map;
+};
+struct PbLexWarp {                  // lexicon state of one line; per pool row (2K rows), except freem[]
+  int node[2 * kPbMaxK];                                    // trie node of the row's entry (0: between words)
+  int fin[2 * kPbMaxK];                                     // node is 0 or ends a word
+  unsigned allow[2 * kPbMaxK][kPbCpl];                      // bit (c & 31) of word c >> 5: c may extend the entry
+  unsigned allow_last[2 * kPbMaxK][kPbCpl];                 // ... and leaves it between words or at a word end
+  unsigned freem[kPbCpl];                                   // the free classes 1 .. C - 1
 };
 
 struct PbGen {                      // one beam generation of one line
@@ -219,21 +247,78 @@ __device__ __forceinline__ void lm_fill_rows(const PbLmArgs& a, PbLmWarp* L, dou
   __syncwarp();
 }
 
-template <int CPL, bool LM>         // class slots per lane: C <= 32 * CPL; LM: fused character n-gram LM
-__global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __restrict__ x, long long sb, long long st,
+// ---- word lexicon ---------------------------------------------------------------------------------------------------
+__device__ __forceinline__ bool lex_free(const PbLexArgs& a, int c) { return c >= a.n_map || !__ldg(a.is_word + c); }
+
+// Fill the masks of rows L->nrow[0 .. nE) (their node / fin already set).  From a finished node (0 or a word end) every
+// free class leads back to state 0, which both masks accept; a child edge c leads to the child, which allow_last
+// accepts only when the child ends a word.  All 32 lanes: first the free-class part word by word, then the child edges.
+template <int CPL>
+__device__ __forceinline__ void lex_fill_rows(const PbLexArgs& a, const PbLmWarp* L, PbLexWarp* X, int nE, int C,
+                                              int lane) {
+  for (int idx = lane; idx < nE * CPL; idx += 32) {
+    const int e = idx / CPL, w = idx - e * CPL;
+    const int r = L->nrow[e];
+    const unsigned m = X->fin[r] ? X->freem[w] : 0u;
+    X->allow[r][w] = m;
+    X->allow_last[r][w] = m;
+  }
+  __syncwarp();
+  for (int e = 0; e < nE; ++e) {
+    const int r = L->nrow[e];
+    const int n = X->node[r];
+    const int j1 = __ldg(a.first + n + 1);
+    for (int j = __ldg(a.first + n) + lane; j < j1; j += 32) {
+      const int c = __ldg(a.label + j);
+      if (c < C) {
+        const unsigned bit = 1u << (c & 31);
+        atomicOr(&X->allow[r][c >> 5], bit);
+        if (__ldg(a.word_end + __ldg(a.child + j))) atomicOr(&X->allow_last[r][c >> 5], bit);
+      }
+    }
+  }
+  __syncwarp();
+}
+// the trie node an entry at node n moves to by the allowed class c: 0 for a free class, else child(n, c)
+__device__ __forceinline__ int lex_step(const PbLexArgs& a, int n, int c) {
+  if (lex_free(a, c)) return 0;
+  int lo = __ldg(a.first + n), hi = __ldg(a.first + n + 1) - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(a.label + mid) < c) lo = mid + 1;
+    else hi = mid;
+  }
+  return __ldg(a.child + lo);
+}
+
+__device__ __forceinline__ PbLexArgs pb_lex_args(const PbLexArgs& a) { return a; }
+// a warp's lexicon state: after `front` bytes per warp (its beam state, pool rows' state and LM row pool)
+__device__ __forceinline__ PbLexWarp* pb_lex_warp(uint8_t* smem, size_t front, int warps, int warp) {
+  return reinterpret_cast<PbLexWarp*>(smem + front * warps) + warp;
+}
+
+// class slots per lane: C <= 32 * CPL; LM: fused character n-gram LM; LEX: word lexicon constraint, whose PbLexArgs
+// come in the pack Lex.  With LEX off the pack is empty and every lexicon variable lives inside `if constexpr (LEX)`,
+// so that the plain and LM kernels keep their parameter list and compile to the same code as before the lexicon.
+// (Min. blocks 1 for LEX: without it ptxas caps some lexicon instantiations at 56-128 registers and spills.)
+template <int CPL, bool LM, bool LEX, typename... Lex>
+__global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const float* __restrict__ x, long long sb, long long st,
                                                               const int* __restrict__ lengths, int B, int T, int C,
                                                               int K, int* __restrict__ ids, int* __restrict__ lens,
-                                                              double* __restrict__ scores, PbLmArgs la) {
+                                                              double* __restrict__ scores, PbLmArgs la, Lex... lex) {
+  static_assert(sizeof...(Lex) == (LEX ? 1 : 0), "LEX takes one PbLexArgs");
   extern __shared__ __align__(16) uint8_t pb_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
   const int b = blockIdx.x * warps + warp;
   if (b >= B) return;
   PbWarp* W = reinterpret_cast<PbWarp*>(pb_smem) + warp;
-  const size_t lm_bytes = LM ? sizeof(PbLmWarp) + sizeof(double) * 2 * K * C : 0;
+  // per warp: PbWarp | PbLmWarp (LM or LEX: the pool rows' bookkeeping) + the LM row pool (LM) | PbLexWarp (LEX) | nodes
+  const size_t lm_bytes = (LM || LEX) ? sizeof(PbLmWarp) + (LM ? sizeof(double) * 2 * K * C : 0) : 0;
   PbLmWarp* L = reinterpret_cast<PbLmWarp*>(pb_smem + sizeof(PbWarp) * warps) + warp;
   double* rows = reinterpret_cast<double*>(pb_smem + (sizeof(PbWarp) + sizeof(PbLmWarp)) * warps) +
                  static_cast<size_t>(warp) * 2 * K * C;
-  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + (sizeof(PbWarp) + lm_bytes) * warps) +
+  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + (sizeof(PbWarp) + lm_bytes + (LEX ? sizeof(PbLexWarp) : 0)) *
+                                                           warps) +
                     static_cast<size_t>(warp) * (static_cast<size_t>(T) * K + 1);
   int Tb = lengths ? lengths[b] : T;
   Tb = min(max(Tb, 0), T);
@@ -247,7 +332,7 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
     g.last[0] = -1; g.len[0] = 0; g.node[0] = 0;
     nodes[0] = 0u;
   }
-  unsigned used = 1u;                 // LM: pool rows held by the current generation
+  unsigned used = 1u;                 // LM / LEX: pool rows held by the current generation
   float unk = -100.f;                 // LM: log10 p(<unk>) (-100 when the LM does not list it)
   if constexpr (LM) {
     const ulonglong2 s = lm_key_at(la.table, lm_hash(kLmUnk + 1, 0ull) & la.mask);
@@ -261,6 +346,22 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
     }
     __syncwarp();
     lm_fill_rows(la, L, rows, 1, C, unk, lane);
+  }
+  if constexpr (LEX) {
+    const PbLexArgs xa = pb_lex_args(lex...);
+    PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
+#pragma unroll
+    for (int u = 0; u < CPL; ++u) {
+      const int c = lane + 32 * u;
+      const unsigned fw = __ballot_sync(0xffffffffu, c >= 1 && c < C && lex_free(xa, c));
+      if (lane == 0) X->freem[u] = fw;
+    }
+    if (lane == 0) {                                     // the empty prefix: between words, row 0
+      L->row[0][0] = 0; L->nrow[0] = 0;
+      X->node[0] = 0; X->fin[0] = 1;
+    }
+    __syncwarp();
+    lex_fill_rows<CPL>(xa, L, X, 1, C, lane);
   }
   float v[CPL], vn[CPL];
 #pragma unroll
@@ -325,6 +426,17 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
           if (u == (mc >> 5)) excl[u] |= 1u << mi;
       }
     }
+    if constexpr (LEX) {                                  // the extensions the lexicon forbids join the folded ones
+      const PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
+      const bool last = t + 1 == Tb;
+      for (int i = 0; i < nb; ++i) {
+        const int r = L->row[cur][i];
+        const unsigned* m = last ? X->allow_last[r] : X->allow[r];
+#pragma unroll
+        for (int u = 0; u < CPL; ++u)
+          if (!((m[u] >> lane) & 1u)) excl[u] |= 1u << i;
+      }
+    }
 
     // ---- K selection rounds ---------------------------------------------------------------------------------
     // Scores are compared as order-preserving 64-bit integer images of the doubles; the sentinel (LLONG_MIN, INT_MAX)
@@ -340,7 +452,11 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
       int bnu[CPL];
 #pragma unroll
       for (int u = 0; u < CPL; ++u) { bku[u] = LLONG_MIN; bnu[u] = 0x7fffffff; }
-      if (lane < nb) { bku[0] = pb_key(LM ? L->skey[lane] : W->stot[lane]); bnu[0] = lane; }
+      bool stay = lane < nb;
+      if constexpr (LEX)                                  // last frame: no stay inside an unfinished word
+        stay = stay &&
+               (t + 1 < Tb || pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->fin[L->row[cur][lane]]);
+      if (stay) { bku[0] = pb_key(LM ? L->skey[lane] : W->stot[lane]); bnu[0] = lane; }
 #pragma unroll 4
       for (int i = 0; i < nb; ++i) {
         const double ti = g.tot[i], pbi = g.pb[i];
@@ -391,6 +507,9 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
         bool ok;
         if (idx == M) {                                       // the owner's stay candidate
           ok = own < nb;
+          if constexpr (LEX)                              // left out: a LLONG_MIN key would still beat the sentinel
+            ok = ok &&
+                 (t + 1 < Tb || pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->fin[L->row[cur][own]]);
           k = ok ? pb_key(LM ? L->skey[own] : W->stot[own]) : LLONG_MIN;
           n = own;
         } else {
@@ -432,7 +551,7 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
       if (ext) { pi = (n - K) / C; c = (n - K) - pi * C; }
     }
     const unsigned em = __ballot_sync(0xffffffffu, ext);
-    int nr = 0;                                               // LM: the entry's pool row
+    int nr = 0;                                               // LM / LEX: the entry's pool row
     if (lane < nnew) {
       // (win_s is the ranking key; with the LM it is not the CTC mass, which is then recomputed: + 0.0 folds -0.0
       // onto +0.0 as the integer image of win_s does, so that alpha = beta = 0 reproduces the plain search bit for bit)
@@ -440,7 +559,7 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
         gn.pb[lane] = W->spb[n]; gn.pnb[lane] = W->spnb[n]; gn.tot[lane] = LM ? W->stot[n] + 0.0 : W->win_s[lane];
         gn.hash[lane] = g.hash[n]; gn.phash[lane] = g.phash[n];
         gn.last[lane] = g.last[n]; gn.len[lane] = g.len[n]; gn.node[lane] = g.node[n];
-        if constexpr (LM) { nr = L->row[cur][n]; L->row[cur ^ 1][lane] = nr; }
+        if constexpr (LM || LEX) { nr = L->row[cur][n]; L->row[cur ^ 1][lane] = nr; }
       } else {
         const int q = __popc(em & ((1u << lane) - 1u));
         const int nd = nnodes + q;
@@ -467,17 +586,37 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
           L->clo[nr] = lo; L->chi[nr] = hi; L->clen[nr] = min(M + 1, M1);
           L->nrow[q] = nr;
           L->row[cur ^ 1][lane] = nr;
+        } else if constexpr (LEX) {                           // the same row pick without the LM's state
+          unsigned fr = ~used & (K == 16 ? 0xffffffffu : (1u << (2 * K)) - 1u);
+          for (int z = 0; z < q; ++z) fr &= fr - 1u;
+          nr = __ffs(fr) - 1;
+          L->nrow[q] = nr;
+          L->row[cur ^ 1][lane] = nr;
+        }
+        if constexpr (LEX) {
+          const PbLexArgs xa = pb_lex_args(lex...);
+          PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
+          const int nn = lex_step(xa, X->node[L->row[cur][pi]], c);
+          X->node[nr] = nn;
+          X->fin[nr] = nn == 0 || __ldg(xa.word_end + nn);
         }
       }
     }
     nnodes += __popc(em);
     nb = nnew;
     cur ^= 1;
+    if constexpr (LM || LEX) used = __reduce_or_sync(0xffffffffu, lane < nnew ? 1u << nr : 0u);
     if constexpr (LM) {
-      used = __reduce_or_sync(0xffffffffu, lane < nnew ? 1u << nr : 0u);
       if (em) {
         __syncwarp();
         lm_fill_rows(la, L, rows, __popc(em), C, unk, lane);
+      }
+    }
+    if constexpr (LEX) {
+      if (em) {
+        __syncwarp();
+        lex_fill_rows<CPL>(pb_lex_args(lex...), L, pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp),
+                           __popc(em), C, lane);
       }
     }
 #pragma unroll
@@ -525,19 +664,22 @@ __global__ void __launch_bounds__(128) ctc_prefix_beam_kernel(const float* __res
       la.ctc_scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
     } else {
       scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
+      if constexpr (LEX) la.ctc_scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
     }
   }
 }
 
-// Shared launcher: shared memory = per warp the beam state, the LM state + row pool (LM only) and the node array;
-// fewer warps per CTA above 200 KB.
-template <bool LM>
+// Shared launcher: shared memory = per warp the beam state, the pool rows' state + the LM row pool (LM or LEX), the
+// lexicon state (LEX) and the node array; fewer warps per CTA above 200 KB.
+template <bool LM, bool LEX>
 static int pb_launch(const float* log_probs, long long stride_b, long long stride_t, const int* lengths, int B, int T,
-                     int C, int K, int* ids, int* lens, double* scores, const PbLmArgs& la, cudaStream_t stream) {
+                     int C, int K, int* ids, int* lens, double* scores, const PbLmArgs& la, const PbLexArgs& xa,
+                     cudaStream_t stream) {
   if (B <= 0 || T <= 0 || C <= 0 || !log_probs || !ids || !lens || !scores) return HTRVT_ERR_SHAPE;
   if (K < 1 || K > kPbMaxK || C > 32 * kPbCpl || static_cast<long long>(T) * K >= 65535) return HTRVT_ERR_SHAPE;
   int warps = 4;
-  const size_t lm_bytes = LM ? sizeof(PbLmWarp) + sizeof(double) * 2 * K * C : 0;
+  const size_t lm_bytes = ((LM || LEX) ? sizeof(PbLmWarp) : 0) + (LM ? sizeof(double) * 2 * K * C : 0) +
+                          (LEX ? sizeof(PbLexWarp) : 0);
   auto need = [&](int w) {
     return static_cast<size_t>(w) * (sizeof(PbWarp) + lm_bytes + (static_cast<size_t>(T) * K + 1) * 4);
   };
@@ -545,12 +687,22 @@ static int pb_launch(const float* log_probs, long long stride_b, long long strid
   const size_t smem = need(warps);
   if (smem > 227 * 1024) return HTRVT_ERR_SHAPE;
   const dim3 grid((B + warps - 1) / warps), block(warps * 32);
+#define PB_KERNEL(CPL, ...)                                                                                    \
+  do {                                                                                                         \
+    if (smem > 48 * 1024 && !HTRVT_ENSURE_SMEM((ctc_prefix_beam_kernel<CPL, LM, __VA_ARGS__>), 227 * 1024))   \
+      return HTRVT_ERR_LAUNCH;                                                                                 \
+  } while (0)
 #define PB_LAUNCH(CPL)                                                                                         \
   do {                                                                                                         \
-    if (smem > 48 * 1024 && !HTRVT_ENSURE_SMEM((ctc_prefix_beam_kernel<CPL, LM>), 227 * 1024))                \
-      return HTRVT_ERR_LAUNCH;                                                                                 \
-    ctc_prefix_beam_kernel<CPL, LM><<<grid, block, smem, stream>>>(log_probs, stride_b, stride_t, lengths, B, T, \
-                                                                   C, K, ids, lens, scores, la);               \
+    if constexpr (LEX) {                                                                                       \
+      PB_KERNEL(CPL, true, PbLexArgs);                                                                         \
+      ctc_prefix_beam_kernel<CPL, LM, true, PbLexArgs><<<grid, block, smem, stream>>>(                         \
+          log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa);                     \
+    } else {                                                                                                   \
+      PB_KERNEL(CPL, false);                                                                                   \
+      ctc_prefix_beam_kernel<CPL, LM, false><<<grid, block, smem, stream>>>(                                   \
+          log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la);                         \
+    }                                                                                                          \
   } while (0)
   if (C <= 32) PB_LAUNCH(1);
   else if (C <= 64) PB_LAUNCH(2);
@@ -558,7 +710,26 @@ static int pb_launch(const float* log_probs, long long stride_b, long long strid
   else if (C <= 128) PB_LAUNCH(4);
   else PB_LAUNCH(8);
 #undef PB_LAUNCH
+#undef PB_KERNEL
   HTRVT_LAUNCH_CHECK();
+  return HTRVT_OK;
+}
+
+// The LM arguments of htrvt_ctc_prefix_beam_lm / _lex, checked
+static int pb_lm_args(const void* lm_table, long long lm_slots, int lm_order, const int* tok_map, int n_tok_map,
+                      double alpha, double beta, double* ctc_scores, PbLmArgs& la) {
+  if (!lm_table || !ctc_scores || lm_slots < 2 || (lm_slots & (lm_slots - 1)) != 0) return HTRVT_ERR_SHAPE;
+  if (lm_order < 1 || lm_order > kLmMaxOrder || n_tok_map < 0 || (n_tok_map > 0 && !tok_map)) return HTRVT_ERR_SHAPE;
+  if (!isfinite(alpha) || !isfinite(beta)) return HTRVT_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(lm_table) & 31) != 0) return HTRVT_ERR_ALIGN;
+  la.table = static_cast<const PbLmSlot*>(lm_table);
+  la.mask = static_cast<unsigned long long>(lm_slots - 1);
+  la.order = lm_order;
+  la.tok_map = tok_map;
+  la.n_map = n_tok_map;
+  la.alpha = alpha;
+  la.beta = beta;
+  la.ctc_scores = ctc_scores;
   return HTRVT_OK;
 }
 
@@ -572,7 +743,8 @@ using namespace htrvt;
 extern "C" int htrvt_ctc_prefix_beam(const float* log_probs, long long stride_b, long long stride_t,
                                      const int* lengths, int B, int T, int C, int K, int* ids, int* lens,
                                      double* scores, cudaStream_t stream) {
-  return pb_launch<false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, PbLmArgs{}, stream);
+  return pb_launch<false, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, PbLmArgs{},
+                                 PbLexArgs{}, stream);
 }
 
 // The same search with a character n-gram LM fused into the ranking (header: include/htrvt.h).  lm_table: lm_slots
@@ -584,18 +756,41 @@ extern "C" int htrvt_ctc_prefix_beam_lm(const float* log_probs, long long stride
                                         long long lm_slots, int lm_order, const int* tok_map, int n_tok_map,
                                         double alpha, double beta, int* ids, int* lens, double* scores,
                                         double* ctc_scores, cudaStream_t stream) {
-  if (!lm_table || !ctc_scores || lm_slots < 2 || (lm_slots & (lm_slots - 1)) != 0) return HTRVT_ERR_SHAPE;
-  if (lm_order < 1 || lm_order > kLmMaxOrder || n_tok_map < 0 || (n_tok_map > 0 && !tok_map)) return HTRVT_ERR_SHAPE;
-  if (!isfinite(alpha) || !isfinite(beta)) return HTRVT_ERR_SHAPE;
-  if ((reinterpret_cast<uintptr_t>(lm_table) & 31) != 0) return HTRVT_ERR_ALIGN;
   PbLmArgs la;
-  la.table = static_cast<const PbLmSlot*>(lm_table);
-  la.mask = static_cast<unsigned long long>(lm_slots - 1);
-  la.order = lm_order;
-  la.tok_map = tok_map;
-  la.n_map = n_tok_map;
-  la.alpha = alpha;
-  la.beta = beta;
-  la.ctc_scores = ctc_scores;
-  return pb_launch<true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, stream);
+  const int st = pb_lm_args(lm_table, lm_slots, lm_order, tok_map, n_tok_map, alpha, beta, ctc_scores, la);
+  if (st != HTRVT_OK) return st;
+  return pb_launch<true, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, PbLexArgs{},
+                               stream);
+}
+
+// The same search constrained to a word lexicon, with or without the LM (header: include/htrvt.h).  The trie (CSR,
+// node 0 = root, edges sorted by label within a node, child ids < n_nodes) is the documented contract that
+// htr-vt_b200/lexicon.py packs and checks; it is not re-validated here.  lm_table == nullptr: no LM, alpha = beta = 0.
+extern "C" int htrvt_ctc_prefix_beam_lex(const float* log_probs, long long stride_b, long long stride_t,
+                                         const int* lengths, int B, int T, int C, int K, const int* first,
+                                         const int* label, const int* child, const unsigned char* word_end,
+                                         int n_nodes, const unsigned char* is_word, int n_class_map,
+                                         const void* lm_table, long long lm_slots, int lm_order, const int* tok_map,
+                                         int n_tok_map, double alpha, double beta, int* ids, int* lens,
+                                         double* scores, double* ctc_scores, cudaStream_t stream) {
+  if (!first || !label || !child || !word_end || n_nodes < 1 || !ctc_scores) return HTRVT_ERR_SHAPE;
+  if (n_class_map < 0 || (n_class_map > 0 && !is_word)) return HTRVT_ERR_SHAPE;
+  PbLexArgs xa;
+  xa.first = first;
+  xa.label = label;
+  xa.child = child;
+  xa.word_end = word_end;
+  xa.is_word = is_word;
+  xa.n_map = n_class_map;
+  if (!lm_table) {
+    if (alpha != 0.0 || beta != 0.0) return HTRVT_ERR_SHAPE;
+    PbLmArgs la{};
+    la.ctc_scores = ctc_scores;
+    return pb_launch<false, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa,
+                                  stream);
+  }
+  PbLmArgs la;
+  const int st = pb_lm_args(lm_table, lm_slots, lm_order, tok_map, n_tok_map, alpha, beta, ctc_scores, la);
+  if (st != HTRVT_OK) return st;
+  return pb_launch<true, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa, stream);
 }

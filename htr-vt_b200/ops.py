@@ -424,6 +424,45 @@ def ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta=0.0, lengths=None, 
     return ids, lens, scores, ctc_scores
 
 
+def ctc_prefix_beam_lex(log_probs, beam_size, lexicon, lm=None, alpha=0.0, beta=0.0, lengths=None, layout="tbc"):
+    """ctc_prefix_beam (lm=None; alpha = beta = 0) or ctc_prefix_beam_lm (lm: a CharNGramLM) constrained to a word
+    lexicon (lexicon.py::Lexicon): every maximal run of word characters in a returned labelling is a lexicon word.
+    Ranking and scores are those of the unconstrained search; the lexicon only removes candidates.  Returns (ids
+    [B,K,T] int32, lens [B,K] int32 (-1 = no such labelling; all K when the line has no accepted labelling), scores
+    [B,K] float64 (fused; = ctc_scores without an LM), ctc_scores [B,K] float64)."""
+    _need_cuda(log_probs)
+    if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
+        raise HtrvtError("ctc_prefix_beam_lex expects fp32 log-probs with a contiguous class axis")
+    if lexicon.first.device != log_probs.device:
+        raise HtrvtError("ctc_prefix_beam_lex: the lexicon lives on %s, the log-probs on %s"
+                         % (lexicon.first.device, log_probs.device))
+    if lm is not None and lm.table.device != log_probs.device:
+        raise HtrvtError("ctc_prefix_beam_lex: the LM table lives on %s, the log-probs on %s"
+                         % (lm.table.device, log_probs.device))
+    if layout == "btc":
+        B, T, C = log_probs.shape
+        sb, st = log_probs.stride(0), log_probs.stride(1)
+    else:
+        T, B, C = log_probs.shape
+        sb, st = log_probs.stride(1), log_probs.stride(0)
+    dev = log_probs.device
+    K = int(beam_size)
+    ids = torch.empty((B, K, T), dtype=torch.int32, device=dev)
+    lens = torch.empty((B, K), dtype=torch.int32, device=dev)
+    scores = torch.empty((B, K), dtype=torch.float64, device=dev)
+    ctc_scores = torch.empty((B, K), dtype=torch.float64, device=dev)
+    ln = None if lengths is None else lengths.to(device=dev, dtype=torch.int32).contiguous()
+    lx = lexicon
+    lm_args = ((None, 0, 0, None, 0) if lm is None else
+               (lm.table, lm.slots, lm.order, lm.token_map, lm.token_map.numel()))
+    check(lib().htrvt_ctc_prefix_beam_lex(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(lx.first), _p(lx.label),
+                                          _p(lx.child), _p(lx.word_end), lx.n_nodes, _p(lx.is_word),
+                                          lx.is_word.numel(), _p(lm_args[0]), lm_args[1], lm_args[2], _p(lm_args[3]),
+                                          lm_args[4], float(alpha), float(beta), _p(ids), _p(lens), _p(scores),
+                                          _p(ctc_scores), _stream()), "htrvt_ctc_prefix_beam_lex")
+    return ids, lens, scores, ctc_scores
+
+
 CtcAlignment = collections.namedtuple("CtcAlignment", "path frame_scores spans token_scores score status")
 
 
@@ -1083,7 +1122,7 @@ def _instrument():
     import functools
     g = globals()
     names = ["gemm_tn", "gemm_nn", "linear_wgrad", "conv_fwd", "conv_dgrad", "conv_dgrad_bn", "conv_wgrad", "conv_wgrad_acc", "conv_wgrad_acc_t", "conv_wgrad_acc_w", "unpack_conv_grads", "attention_fwd",
-             "attention_bwd", "attention2_fwd", "attention2_bwd", "attention_f32", "attention2_f32", "split3", "conv_fwd_split", "bn_act_f32", "maxpool_f32", "tokens_f32", "row_ln_f32", "gelu_split", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "ctc_prefix_beam_lm", "ctc_align", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
+             "attention_bwd", "attention2_fwd", "attention2_bwd", "attention_f32", "attention2_f32", "split3", "conv_fwd_split", "bn_act_f32", "maxpool_f32", "tokens_f32", "row_ln_f32", "gelu_split", "ctc_loss_grad", "greedy_decode_ids", "ctc_collapse", "ctc_kbest_paths", "ctc_prefix_beam", "ctc_prefix_beam_lm", "ctc_prefix_beam_lex", "ctc_align", "augment_lines", "sample_ln_fwd", "sample_ln_bwd", "line_prep_u8", "edit_distance",
              "row_ln_fwd", "row_ln_bwd", "tokens_fwd", "tokens_bwd", "gelu_fwd", "gelu_bwd", "colsum_bf16", "cast_bf16", "cast_colsum_bf16", "dropout_",
              "pack_conv_weight", "pack_weights", "conv1_fwd", "bn_finalize", "bn_act_fwd", "pool_fwd", "pool_bwd", "bn_bwd", "bn_bwd_apply",
              "conv1_wgrad", "stem_head_moments", "stem_head_fwd", "stem_head_bwd"]

@@ -109,6 +109,31 @@ int htrvt_ctc_prefix_beam_lm(const float* log_probs, long long stride_b, long lo
                              const int* tok_map, int n_tok_map, double alpha, double beta, int* ids, int* lens,
                              double* scores, double* ctc_scores, void* stream);
 
+/* ---- CTC prefix beam search constrained to a word lexicon --------------------------------------------------------
+ * htrvt_ctc_prefix_beam_lex is htrvt_ctc_prefix_beam (lm_table == nullptr; alpha = beta = 0) or
+ * htrvt_ctc_prefix_beam_lm (the same LM arguments) in which every word of the output comes from a word list (Scheidl
+ * et al. 2018, "Word Beam Search", "Words" mode).  Classes split into word characters (is_word[c] != 0) and free
+ * characters (all others, ids >= n_class_map included).  A labelling is accepted when every maximal run of word
+ * characters in it is a lexicon word.  Each entry carries a trie node, 0 = between words: between words a free
+ * character stays at 0 and a word character c moves to child(root, c); inside a word at node n a word character c
+ * moves to child(n, c) and a free character is allowed only if n ends a word (back to 0); a missing child is not
+ * allowed; a stay never changes the node.  In a line's last frame no candidate that leaves its entry at a node that
+ * does not end a word is eligible, so the survivors are the K best accepted labellings (lens -1 for all K when none
+ * exists; a line of zero frames gives the empty labelling).  Ranking, ties and scores are those of the plain / LM
+ * search: the lexicon only removes candidates, and with no word character the results equal theirs bit for bit.
+ * Trie in CSR form: first int32 [n_nodes + 1] (node 0 = root), label / child int32 [first[n_nodes]] (the edges of
+ * node n are first[n] .. first[n + 1] - 1, sorted by label, child ids < n_nodes), word_end uint8 [n_nodes]; its
+ * consistency is the caller's contract (htr-vt_b200/lexicon.py packs and checks it), not re-checked on the device.
+ * ctc_scores = lae(pb, pnb), scores = the LM's fused score (= ctc_scores without an LM).  HTRVT_ERR_SHAPE: a null
+ * trie array, n_nodes < 1, n_class_map > 0 with no is_word, alpha or beta != 0 without an LM, the LM checks of
+ * htrvt_ctc_prefix_beam_lm with one, or the limits of htrvt_ctc_prefix_beam (K <= 16, C <= 256, T * K < 65535). */
+int htrvt_ctc_prefix_beam_lex(const float* log_probs, long long stride_b, long long stride_t, const int* lengths, int B,
+                              int T, int C, int K, const int* first, const int* label, const int* child,
+                              const unsigned char* word_end, int n_nodes, const unsigned char* is_word,
+                              int n_class_map, const void* lm_table, long long lm_slots, int lm_order,
+                              const int* tok_map, int n_tok_map, double alpha, double beta, int* ids, int* lens,
+                              double* scores, double* ctc_scores, void* stream);
+
 /* ---- CTC forced alignment of a known transcription -----------------------------------------------------------
  * htrvt_ctc_align: the single best path (Viterbi) through the CTC trellis of each line's labels, blank = 0, with the
  * frames each label occupies: the alignment torchaudio.functional.forced_align computes one line at a time on the host.
