@@ -17,12 +17,13 @@ from .beam import (beam_search_with_lm_batch, ctc_lexicon_decode, ctc_lm_decode,
                    simple_ctc_beam_search_with_lm)
 from .lexicon import Lexicon  # noqa: F401
 from .lm import CharNGramLM  # noqa: F401
+from .wordlm import WordNGramLM  # noqa: F401
 from .prefetch import HostPrefetcher, RunningLoss  # noqa: F401
 from .augment import SameTrCollate, augment_lines, draw_collate_params  # noqa: F401
 from .align import align_text, ctc_align, forced_align  # noqa: F401
 
 __all__ = ["CTCLoss", "ctc_loss_from_logits", "greedy_decode", "CTCLabelConverter", "ErrorRateMeter", "cer_from_ids",
            "edit_distances", "format_string_for_wer", "simple_ctc_beam_search_with_lm", "beam_search_with_lm_batch",
-           "kbest_candidates", "ctc_lm_decode", "CharNGramLM", "ctc_lexicon_decode", "Lexicon", "HostPrefetcher",
-           "RunningLoss", "SameTrCollate",
+           "kbest_candidates", "ctc_lm_decode", "CharNGramLM", "ctc_lexicon_decode", "Lexicon", "WordNGramLM",
+           "HostPrefetcher", "RunningLoss", "SameTrCollate",
            "augment_lines", "draw_collate_params", "ctc_align", "forced_align", "align_text"]

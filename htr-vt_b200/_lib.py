@@ -56,6 +56,8 @@ SIGNATURES = {
                                       ctypes.c_double, _P, _P, _P, _P, _P]),
     "htrvt_ctc_prefix_beam_lex": (_I, [_P, _L, _L, _P, _I, _I, _I, _I, _P, _P, _P, _P, _I, _P, _I, _P, _L, _I, _P, _I,
                                        ctypes.c_double, ctypes.c_double, _P, _P, _P, _P, _P]),
+    "htrvt_ctc_prefix_beam_lex_wlm": (_I, [_P, _L, _L, _P, _I, _I, _I, _I, _P, _P, _P, _P, _I, _P, _I, _P, _L, _I, _P,
+                                           _P, ctypes.c_double, ctypes.c_double, _P, _P, _P, _P, _P]),
     "htrvt_ctc_align_workspace_bytes": (_Z, [_I, _I, _I]),
     "htrvt_ctc_align": (_I, [_P, _L, _L, _I, _P, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _P, _Z, _P]),
     "htrvt_set_pdl": (_I, [_I]),

@@ -18,7 +18,9 @@ log10 p(char | context) + beta, and the line's end adds the </s> term, so the LM
 instead of only picking among the K the acoustic model kept.
 
 `kbest_candidates(..., search="prefix", lexicon=Lexicon)` and `ctc_lexicon_decode` constrain that search to a word
-lexicon (lexicon.py, csrc/prefix_beam.cu): every word of a candidate comes from the list, with or without the LM.
+lexicon (lexicon.py, csrc/prefix_beam.cu): every word of a candidate comes from the list, with or without the LM.  The
+LM may also be a word n-gram LM built on that lexicon (WordNGramLM, wordlm.py): every finished word is then scored by
+alpha * ln(10) * log10 p(word | previous words) + beta inside the search.
 """
 import numpy as np
 import torch
@@ -54,7 +56,9 @@ def kbest_candidates(log_probs, converter, beam_size=5, lengths=None, layout="tb
     or "prefix" (CTC prefix beam search; score = log-probability of the labelling).  lm (a CharNGramLM, prefix search
     only) with weight alpha and per-character bonus beta: the candidates come from the LM-fused search, in its order,
     and score = CTC log-prob + alpha * ln(10) * log10 P(string </s>) + beta * len.  lexicon (a Lexicon, prefix search
-    only, with or without lm): only labellings whose every word is in the lexicon, ranked and scored as without it."""
+    only, with or without lm): only labellings whose every word is in the lexicon, ranked and scored as without it.
+    With lexicon, lm may be a WordNGramLM built on it: score = CTC log-prob + alpha * ln(10) * log10 P(w_1 .. w_m
+    </s>) + beta * m over the string's m words (a word LM without a lexicon is a ValueError)."""
     if search not in ("paths", "prefix"):
         raise ValueError("search must be 'paths' or 'prefix'")
     if lexicon is not None:
@@ -124,8 +128,10 @@ def ctc_lm_decode(preds_log, converter, lm, alpha, beta=0.0, beam_size=8, length
 
 def ctc_lexicon_decode(preds_log, converter, lexicon, beam_size=8, lengths=None, lm=None, alpha=0.0, beta=0.0):
     """preds_log [T, B, C] (validation_with_kenlm's layout) -> B strings: the best-ranked labelling per line of the CTC
-    prefix beam search constrained to lexicon (a Lexicon on the same device), with the character LM lm (weights alpha,
-    beta) fused in when given ("" for the empty labelling, and for a line with no accepted labelling)."""
+    prefix beam search constrained to lexicon (a Lexicon on the same device), with lm (weights alpha, beta) fused in
+    when given ("" for the empty labelling, and for a line with no accepted labelling).  lm: a CharNGramLM (score =
+    CTC log-prob + alpha * ln(10) * log10 P(string </s>) + beta * len) or a WordNGramLM built on lexicon (score = CTC
+    log-prob + alpha * ln(10) * log10 P(w_1 .. w_m </s>) + beta * m over the string's m words)."""
     if not preds_log.is_cuda:
         raise ops.HtrvtError("ctc_lexicon_decode needs a CUDA tensor (no CPU fallback)")
     lp = preds_log.float()

@@ -36,20 +36,31 @@
 // `excl`, so the selection rounds skip them; in the line's last frame `allow_last` is used and an entry left inside an
 // unfinished word cannot stay.  Ranking and scores are otherwise those of the plain / LM search: the lexicon only
 // removes candidates.
+//
+// The word-LM instantiation (LM = LEX = true with PbWlmArgs, htrvt_ctc_prefix_beam_lex_wlm) scores the WORDS of the
+// lexicon-constrained search with a word n-gram LM (Scheidl et al. 2018, "NGrams" mode).  Each pool row holds `done`
+// (the float64 sum of alpha * ln10 * log10 p(word | <s> previous words) + beta over the entry's finished words) and the
+// word context; its ranking value lm is done, plus alpha * ln10 * smear(node) inside a word (the best unigram
+// log10 prob of the lexicon words below the node).  A created row costs at most two n-gram queries: the completion of
+// the word ending at its node and the </s> term after it.
 #include "common.cuh"
 #include <climits>
+#include <type_traits>
 
 namespace htrvt {
 
 constexpr int kPbMaxK = 16;         // beam entries
 constexpr int kPbCpl = 8;           // classes per lane held in registers: C <= 256
 constexpr int kLmMaxOrder = 8;      // n-gram order: contexts of up to 7 tokens, keys of up to 8 16-bit fields
+constexpr int kWlmMaxOrder = 6;     // word n-gram order: keys of up to 6 21-bit fields
+constexpr int kWlmBits = 21;        // key-field width of the word LM's table (token ids < 2^21 - 1)
 constexpr double kLn10 = 2.302585092994046;
 constexpr int kLmUnk = 0, kLmBos = 1, kLmEos = 2;   // token ids of <unk>, <s>, </s>
 
 // One slot of the LM's open-addressing table (32 bytes, one sector).  Key = the n-gram's tokens, LAST token first, as
-// 16-bit fields (token + 1; 0 = no token) in lo (fields 0-3) and hi (fields 4-7); lo == 0 marks an empty slot.  Keys
-// are compared in full, so a hash collision never matches.  Linear probing from lm_hash(lo, hi) & (slots - 1).
+// FB-bit fields (token + 1; 0 = no token), 64 / FB of them per word: lo holds the first, hi the next (character LM:
+// FB = 16, fields 0-3 and 4-7; word LM: FB = 21, fields 0-2 and 3-5); lo == 0 marks an empty slot.  Keys are compared
+// in full, so a hash collision never matches.  Linear probing from lm_hash(lo, hi) & (slots - 1).
 struct PbLmSlot {
   unsigned long long lo, hi;
   float p, b;                        // log10 probability, log10 backoff
@@ -91,6 +102,19 @@ struct PbLexWarp {                  // lexicon state of one line; per pool row (
   unsigned allow[2 * kPbMaxK][kPbCpl];                      // bit (c & 31) of word c >> 5: c may extend the entry
   unsigned allow_last[2 * kPbMaxK][kPbCpl];                 // ... and leaves it between words or at a word end
   unsigned freem[kPbCpl];                                   // the free classes 1 .. C - 1
+};
+
+// Word n-gram LM over the lexicon's trie (htr-vt_b200/wordlm.py packs it); the table, order and weights come in
+// PbLmArgs (tok_map unused).  node_tok: trie node -> token id of the word ending there; smear: trie node -> the largest
+// unigram log10 prob of the lexicon words that start with the node's prefix.
+struct PbWlmArgs {
+  PbLexArgs lex;
+  const int* node_tok;
+  const float* smear;
+};
+struct PbWlmWarp {                  // word-LM state of one line
+  double done[2 * kPbMaxK];                                 // per pool row: the finished words' LM terms
+  double comp[kPbMaxK], eosq[kPbMaxK];                      // per row created this frame: completion, </s> term
 };
 
 struct PbGen {                      // one beam generation of one line
@@ -155,16 +179,27 @@ __device__ __forceinline__ long long lm_walk(const PbLmSlot* t, unsigned long lo
   }
   return -1;
 }
-// the first m fields of a context (key-field layout)
+// the first m fields of a context (key-field layout, FB-bit fields)
+template <int FB>
 __device__ __forceinline__ void lm_ctx_prefix(unsigned long long clo, unsigned long long chi, int m,
                                               unsigned long long& lo, unsigned long long& hi) {
-  if (m >= 4) {
+  constexpr int P = 64 / FB;                               // fields per word
+  if (m >= P) {
     lo = clo;
-    hi = chi & ((1ull << (16 * (m - 4))) - 1ull);
+    hi = chi & ((1ull << (FB * (m - P))) - 1ull);
   } else {
-    lo = clo & ((1ull << (16 * m)) - 1ull);
+    lo = clo & ((1ull << (FB * m)) - 1ull);
     hi = 0ull;
   }
+}
+// (lo, hi) shifted by one field with token tok in field 0: a key (w first) or a context (most recent token first)
+template <int FB>
+__device__ __forceinline__ void lm_push(unsigned long long lo, unsigned long long hi, int tok, unsigned long long& klo,
+                                        unsigned long long& khi) {
+  constexpr int P = 64 / FB;
+  constexpr unsigned long long used = FB * P == 64 ? ~0ull : (1ull << (FB * P)) - 1ull;
+  klo = ((lo << FB) | static_cast<unsigned long long>(tok + 1)) & used;
+  khi = ((hi << FB) | (lo >> (FB * (P - 1)))) & used;
 }
 __device__ __forceinline__ int lm_tok(const PbLmArgs& a, int c) { return c < a.n_map ? __ldg(a.tok_map + c) : kLmUnk; }
 
@@ -182,7 +217,7 @@ __device__ __forceinline__ void lm_fill_rows(const PbLmArgs& a, PbLmWarp* L, dou
     float bw = 0.f;
     if (k <= L->clen[r]) {
       unsigned long long lo, hi;
-      lm_ctx_prefix(L->clo[r], L->chi[r], k, lo, hi);
+      lm_ctx_prefix<16>(L->clo[r], L->chi[r], k, lo, hi);
       const unsigned long long i = lm_hash(lo, hi) & a.mask;
       const long long f = lm_walk(a.table, a.mask, lo, hi, i, lm_key_at(a.table, i));
       if (f >= 0) bw = lm_val_at(a.table, static_cast<unsigned long long>(f)).y;
@@ -212,9 +247,8 @@ __device__ __forceinline__ void lm_fill_rows(const PbLmArgs& a, PbLmWarp* L, dou
     for (int m = 0; m < kLmMaxOrder; ++m) {                   // key of (last m context tokens, w): w first
       if (m <= M) {
         unsigned long long lo, hi;
-        lm_ctx_prefix(clo, chi, m, lo, hi);
-        klo[m] = (lo << 16) | static_cast<unsigned long long>(tok + 1);
-        khi[m] = (hi << 16) | (lo >> 48);
+        lm_ctx_prefix<16>(clo, chi, m, lo, hi);
+        lm_push<16>(lo, hi, tok, klo[m], khi[m]);
         ix[m] = lm_hash(klo[m], khi[m]) & a.mask;
         s[m] = lm_key_at(a.table, ix[m]);
         p[m] = lm_val_at(a.table, ix[m]).x;
@@ -253,9 +287,11 @@ __device__ __forceinline__ bool lex_free(const PbLexArgs& a, int c) { return c >
 // Fill the masks of rows L->nrow[0 .. nE) (their node / fin already set).  From a finished node (0 or a word end) every
 // free class leads back to state 0, which both masks accept; a child edge c leads to the child, which allow_last
 // accepts only when the child ends a word.  All 32 lanes: first the free-class part word by word, then the child edges.
-template <int CPL>
+// WLM: the child edges' LM row entries too, done + alpha ln10 smear(child) (the other classes are already filled).
+template <int CPL, bool WLM = false>
 __device__ __forceinline__ void lex_fill_rows(const PbLexArgs& a, const PbLmWarp* L, PbLexWarp* X, int nE, int C,
-                                              int lane) {
+                                              int lane, double* rows = nullptr, const double* done = nullptr,
+                                              const float* smear = nullptr, double alpha = 0.0) {
   for (int idx = lane; idx < nE * CPL; idx += 32) {
     const int e = idx / CPL, w = idx - e * CPL;
     const int r = L->nrow[e];
@@ -274,6 +310,10 @@ __device__ __forceinline__ void lex_fill_rows(const PbLexArgs& a, const PbLmWarp
         const unsigned bit = 1u << (c & 31);
         atomicOr(&X->allow[r][c >> 5], bit);
         if (__ldg(a.word_end + __ldg(a.child + j))) atomicOr(&X->allow_last[r][c >> 5], bit);
+        if constexpr (WLM) {
+          const double sm = static_cast<double>(__ldg(smear + __ldg(a.child + j)));
+          rows[r * C + c] = __dadd_rn(done[r], __dmul_rn(alpha, __dmul_rn(kLn10, sm)));
+        }
       }
     }
   }
@@ -291,33 +331,146 @@ __device__ __forceinline__ int lex_step(const PbLexArgs& a, int n, int c) {
   return __ldg(a.child + lo);
 }
 
+// ---- word n-gram LM -------------------------------------------------------------------------------------------------
+// log10 p(tok | context) by ARPA backoff (the arithmetic of lm_fill_rows) for one query in one lane: context (clo, chi)
+// of M <= kWlmMaxOrder - 1 tokens; the first slots of every level's n-gram key and context key are loaded before any
+// of them is looked at.
+__device__ __forceinline__ double wlm_logprob(const PbLmArgs& a, unsigned long long clo, unsigned long long chi, int M,
+                                              int tok, float unk) {
+  unsigned long long klo[kWlmMaxOrder], khi[kWlmMaxOrder], ix[kWlmMaxOrder];
+  unsigned long long blo[kWlmMaxOrder], bhi[kWlmMaxOrder], bix[kWlmMaxOrder];
+  ulonglong2 s[kWlmMaxOrder], bs[kWlmMaxOrder];
+  float p[kWlmMaxOrder], bw[kWlmMaxOrder];
+#pragma unroll
+  for (int m = 0; m < kWlmMaxOrder; ++m) {                   // level m: (last m context tokens, tok) and its context
+    if (m <= M) {
+      lm_ctx_prefix<kWlmBits>(clo, chi, m, blo[m], bhi[m]);
+      lm_push<kWlmBits>(blo[m], bhi[m], tok, klo[m], khi[m]);
+      ix[m] = lm_hash(klo[m], khi[m]) & a.mask;
+      s[m] = lm_key_at(a.table, ix[m]);
+      p[m] = lm_val_at(a.table, ix[m]).x;
+      if (m > 0) {
+        bix[m] = lm_hash(blo[m], bhi[m]) & a.mask;
+        bs[m] = lm_key_at(a.table, bix[m]);
+        bw[m] = lm_val_at(a.table, bix[m]).y;
+      }
+    }
+  }
+  double S = 0.0;
+  bool found = false;
+#pragma unroll
+  for (int m = kWlmMaxOrder - 1; m >= 0; --m) {
+    if (m <= M && !found) {
+      if (s[m].x == klo[m] && s[m].y == khi[m]) {
+        S += static_cast<double>(p[m]);
+        found = true;
+      } else {
+        const long long f = s[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, klo[m], khi[m], ix[m], s[m]);
+        if (f >= 0) {
+          S += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(f)).x);
+          found = true;
+        } else if (m > 0) {                                  // the context's bow, 0 when it is not listed
+          if (bs[m].x == blo[m] && bs[m].y == bhi[m]) {
+            S += static_cast<double>(bw[m]);
+          } else {
+            const long long g = bs[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, blo[m], bhi[m], bix[m], bs[m]);
+            if (g >= 0) S += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(g)).y);
+          }
+        }
+      }
+    }
+  }
+  if (!found) S += static_cast<double>(unk);
+  return S;
+}
+
+// Fill the word-LM rows L->nrow[0 .. nE) (node / fin, done and context already set), before lex_fill_rows<CPL, true>
+// writes their child edges.  An entry at a finished node n (0 or a word end) with context h: comp = alpha ln10
+// log10 p(node_tok[n] | h) + beta when n != 0, eos = [comp +] alpha ln10 log10 p(</s> | h') with h' = node_tok[n] h
+// truncated (h when n == 0); row[c] = done (+ comp when n != 0) for the free classes c.  Inside a word nothing is
+// queried (no free class is allowed there and the entry cannot end the line).  Query lane 2 e: comp, 2 e + 1: </s>.
+__device__ __forceinline__ void wlm_fill_rows(const PbLmArgs& a, const PbWlmArgs& w, PbLmWarp* L, const PbLexWarp* X,
+                                              PbWlmWarp* Y, double* rows, int nE, int C, float unk, int lane) {
+  const int M1 = a.order - 1;
+  for (int idx = lane; idx < 2 * nE; idx += 32) {
+    const int e = idx >> 1, r = L->nrow[e], n = X->node[r];
+    if (!X->fin[r]) continue;
+    unsigned long long lo = L->clo[r], hi = L->chi[r];
+    int M = L->clen[r], tok = kLmEos;
+    if ((idx & 1) == 0) {
+      if (n == 0) {
+        Y->comp[e] = 0.0;
+        continue;
+      }
+      tok = __ldg(w.node_tok + n);
+    } else if (n != 0) {
+      lm_push<kWlmBits>(lo, hi, __ldg(w.node_tok + n), lo, hi);
+      lm_ctx_prefix<kWlmBits>(lo, hi, M1, lo, hi);
+      M = min(M + 1, M1);
+    }
+    const double t = __dmul_rn(a.alpha, __dmul_rn(kLn10, wlm_logprob(a, lo, hi, M, tok, unk)));
+    if ((idx & 1) == 0) Y->comp[e] = __dadd_rn(t, a.beta);
+    else Y->eosq[e] = t;
+  }
+  __syncwarp();
+  const int Cm = C - 1;
+  for (int idx = lane; idx < nE * C; idx += 32) {             // nE * (C - 1) labels, then nE eos terms
+    const int e = idx < nE * Cm ? idx / Cm : idx - nE * Cm;
+    const int r = L->nrow[e];
+    const bool wend = X->fin[r] && X->node[r] != 0;
+    if (idx < nE * Cm) {
+      const int c = idx - e * Cm + 1;
+      const bool fr = (X->freem[c >> 5] >> (c & 31)) & 1u;
+      rows[r * C + c] = (fr && wend) ? __dadd_rn(Y->done[r], Y->comp[e]) : Y->done[r];
+    } else {
+      L->eos[r] = !X->fin[r] ? 0.0 : wend ? __dadd_rn(Y->comp[e], Y->eosq[e]) : Y->eosq[e];
+    }
+  }
+  __syncwarp();
+}
+
+// the lexicon pack of the word-LM instantiation
+template <typename... Lex>
+constexpr bool kPbWlm = false;
+template <>
+constexpr bool kPbWlm<PbWlmArgs> = true;
+
 __device__ __forceinline__ PbLexArgs pb_lex_args(const PbLexArgs& a) { return a; }
+__device__ __forceinline__ PbLexArgs pb_lex_args(const PbWlmArgs& a) { return a.lex; }
+__device__ __forceinline__ PbWlmArgs pb_wlm_args(const PbWlmArgs& a) { return a; }
 // a warp's lexicon state: after `front` bytes per warp (its beam state, pool rows' state and LM row pool)
 __device__ __forceinline__ PbLexWarp* pb_lex_warp(uint8_t* smem, size_t front, int warps, int warp) {
   return reinterpret_cast<PbLexWarp*>(smem + front * warps) + warp;
 }
+// a warp's word-LM state: after the lexicon states
+__device__ __forceinline__ PbWlmWarp* pb_wlm_warp(uint8_t* smem, size_t front, int warps, int warp) {
+  return reinterpret_cast<PbWlmWarp*>(smem + (front + sizeof(PbLexWarp)) * warps) + warp;
+}
 
-// class slots per lane: C <= 32 * CPL; LM: fused character n-gram LM; LEX: word lexicon constraint, whose PbLexArgs
-// come in the pack Lex.  With LEX off the pack is empty and every lexicon variable lives inside `if constexpr (LEX)`,
-// so that the plain and LM kernels keep their parameter list and compile to the same code as before the lexicon.
+// class slots per lane: C <= 32 * CPL; LM: fused n-gram LM; LEX: word lexicon constraint, whose PbLexArgs come in the
+// pack Lex.  With LEX off the pack is empty and every lexicon variable lives inside `if constexpr (LEX)`, so that the
+// plain and LM kernels keep their parameter list and compile to the same code as before the lexicon.  LM and LEX with
+// a PbWlmArgs in the pack (kPbWlm): the LM is the word LM, every character-LM step inside `if constexpr (!kPbWlm)`.
 // (Min. blocks 1 for LEX: without it ptxas caps some lexicon instantiations at 56-128 registers and spills.)
 template <int CPL, bool LM, bool LEX, typename... Lex>
 __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const float* __restrict__ x, long long sb, long long st,
                                                               const int* __restrict__ lengths, int B, int T, int C,
                                                               int K, int* __restrict__ ids, int* __restrict__ lens,
                                                               double* __restrict__ scores, PbLmArgs la, Lex... lex) {
-  static_assert(sizeof...(Lex) == (LEX ? 1 : 0), "LEX takes one PbLexArgs");
+  static_assert(sizeof...(Lex) == (LEX ? 1 : 0), "LEX takes one PbLexArgs or PbWlmArgs");
   extern __shared__ __align__(16) uint8_t pb_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
   const int b = blockIdx.x * warps + warp;
   if (b >= B) return;
   PbWarp* W = reinterpret_cast<PbWarp*>(pb_smem) + warp;
-  // per warp: PbWarp | PbLmWarp (LM or LEX: the pool rows' bookkeeping) + the LM row pool (LM) | PbLexWarp (LEX) | nodes
+  // per warp: PbWarp | PbLmWarp (LM or LEX: the pool rows' bookkeeping) + the LM row pool (LM) | PbLexWarp (LEX) |
+  // PbWlmWarp (word LM) | nodes
   const size_t lm_bytes = (LM || LEX) ? sizeof(PbLmWarp) + (LM ? sizeof(double) * 2 * K * C : 0) : 0;
   PbLmWarp* L = reinterpret_cast<PbLmWarp*>(pb_smem + sizeof(PbWarp) * warps) + warp;
   double* rows = reinterpret_cast<double*>(pb_smem + (sizeof(PbWarp) + sizeof(PbLmWarp)) * warps) +
                  static_cast<size_t>(warp) * 2 * K * C;
-  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + (sizeof(PbWarp) + lm_bytes + (LEX ? sizeof(PbLexWarp) : 0)) *
+  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + (sizeof(PbWarp) + lm_bytes + (LEX ? sizeof(PbLexWarp) : 0) +
+                                                           (kPbWlm<Lex...> ? sizeof(PbWlmWarp) : 0)) *
                                                            warps) +
                     static_cast<size_t>(warp) * (static_cast<size_t>(T) * K + 1);
   int Tb = lengths ? lengths[b] : T;
@@ -343,9 +496,10 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
       L->clen[0] = min(1, la.order - 1);
       L->clo[0] = la.order > 1 ? static_cast<unsigned long long>(kLmBos + 1) : 0ull;
       L->chi[0] = 0ull;
+      if constexpr (kPbWlm<Lex...>) pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->done[0] = 0.0;
     }
     __syncwarp();
-    lm_fill_rows(la, L, rows, 1, C, unk, lane);
+    if constexpr (!kPbWlm<Lex...>) lm_fill_rows(la, L, rows, 1, C, unk, lane);
   }
   if constexpr (LEX) {
     const PbLexArgs xa = pb_lex_args(lex...);
@@ -361,7 +515,14 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
       X->node[0] = 0; X->fin[0] = 1;
     }
     __syncwarp();
-    lex_fill_rows<CPL>(xa, L, X, 1, C, lane);
+    if constexpr (kPbWlm<Lex...>) {
+      const PbWlmArgs wa = pb_wlm_args(lex...);
+      PbWlmWarp* Y = pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
+      wlm_fill_rows(la, wa, L, X, Y, rows, 1, C, unk, lane);
+      lex_fill_rows<CPL, true>(xa, L, X, 1, C, lane, rows, Y->done, wa.smear, la.alpha);
+    } else {
+      lex_fill_rows<CPL>(xa, L, X, 1, C, lane);
+    }
   }
   float v[CPL], vn[CPL];
 #pragma unroll
@@ -580,10 +741,29 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
           L->lm[nr] = rows[pr * C + c];
           const int M = L->clen[pr];
           const int M1 = la.order - 1;
-          unsigned long long lo = (L->clo[pr] << 16) | static_cast<unsigned long long>(lm_tok(la, c) + 1);
-          unsigned long long hi = (L->chi[pr] << 16) | (L->clo[pr] >> 48);
-          lm_ctx_prefix(lo, hi, M1, lo, hi);
-          L->clo[nr] = lo; L->chi[nr] = hi; L->clen[nr] = min(M + 1, M1);
+          if constexpr (kPbWlm<Lex...>) {                     // a free class after a word end finishes that word
+            const PbWlmArgs wa = pb_wlm_args(lex...);
+            PbWlmWarp* Y = pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
+            const int pn = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->node[pr];
+            unsigned long long lo = L->clo[pr], hi = L->chi[pr];
+            int m = M;
+            if (lex_free(wa.lex, c)) {
+              Y->done[nr] = L->lm[nr];
+              if (pn != 0) {
+                lm_push<kWlmBits>(lo, hi, __ldg(wa.node_tok + pn), lo, hi);
+                lm_ctx_prefix<kWlmBits>(lo, hi, M1, lo, hi);
+                m = min(M + 1, M1);
+              }
+            } else {
+              Y->done[nr] = Y->done[pr];
+            }
+            L->clo[nr] = lo; L->chi[nr] = hi; L->clen[nr] = m;
+          } else {
+            unsigned long long lo = (L->clo[pr] << 16) | static_cast<unsigned long long>(lm_tok(la, c) + 1);
+            unsigned long long hi = (L->chi[pr] << 16) | (L->clo[pr] >> 48);
+            lm_ctx_prefix<16>(lo, hi, M1, lo, hi);
+            L->clo[nr] = lo; L->chi[nr] = hi; L->clen[nr] = min(M + 1, M1);
+          }
           L->nrow[q] = nr;
           L->row[cur ^ 1][lane] = nr;
         } else if constexpr (LEX) {                           // the same row pick without the LM's state
@@ -606,13 +786,22 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
     nb = nnew;
     cur ^= 1;
     if constexpr (LM || LEX) used = __reduce_or_sync(0xffffffffu, lane < nnew ? 1u << nr : 0u);
-    if constexpr (LM) {
+    if constexpr (LM && !kPbWlm<Lex...>) {
       if (em) {
         __syncwarp();
         lm_fill_rows(la, L, rows, __popc(em), C, unk, lane);
       }
     }
-    if constexpr (LEX) {
+    if constexpr (kPbWlm<Lex...>) {
+      if (em) {
+        __syncwarp();
+        const PbWlmArgs wa = pb_wlm_args(lex...);
+        PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
+        PbWlmWarp* Y = pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
+        wlm_fill_rows(la, wa, L, X, Y, rows, __popc(em), C, unk, lane);
+        lex_fill_rows<CPL, true>(wa.lex, L, X, __popc(em), C, lane, rows, Y->done, wa.smear, la.alpha);
+      }
+    } else if constexpr (LEX) {
       if (em) {
         __syncwarp();
         lex_fill_rows<CPL>(pb_lex_args(lex...), L, pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp),
@@ -633,7 +822,10 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
     long long mk = LLONG_MIN;
     if (lane < nb) {
       const int r = L->row[cur][lane];
-      fused = (g.tot[lane] + L->lm[r]) + L->eos[r];
+      if constexpr (kPbWlm<Lex...>)                       // (every survivor is between words or at a word end)
+        fused = (g.tot[lane] + pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->done[r]) + L->eos[r];
+      else
+        fused = (g.tot[lane] + L->lm[r]) + L->eos[r];
       mk = pb_key(fused);
     }
     int rank = 0;
@@ -670,16 +862,17 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
 }
 
 // Shared launcher: shared memory = per warp the beam state, the pool rows' state + the LM row pool (LM or LEX), the
-// lexicon state (LEX) and the node array; fewer warps per CTA above 200 KB.
-template <bool LM, bool LEX>
+// lexicon state (LEX), the word-LM state (XA = PbWlmArgs) and the node array; fewer warps per CTA above 200 KB.
+template <bool LM, bool LEX, typename XA = PbLexArgs>
 static int pb_launch(const float* log_probs, long long stride_b, long long stride_t, const int* lengths, int B, int T,
-                     int C, int K, int* ids, int* lens, double* scores, const PbLmArgs& la, const PbLexArgs& xa,
+                     int C, int K, int* ids, int* lens, double* scores, const PbLmArgs& la, const XA& xa,
                      cudaStream_t stream) {
+  constexpr bool WLM = std::is_same<XA, PbWlmArgs>::value;
   if (B <= 0 || T <= 0 || C <= 0 || !log_probs || !ids || !lens || !scores) return HTRVT_ERR_SHAPE;
   if (K < 1 || K > kPbMaxK || C > 32 * kPbCpl || static_cast<long long>(T) * K >= 65535) return HTRVT_ERR_SHAPE;
   int warps = 4;
   const size_t lm_bytes = ((LM || LEX) ? sizeof(PbLmWarp) : 0) + (LM ? sizeof(double) * 2 * K * C : 0) +
-                          (LEX ? sizeof(PbLexWarp) : 0);
+                          (LEX ? sizeof(PbLexWarp) : 0) + (WLM ? sizeof(PbWlmWarp) : 0);
   auto need = [&](int w) {
     return static_cast<size_t>(w) * (sizeof(PbWarp) + lm_bytes + (static_cast<size_t>(T) * K + 1) * 4);
   };
@@ -695,8 +888,8 @@ static int pb_launch(const float* log_probs, long long stride_b, long long strid
 #define PB_LAUNCH(CPL)                                                                                         \
   do {                                                                                                         \
     if constexpr (LEX) {                                                                                       \
-      PB_KERNEL(CPL, true, PbLexArgs);                                                                         \
-      ctc_prefix_beam_kernel<CPL, LM, true, PbLexArgs><<<grid, block, smem, stream>>>(                         \
+      PB_KERNEL(CPL, true, XA);                                                                                \
+      ctc_prefix_beam_kernel<CPL, LM, true, XA><<<grid, block, smem, stream>>>(                                \
           log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa);                     \
     } else {                                                                                                   \
       PB_KERNEL(CPL, false);                                                                                   \
@@ -730,6 +923,20 @@ static int pb_lm_args(const void* lm_table, long long lm_slots, int lm_order, co
   la.alpha = alpha;
   la.beta = beta;
   la.ctc_scores = ctc_scores;
+  return HTRVT_OK;
+}
+
+// The trie arguments of htrvt_ctc_prefix_beam_lex / _lex_wlm, checked for presence
+static int pb_lex_args_checked(const int* first, const int* label, const int* child, const unsigned char* word_end,
+                               int n_nodes, const unsigned char* is_word, int n_class_map, PbLexArgs& xa) {
+  if (!first || !label || !child || !word_end || n_nodes < 1) return HTRVT_ERR_SHAPE;
+  if (n_class_map < 0 || (n_class_map > 0 && !is_word)) return HTRVT_ERR_SHAPE;
+  xa.first = first;
+  xa.label = label;
+  xa.child = child;
+  xa.word_end = word_end;
+  xa.is_word = is_word;
+  xa.n_map = n_class_map;
   return HTRVT_OK;
 }
 
@@ -773,15 +980,9 @@ extern "C" int htrvt_ctc_prefix_beam_lex(const float* log_probs, long long strid
                                          const void* lm_table, long long lm_slots, int lm_order, const int* tok_map,
                                          int n_tok_map, double alpha, double beta, int* ids, int* lens,
                                          double* scores, double* ctc_scores, cudaStream_t stream) {
-  if (!first || !label || !child || !word_end || n_nodes < 1 || !ctc_scores) return HTRVT_ERR_SHAPE;
-  if (n_class_map < 0 || (n_class_map > 0 && !is_word)) return HTRVT_ERR_SHAPE;
   PbLexArgs xa;
-  xa.first = first;
-  xa.label = label;
-  xa.child = child;
-  xa.word_end = word_end;
-  xa.is_word = is_word;
-  xa.n_map = n_class_map;
+  const int sx = pb_lex_args_checked(first, label, child, word_end, n_nodes, is_word, n_class_map, xa);
+  if (sx != HTRVT_OK || !ctc_scores) return HTRVT_ERR_SHAPE;
   if (!lm_table) {
     if (alpha != 0.0 || beta != 0.0) return HTRVT_ERR_SHAPE;
     PbLmArgs la{};
@@ -793,4 +994,27 @@ extern "C" int htrvt_ctc_prefix_beam_lex(const float* log_probs, long long strid
   const int st = pb_lm_args(lm_table, lm_slots, lm_order, tok_map, n_tok_map, alpha, beta, ctc_scores, la);
   if (st != HTRVT_OK) return st;
   return pb_launch<true, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa, stream);
+}
+
+// The lexicon-constrained search with a word n-gram LM (header: include/htrvt.h).  Trie as htrvt_ctc_prefix_beam_lex;
+// lm_table as htrvt_ctc_prefix_beam_lm with 21-bit key fields (htr-vt_b200/wordlm.py packs it), lm_order 1..6;
+// node_tok int32 / smear float32 [n_nodes], not re-validated here.
+extern "C" int htrvt_ctc_prefix_beam_lex_wlm(const float* log_probs, long long stride_b, long long stride_t,
+                                             const int* lengths, int B, int T, int C, int K, const int* first,
+                                             const int* label, const int* child, const unsigned char* word_end,
+                                             int n_nodes, const unsigned char* is_word, int n_class_map,
+                                             const void* lm_table, long long lm_slots, int lm_order,
+                                             const int* node_tok, const float* smear, double alpha, double beta,
+                                             int* ids, int* lens, double* scores, double* ctc_scores,
+                                             cudaStream_t stream) {
+  PbWlmArgs wa;
+  if (pb_lex_args_checked(first, label, child, word_end, n_nodes, is_word, n_class_map, wa.lex) != HTRVT_OK)
+    return HTRVT_ERR_SHAPE;
+  if (!node_tok || !smear || lm_order > kWlmMaxOrder) return HTRVT_ERR_SHAPE;
+  wa.node_tok = node_tok;
+  wa.smear = smear;
+  PbLmArgs la;
+  const int st = pb_lm_args(lm_table, lm_slots, lm_order, nullptr, 0, alpha, beta, ctc_scores, la);
+  if (st != HTRVT_OK) return st;
+  return pb_launch<true, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, wa, stream);
 }

@@ -109,17 +109,19 @@ def lm_hash(lo, hi):
         return h ^ (h >> np.uint64(29))
 
 
-def pack_keys(tokens):
-    """tokens int [N, k] (token ids, first to last) -> (lo, hi) uint64 [N]: last token first, 16-bit fields of id + 1."""
+def pack_keys(tokens, bits=16):
+    """tokens int [N, k] (token ids, first to last) -> (lo, hi) uint64 [N]: last token first, bits-wide fields of
+    id + 1, 64 // bits of them per word (16: the character LM's 4 + 4 fields; 21: the word LM's 3 + 3)."""
     tokens = np.asarray(tokens, dtype=np.int64)
     N, k = tokens.shape
-    if k > MAX_ORDER or (tokens.size and (tokens.min() < 0 or tokens.max() > 0xFFFE)):
-        raise ValueError("n-gram keys hold at most 8 token ids in 0..65534")
+    per = 64 // bits
+    if k > 2 * per or (tokens.size and (tokens.min() < 0 or tokens.max() > (1 << bits) - 2)):
+        raise ValueError("n-gram keys hold at most %d token ids in 0..%d" % (2 * per, (1 << bits) - 2))
     lo = np.zeros(N, dtype=np.uint64)
     hi = np.zeros(N, dtype=np.uint64)
     for f in range(k):
-        v = (tokens[:, k - 1 - f] + 1).astype(np.uint64) << np.uint64(16 * (f % 4))
-        if f < 4:
+        v = (tokens[:, k - 1 - f] + 1).astype(np.uint64) << np.uint64(bits * (f % per))
+        if f < per:
             lo |= v
         else:
             hi |= v

@@ -8,6 +8,7 @@ import ctypes
 import torch
 
 from ._lib import HtrvtError, check, lib
+from .wordlm import WordNGramLM
 
 EPI_BF16, EPI_BIAS, _EPI_2, _EPI_3, EPI_ACCUM, EPI_STATS, _EPI_6, EPI_RELU = (1 << i for i in range(8))
 EPI_F16 = 1 << 10
@@ -399,6 +400,8 @@ def ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta=0.0, lengths=None, 
     CTC log-prob + sum of (alpha * ln10 * log10 p(label | context) + beta), survivors by that plus the </s> term.
     Returns (ids [B,K,T] int32, lens [B,K] int32, scores [B,K] float64 (fused), ctc_scores [B,K] float64), in fused
     order.  alpha = beta = 0 reproduces ctc_prefix_beam's ids, lens and scores bit for bit."""
+    if isinstance(lm, WordNGramLM):
+        raise ValueError("a word LM scores the words of a lexicon: use ctc_prefix_beam_lex")
     _need_cuda(log_probs)
     if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
         raise HtrvtError("ctc_prefix_beam_lm expects fp32 log-probs with a contiguous class axis")
@@ -427,9 +430,13 @@ def ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta=0.0, lengths=None, 
 def ctc_prefix_beam_lex(log_probs, beam_size, lexicon, lm=None, alpha=0.0, beta=0.0, lengths=None, layout="tbc"):
     """ctc_prefix_beam (lm=None; alpha = beta = 0) or ctc_prefix_beam_lm (lm: a CharNGramLM) constrained to a word
     lexicon (lexicon.py::Lexicon): every maximal run of word characters in a returned labelling is a lexicon word.
-    Ranking and scores are those of the unconstrained search; the lexicon only removes candidates.  Returns (ids
-    [B,K,T] int32, lens [B,K] int32 (-1 = no such labelling; all K when the line has no accepted labelling), scores
-    [B,K] float64 (fused; = ctc_scores without an LM), ctc_scores [B,K] float64)."""
+    Ranking and scores are those of the unconstrained search; the lexicon only removes candidates.  lm may instead be
+    a WordNGramLM built on this lexicon (wordlm.py): every finished word then adds alpha * ln10 * log10 p(word | <s>
+    previous words) + beta, the line's end the </s> term, and a word being spelled ranks with its smear term.  Returns
+    (ids [B,K,T] int32, lens [B,K] int32 (-1 = no such labelling; all K when the line has no accepted labelling),
+    scores [B,K] float64 (fused; = ctc_scores without an LM), ctc_scores [B,K] float64)."""
+    if isinstance(lm, WordNGramLM) and lm.lexicon is not lexicon:
+        raise ValueError("ctc_prefix_beam_lex: the word LM was built on another lexicon")
     _need_cuda(log_probs)
     if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
         raise HtrvtError("ctc_prefix_beam_lex expects fp32 log-probs with a contiguous class axis")
@@ -453,6 +460,14 @@ def ctc_prefix_beam_lex(log_probs, beam_size, lexicon, lm=None, alpha=0.0, beta=
     ctc_scores = torch.empty((B, K), dtype=torch.float64, device=dev)
     ln = None if lengths is None else lengths.to(device=dev, dtype=torch.int32).contiguous()
     lx = lexicon
+    if isinstance(lm, WordNGramLM):
+        check(lib().htrvt_ctc_prefix_beam_lex_wlm(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(lx.first),
+                                                  _p(lx.label), _p(lx.child), _p(lx.word_end), lx.n_nodes,
+                                                  _p(lx.is_word), lx.is_word.numel(), _p(lm.table), lm.slots, lm.order,
+                                                  _p(lm.node_tok), _p(lm.smear), float(alpha), float(beta), _p(ids),
+                                                  _p(lens), _p(scores), _p(ctc_scores), _stream()),
+              "htrvt_ctc_prefix_beam_lex_wlm")
+        return ids, lens, scores, ctc_scores
     lm_args = ((None, 0, 0, None, 0) if lm is None else
                (lm.table, lm.slots, lm.order, lm.token_map, lm.token_map.numel()))
     check(lib().htrvt_ctc_prefix_beam_lex(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(lx.first), _p(lx.label),

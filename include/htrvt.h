@@ -134,6 +134,27 @@ int htrvt_ctc_prefix_beam_lex(const float* log_probs, long long stride_b, long l
                               const int* tok_map, int n_tok_map, double alpha, double beta, int* ids, int* lens,
                               double* scores, double* ctc_scores, void* stream);
 
+/* ---- CTC prefix beam search constrained to a word lexicon, with a fused word n-gram LM -------------------------
+ * htrvt_ctc_prefix_beam_lex_wlm is htrvt_ctc_prefix_beam_lex (same trie arguments, same constraint) whose LM scores
+ * WORDS (Scheidl et al. 2018, "Word Beam Search", "NGrams" mode): the tokens of a labelling are its maximal runs of
+ * word characters; free characters are no tokens.  For words w_1 .. w_m the fused score is
+ * lae(pb, pnb) + sum_i [alpha * ln10 * log10 p(w_i | <s> w_1 .. w_i-1) + beta] + alpha * ln10 * log10 p(</s> | <s>
+ * w_1 .. w_m), ARPA backoff as htrvt_ctc_prefix_beam_lm.  An entry inside a word at trie node n ranks with
+ * alpha * ln10 * smear[n] added (no such term between words); the returned scores carry no smear term, and the
+ * survivors are re-ranked stably by them.  lm_table as htrvt_ctc_prefix_beam_lm with 21-bit key fields (token + 1,
+ * three per 64-bit word: lo fields 0-2, hi fields 3-5; the layout htr-vt_b200/wordlm.py packs), lm_order 1..6;
+ * token ids <unk> = 0, <s> = 1, </s> = 2; node_tok int32 [n_nodes]: the token of the word ending at each node (read
+ * at word ends only); smear float32 [n_nodes]: the largest unigram log10 prob of the lexicon words that start with
+ * the node's prefix.  ids / lens / scores / ctc_scores as htrvt_ctc_prefix_beam_lex.  HTRVT_ERR_SHAPE: a null trie
+ * array, node_tok or smear, n_nodes < 1, non-finite alpha or beta, lm_order outside 1..6, a slot count that is not a
+ * power of two, or the limits of htrvt_ctc_prefix_beam (K <= 16, C <= 256, T * K < 65535). */
+int htrvt_ctc_prefix_beam_lex_wlm(const float* log_probs, long long stride_b, long long stride_t, const int* lengths,
+                                  int B, int T, int C, int K, const int* first, const int* label, const int* child,
+                                  const unsigned char* word_end, int n_nodes, const unsigned char* is_word,
+                                  int n_class_map, const void* lm_table, long long lm_slots, int lm_order,
+                                  const int* node_tok, const float* smear, double alpha, double beta, int* ids,
+                                  int* lens, double* scores, double* ctc_scores, void* stream);
+
 /* ---- CTC forced alignment of a known transcription -----------------------------------------------------------
  * htrvt_ctc_align: the single best path (Viterbi) through the CTC trellis of each line's labels, blank = 0, with the
  * frames each label occupies: the alignment torchaudio.functional.forced_align computes one line at a time on the host.
