@@ -102,28 +102,32 @@ def simple_ctc_beam_search_with_lm(log_probs, converter, lm_scorer, beam_size=5,
     return _pick(kbest_candidates(lp, converter, beam_size, search=search)[0], lm_scorer)
 
 
+def _batch_log_probs(preds_log, name):
+    """preds_log on the GPU as fp32 with a contiguous class axis."""
+    if not preds_log.is_cuda:
+        raise ops.HtrvtError("%s needs a CUDA tensor (no CPU fallback)" % name)
+    lp = preds_log.float()
+    return lp if lp.stride(-1) == 1 else lp.contiguous()
+
+
+def _best_strings(ids, lens, converter):
+    """The best-ranked labelling of every line of a prefix search's (ids, lens) as a string."""
+    return _candidate_strings(ids[:, 0].cpu().numpy(), np.maximum(lens[:, 0].cpu().numpy(), 0), converter,
+                              merge_repeats=False)
+
+
 def beam_search_with_lm_batch(preds_log, converter, lm_scorer, beam_size=5, lengths=None, search="paths"):
     """preds_log [T, B, C] (validation_with_kenlm's `preds_log`) -> list of B strings: one kernel, one D2H copy."""
-    if not preds_log.is_cuda:
-        raise ops.HtrvtError("beam_search_with_lm_batch needs a CUDA tensor (no CPU fallback)")
-    lp = preds_log.float()
-    if lp.stride(-1) != 1:
-        lp = lp.contiguous()
+    lp = _batch_log_probs(preds_log, "beam_search_with_lm_batch")
     return [_pick(c, lm_scorer) for c in kbest_candidates(lp, converter, beam_size, lengths, search=search)]
 
 
 def ctc_lm_decode(preds_log, converter, lm, alpha, beta=0.0, beam_size=8, lengths=None):
     """preds_log [T, B, C] (validation_with_kenlm's layout) -> B strings: the best-ranked labelling of the LM-fused CTC
     prefix beam search per line ("" when that is the empty labelling).  lm: CharNGramLM on the same device."""
-    if not preds_log.is_cuda:
-        raise ops.HtrvtError("ctc_lm_decode needs a CUDA tensor (no CPU fallback)")
-    lp = preds_log.float()
-    if lp.stride(-1) != 1:
-        lp = lp.contiguous()
+    lp = _batch_log_probs(preds_log, "ctc_lm_decode")
     ids, lens, _, _ = ops.ctc_prefix_beam_lm(lp, beam_size, lm, alpha, beta, lengths, "tbc")
-    best_ids = ids[:, 0].cpu().numpy()
-    best_lens = np.maximum(lens[:, 0].cpu().numpy(), 0)
-    return _candidate_strings(best_ids, best_lens, converter, merge_repeats=False)
+    return _best_strings(ids, lens, converter)
 
 
 def ctc_lexicon_decode(preds_log, converter, lexicon, beam_size=8, lengths=None, lm=None, alpha=0.0, beta=0.0):
@@ -132,12 +136,6 @@ def ctc_lexicon_decode(preds_log, converter, lexicon, beam_size=8, lengths=None,
     when given ("" for the empty labelling, and for a line with no accepted labelling).  lm: a CharNGramLM (score =
     CTC log-prob + alpha * ln(10) * log10 P(string </s>) + beta * len) or a WordNGramLM built on lexicon (score = CTC
     log-prob + alpha * ln(10) * log10 P(w_1 .. w_m </s>) + beta * m over the string's m words)."""
-    if not preds_log.is_cuda:
-        raise ops.HtrvtError("ctc_lexicon_decode needs a CUDA tensor (no CPU fallback)")
-    lp = preds_log.float()
-    if lp.stride(-1) != 1:
-        lp = lp.contiguous()
+    lp = _batch_log_probs(preds_log, "ctc_lexicon_decode")
     ids, lens, _, _ = ops.ctc_prefix_beam_lex(lp, beam_size, lexicon, lm, alpha, beta, lengths, "tbc")
-    best_ids = ids[:, 0].cpu().numpy()
-    best_lens = np.maximum(lens[:, 0].cpu().numpy(), 0)
-    return _candidate_strings(best_ids, best_lens, converter, merge_repeats=False)
+    return _best_strings(ids, lens, converter)

@@ -45,7 +45,6 @@
 // the word ending at its node and the </s> term after it.
 #include "common.cuh"
 #include <climits>
-#include <type_traits>
 
 namespace htrvt {
 
@@ -105,10 +104,9 @@ struct PbLexWarp {                  // lexicon state of one line; per pool row (
 };
 
 // Word n-gram LM over the lexicon's trie (htr-vt_b200/wordlm.py packs it); the table, order and weights come in
-// PbLmArgs (tok_map unused).  node_tok: trie node -> token id of the word ending there; smear: trie node -> the largest
-// unigram log10 prob of the lexicon words that start with the node's prefix.
+// PbLmArgs (tok_map unused), the trie in PbLexArgs.  node_tok: trie node -> token id of the word ending there; smear:
+// trie node -> the largest unigram log10 prob of the lexicon words that start with the node's prefix.
 struct PbWlmArgs {
-  PbLexArgs lex;
   const int* node_tok;
   const float* smear;
 };
@@ -203,11 +201,42 @@ __device__ __forceinline__ void lm_push(unsigned long long lo, unsigned long lon
 }
 __device__ __forceinline__ int lm_tok(const PbLmArgs& a, int c) { return c < a.n_map ? __ldg(a.tok_map + c) : kLmUnk; }
 
+// log10 p(w | context) by ARPA backoff over the levels m = M .. 0 of one query, whose first slots are already loaded
+// (level m: key (klo[m], khi[m]) = (last m context tokens, w), first slot ix[m] with key s[m] and prob p[m]): the listed
+// prob of the longest level in the table, plus the bow of every longer level's context, summed in float64
+// longest-context bow first and the found prob last; unk when no level is listed.  add_bow(m, S) adds level m's
+// context bow (0 when that context is unlisted) to S.
+template <int N, typename AddBow>
+__device__ __forceinline__ double lm_backoff(const PbLmArgs& a, const unsigned long long* klo,
+                                             const unsigned long long* khi, const unsigned long long* ix,
+                                             const ulonglong2* s, const float* p, int M, float unk, AddBow add_bow) {
+  double S = 0.0;
+  bool found = false;
+#pragma unroll
+  for (int m = N - 1; m >= 0; --m) {
+    if (m <= M && !found) {
+      if (s[m].x == klo[m] && s[m].y == khi[m]) {
+        S += static_cast<double>(p[m]);
+        found = true;
+      } else {
+        const long long f = s[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, klo[m], khi[m], ix[m], s[m]);
+        if (f >= 0) {
+          S += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(f)).x);
+          found = true;
+        } else if (m > 0) {
+          add_bow(m, S);
+        }
+      }
+    }
+  }
+  if (!found) S += static_cast<double>(unk);
+  return S;
+}
+
 // Fill the rows L->nrow[0 .. nE) (their lm / context already set): row[c] = lm + alpha ln10 S(c) + beta for every label
-// c, eos = alpha ln10 S(</s>), with S(w) = log10 p(w | context) by ARPA backoff: the listed prob of the longest
-// (context suffix, w), plus the bows of the longer context suffixes, summed in float64 longest-context bow first and the
-// found prob last (the unigram level falls back to <unk>'s prob).  All 32 lanes, (row, class) pairs spread over lanes;
-// a lane issues the first-slot loads of every level of its query before it looks at any of them.
+// c, eos = alpha ln10 S(</s>), with S(w) = log10 p(w | context) (lm_backoff; the context bows are looked up first, once
+// per row).  All 32 lanes, (row, class) pairs spread over lanes; a lane issues the first-slot loads of every level of
+// its query before it looks at any of them.
 __device__ __forceinline__ void lm_fill_rows(const PbLmArgs& a, PbLmWarp* L, double* rows, int nE, int C, float unk,
                                           int lane) {
   const int M1 = a.order - 1;
@@ -254,26 +283,9 @@ __device__ __forceinline__ void lm_fill_rows(const PbLmArgs& a, PbLmWarp* L, dou
         p[m] = lm_val_at(a.table, ix[m]).x;
       }
     }
-    double S = 0.0;
-    bool found = false;
-#pragma unroll
-    for (int m = kLmMaxOrder - 1; m >= 0; --m) {
-      if (m <= M && !found) {
-        if (s[m].x == klo[m] && s[m].y == khi[m]) {
-          S += static_cast<double>(p[m]);
-          found = true;
-        } else {
-          const long long f = s[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, klo[m], khi[m], ix[m], s[m]);
-          if (f >= 0) {
-            S += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(f)).x);
-            found = true;
-          } else if (m > 0) {
-            S += static_cast<double>(L->bow[e][m - 1]);
-          }
-        }
-      }
-    }
-    if (!found) S += static_cast<double>(unk);
+    const double S = lm_backoff<kLmMaxOrder>(a, klo, khi, ix, s, p, M, unk, [&](int m, double& sum) {
+      sum += static_cast<double>(L->bow[e][m - 1]);
+    });
     const double t = __dmul_rn(a.alpha, __dmul_rn(kLn10, S));   // no contraction: the oracle's arithmetic
     if (c < 0) L->eos[r] = t;
     else rows[r * C + c] = __dadd_rn(L->lm[r], __dadd_rn(t, a.beta));
@@ -288,10 +300,10 @@ __device__ __forceinline__ bool lex_free(const PbLexArgs& a, int c) { return c >
 // free class leads back to state 0, which both masks accept; a child edge c leads to the child, which allow_last
 // accepts only when the child ends a word.  All 32 lanes: first the free-class part word by word, then the child edges.
 // WLM: the child edges' LM row entries too, done + alpha ln10 smear(child) (the other classes are already filled).
-template <int CPL, bool WLM = false>
+template <int CPL, bool WLM>
 __device__ __forceinline__ void lex_fill_rows(const PbLexArgs& a, const PbLmWarp* L, PbLexWarp* X, int nE, int C,
-                                              int lane, double* rows = nullptr, const double* done = nullptr,
-                                              const float* smear = nullptr, double alpha = 0.0) {
+                                              int lane, double* rows, const double* done, const float* smear,
+                                              double alpha) {
   for (int idx = lane; idx < nE * CPL; idx += 32) {
     const int e = idx / CPL, w = idx - e * CPL;
     const int r = L->nrow[e];
@@ -332,9 +344,8 @@ __device__ __forceinline__ int lex_step(const PbLexArgs& a, int n, int c) {
 }
 
 // ---- word n-gram LM -------------------------------------------------------------------------------------------------
-// log10 p(tok | context) by ARPA backoff (the arithmetic of lm_fill_rows) for one query in one lane: context (clo, chi)
-// of M <= kWlmMaxOrder - 1 tokens; the first slots of every level's n-gram key and context key are loaded before any
-// of them is looked at.
+// log10 p(tok | context) (lm_backoff) for one query in one lane: context (clo, chi) of M <= kWlmMaxOrder - 1 tokens;
+// the first slots of every level's n-gram key and context key are loaded before any of them is looked at.
 __device__ __forceinline__ double wlm_logprob(const PbLmArgs& a, unsigned long long clo, unsigned long long chi, int M,
                                               int tok, float unk) {
   unsigned long long klo[kWlmMaxOrder], khi[kWlmMaxOrder], ix[kWlmMaxOrder];
@@ -356,32 +367,14 @@ __device__ __forceinline__ double wlm_logprob(const PbLmArgs& a, unsigned long l
       }
     }
   }
-  double S = 0.0;
-  bool found = false;
-#pragma unroll
-  for (int m = kWlmMaxOrder - 1; m >= 0; --m) {
-    if (m <= M && !found) {
-      if (s[m].x == klo[m] && s[m].y == khi[m]) {
-        S += static_cast<double>(p[m]);
-        found = true;
-      } else {
-        const long long f = s[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, klo[m], khi[m], ix[m], s[m]);
-        if (f >= 0) {
-          S += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(f)).x);
-          found = true;
-        } else if (m > 0) {                                  // the context's bow, 0 when it is not listed
-          if (bs[m].x == blo[m] && bs[m].y == bhi[m]) {
-            S += static_cast<double>(bw[m]);
-          } else {
-            const long long g = bs[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, blo[m], bhi[m], bix[m], bs[m]);
-            if (g >= 0) S += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(g)).y);
-          }
-        }
-      }
+  return lm_backoff<kWlmMaxOrder>(a, klo, khi, ix, s, p, M, unk, [&](int m, double& sum) {
+    if (bs[m].x == blo[m] && bs[m].y == bhi[m]) {
+      sum += static_cast<double>(bw[m]);
+    } else {
+      const long long g = bs[m].x == 0ull ? -1 : lm_walk(a.table, a.mask, blo[m], bhi[m], bix[m], bs[m]);
+      if (g >= 0) sum += static_cast<double>(lm_val_at(a.table, static_cast<unsigned long long>(g)).y);
     }
-  }
-  if (!found) S += static_cast<double>(unk);
-  return S;
+  });
 }
 
 // Fill the word-LM rows L->nrow[0 .. nE) (node / fin, done and context already set), before lex_fill_rows<CPL, true>
@@ -429,49 +422,48 @@ __device__ __forceinline__ void wlm_fill_rows(const PbLmArgs& a, const PbWlmArgs
   __syncwarp();
 }
 
-// the lexicon pack of the word-LM instantiation
-template <typename... Lex>
-constexpr bool kPbWlm = false;
-template <>
-constexpr bool kPbWlm<PbWlmArgs> = true;
-
-__device__ __forceinline__ PbLexArgs pb_lex_args(const PbLexArgs& a) { return a; }
-__device__ __forceinline__ PbLexArgs pb_lex_args(const PbWlmArgs& a) { return a.lex; }
-__device__ __forceinline__ PbWlmArgs pb_wlm_args(const PbWlmArgs& a) { return a; }
-// a warp's lexicon state: after `front` bytes per warp (its beam state, pool rows' state and LM row pool)
-__device__ __forceinline__ PbLexWarp* pb_lex_warp(uint8_t* smem, size_t front, int warps, int warp) {
-  return reinterpret_cast<PbLexWarp*>(smem + front * warps) + warp;
+// Shared memory of a CTA of `warps` lines: the byte offset of each region and the total.  Region-major over the warps,
+// in this order: PbWarp; PbLmWarp (LM or LEX: the pool rows' bookkeeping); the LM row pool, 2K rows of C doubles (LM);
+// PbLexWarp (LEX); PbWlmWarp (WLM); the node array, T K + 1 entries.  A region starts at warps times the per-warp bytes
+// of the regions before it.  The launcher sizes the launch with it and the kernel finds its warp's state with it.
+struct PbSmem {
+  size_t lm, rows, lex, wlm, nodes, bytes;
+};
+__host__ __device__ __forceinline__ PbSmem pb_smem_layout(bool LM, bool LEX, bool WLM, int K, int C, int T, int warps) {
+  // (the pool rows' bytes summed first: ptxas schedules the LM kernels' prologue by the grouping of these sums)
+  const size_t pool = (LM || LEX) ? sizeof(PbLmWarp) + (LM ? sizeof(double) * 2 * K * C : 0) : 0;
+  const size_t lm = sizeof(PbWarp);
+  const size_t rows = lm + ((LM || LEX) ? sizeof(PbLmWarp) : 0);
+  const size_t lex = lm + pool;
+  const size_t wlm = lex + (LEX ? sizeof(PbLexWarp) : 0);
+  const size_t nodes = wlm + (WLM ? sizeof(PbWlmWarp) : 0);
+  const size_t bytes = nodes + (static_cast<size_t>(T) * K + 1) * 4;
+  return {lm * warps, rows * warps, lex * warps, wlm * warps, nodes * warps, bytes * warps};
 }
-// a warp's word-LM state: after the lexicon states
-__device__ __forceinline__ PbWlmWarp* pb_wlm_warp(uint8_t* smem, size_t front, int warps, int warp) {
-  return reinterpret_cast<PbWlmWarp*>(smem + (front + sizeof(PbLexWarp)) * warps) + warp;
-}
 
-// class slots per lane: C <= 32 * CPL; LM: fused n-gram LM; LEX: word lexicon constraint, whose PbLexArgs come in the
-// pack Lex.  With LEX off the pack is empty and every lexicon variable lives inside `if constexpr (LEX)`, so that the
-// plain and LM kernels keep their parameter list and compile to the same code as before the lexicon.  LM and LEX with
-// a PbWlmArgs in the pack (kPbWlm): the LM is the word LM, every character-LM step inside `if constexpr (!kPbWlm)`.
+// class slots per lane: C <= 32 * CPL; LM: fused n-gram LM; LEX: word lexicon constraint; WLM (with LM and LEX): the
+// LM is the word LM, every character-LM step inside `if constexpr (!WLM)`.  Every instantiation takes the three
+// argument structs; a variant leaves those it does not use zero-filled, and every state it does not use is touched
+// only inside `if constexpr` on its flag.
 // (Min. blocks 1 for LEX: without it ptxas caps some lexicon instantiations at 56-128 registers and spills.)
-template <int CPL, bool LM, bool LEX, typename... Lex>
+template <int CPL, bool LM, bool LEX, bool WLM>
 __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const float* __restrict__ x, long long sb, long long st,
                                                               const int* __restrict__ lengths, int B, int T, int C,
                                                               int K, int* __restrict__ ids, int* __restrict__ lens,
-                                                              double* __restrict__ scores, PbLmArgs la, Lex... lex) {
-  static_assert(sizeof...(Lex) == (LEX ? 1 : 0), "LEX takes one PbLexArgs or PbWlmArgs");
+                                                              double* __restrict__ scores, PbLmArgs la, PbLexArgs xa,
+                                                              PbWlmArgs wa) {
+  static_assert(!WLM || (LM && LEX), "the word LM runs inside the lexicon-constrained LM search");
   extern __shared__ __align__(16) uint8_t pb_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
   const int b = blockIdx.x * warps + warp;
   if (b >= B) return;
   PbWarp* W = reinterpret_cast<PbWarp*>(pb_smem) + warp;
-  // per warp: PbWarp | PbLmWarp (LM or LEX: the pool rows' bookkeeping) + the LM row pool (LM) | PbLexWarp (LEX) |
-  // PbWlmWarp (word LM) | nodes
-  const size_t lm_bytes = (LM || LEX) ? sizeof(PbLmWarp) + (LM ? sizeof(double) * 2 * K * C : 0) : 0;
-  PbLmWarp* L = reinterpret_cast<PbLmWarp*>(pb_smem + sizeof(PbWarp) * warps) + warp;
-  double* rows = reinterpret_cast<double*>(pb_smem + (sizeof(PbWarp) + sizeof(PbLmWarp)) * warps) +
-                 static_cast<size_t>(warp) * 2 * K * C;
-  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + (sizeof(PbWarp) + lm_bytes + (LEX ? sizeof(PbLexWarp) : 0) +
-                                                           (kPbWlm<Lex...> ? sizeof(PbWlmWarp) : 0)) *
-                                                           warps) +
+  const PbSmem sm = pb_smem_layout(LM, LEX, WLM, K, C, T, warps);
+  PbLmWarp* L = reinterpret_cast<PbLmWarp*>(pb_smem + sm.lm) + warp;
+  double* rows = reinterpret_cast<double*>(pb_smem + sm.rows) + static_cast<size_t>(warp) * 2 * K * C;
+  PbLexWarp* X = reinterpret_cast<PbLexWarp*>(pb_smem + sm.lex) + warp;
+  PbWlmWarp* Y = reinterpret_cast<PbWlmWarp*>(pb_smem + sm.wlm) + warp;
+  uint32_t* nodes = reinterpret_cast<uint32_t*>(pb_smem + sm.nodes) +
                     static_cast<size_t>(warp) * (static_cast<size_t>(T) * K + 1);
   int Tb = lengths ? lengths[b] : T;
   Tb = min(max(Tb, 0), T);
@@ -496,14 +488,12 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
       L->clen[0] = min(1, la.order - 1);
       L->clo[0] = la.order > 1 ? static_cast<unsigned long long>(kLmBos + 1) : 0ull;
       L->chi[0] = 0ull;
-      if constexpr (kPbWlm<Lex...>) pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->done[0] = 0.0;
+      if constexpr (WLM) Y->done[0] = 0.0;
     }
     __syncwarp();
-    if constexpr (!kPbWlm<Lex...>) lm_fill_rows(la, L, rows, 1, C, unk, lane);
+    if constexpr (!WLM) lm_fill_rows(la, L, rows, 1, C, unk, lane);
   }
   if constexpr (LEX) {
-    const PbLexArgs xa = pb_lex_args(lex...);
-    PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
 #pragma unroll
     for (int u = 0; u < CPL; ++u) {
       const int c = lane + 32 * u;
@@ -515,14 +505,8 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
       X->node[0] = 0; X->fin[0] = 1;
     }
     __syncwarp();
-    if constexpr (kPbWlm<Lex...>) {
-      const PbWlmArgs wa = pb_wlm_args(lex...);
-      PbWlmWarp* Y = pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
-      wlm_fill_rows(la, wa, L, X, Y, rows, 1, C, unk, lane);
-      lex_fill_rows<CPL, true>(xa, L, X, 1, C, lane, rows, Y->done, wa.smear, la.alpha);
-    } else {
-      lex_fill_rows<CPL>(xa, L, X, 1, C, lane);
-    }
+    if constexpr (WLM) wlm_fill_rows(la, wa, L, X, Y, rows, 1, C, unk, lane);
+    lex_fill_rows<CPL, WLM>(xa, L, X, 1, C, lane, rows, Y->done, wa.smear, la.alpha);
   }
   float v[CPL], vn[CPL];
 #pragma unroll
@@ -588,7 +572,6 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
       }
     }
     if constexpr (LEX) {                                  // the extensions the lexicon forbids join the folded ones
-      const PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
       const bool last = t + 1 == Tb;
       for (int i = 0; i < nb; ++i) {
         const int r = L->row[cur][i];
@@ -615,8 +598,7 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
       for (int u = 0; u < CPL; ++u) { bku[u] = LLONG_MIN; bnu[u] = 0x7fffffff; }
       bool stay = lane < nb;
       if constexpr (LEX)                                  // last frame: no stay inside an unfinished word
-        stay = stay &&
-               (t + 1 < Tb || pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->fin[L->row[cur][lane]]);
+        stay = stay && (t + 1 < Tb || X->fin[L->row[cur][lane]]);
       if (stay) { bku[0] = pb_key(LM ? L->skey[lane] : W->stot[lane]); bnu[0] = lane; }
 #pragma unroll 4
       for (int i = 0; i < nb; ++i) {
@@ -669,8 +651,7 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
         if (idx == M) {                                       // the owner's stay candidate
           ok = own < nb;
           if constexpr (LEX)                              // left out: a LLONG_MIN key would still beat the sentinel
-            ok = ok &&
-                 (t + 1 < Tb || pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->fin[L->row[cur][own]]);
+            ok = ok && (t + 1 < Tb || X->fin[L->row[cur][own]]);
           k = ok ? pb_key(LM ? L->skey[own] : W->stot[own]) : LLONG_MIN;
           n = own;
         } else {
@@ -733,21 +714,21 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
         gn.pb[lane] = -INFINITY; gn.pnb[lane] = s; gn.tot[lane] = s;
         gn.hash[lane] = pb_hash(g.hash[pi], c); gn.phash[lane] = g.hash[pi];
         gn.last[lane] = c; gn.len[lane] = g.len[pi] + 1; gn.node[lane] = nd;
-        if constexpr (LM) {                                   // a free row (not held by generation cur), q-th of them
+        if constexpr (LM || LEX) {                            // a free row (not held by generation cur), q-th of them
           unsigned fr = ~used & (K == 16 ? 0xffffffffu : (1u << (2 * K)) - 1u);
           for (int z = 0; z < q; ++z) fr &= fr - 1u;
           nr = __ffs(fr) - 1;
+        }
+        if constexpr (LM) {
           const int pr = L->row[cur][pi];
           L->lm[nr] = rows[pr * C + c];
           const int M = L->clen[pr];
           const int M1 = la.order - 1;
-          if constexpr (kPbWlm<Lex...>) {                     // a free class after a word end finishes that word
-            const PbWlmArgs wa = pb_wlm_args(lex...);
-            PbWlmWarp* Y = pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
-            const int pn = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->node[pr];
+          if constexpr (WLM) {                                // a free class after a word end finishes that word
+            const int pn = X->node[pr];
             unsigned long long lo = L->clo[pr], hi = L->chi[pr];
             int m = M;
-            if (lex_free(wa.lex, c)) {
+            if (lex_free(xa, c)) {
               Y->done[nr] = L->lm[nr];
               if (pn != 0) {
                 lm_push<kWlmBits>(lo, hi, __ldg(wa.node_tok + pn), lo, hi);
@@ -764,18 +745,12 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
             lm_ctx_prefix<16>(lo, hi, M1, lo, hi);
             L->clo[nr] = lo; L->chi[nr] = hi; L->clen[nr] = min(M + 1, M1);
           }
-          L->nrow[q] = nr;
-          L->row[cur ^ 1][lane] = nr;
-        } else if constexpr (LEX) {                           // the same row pick without the LM's state
-          unsigned fr = ~used & (K == 16 ? 0xffffffffu : (1u << (2 * K)) - 1u);
-          for (int z = 0; z < q; ++z) fr &= fr - 1u;
-          nr = __ffs(fr) - 1;
+        }
+        if constexpr (LM || LEX) {                            // after the LM's row state (keeps the LM kernels' code)
           L->nrow[q] = nr;
           L->row[cur ^ 1][lane] = nr;
         }
         if constexpr (LEX) {
-          const PbLexArgs xa = pb_lex_args(lex...);
-          PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
           const int nn = lex_step(xa, X->node[L->row[cur][pi]], c);
           X->node[nr] = nn;
           X->fin[nr] = nn == 0 || __ldg(xa.word_end + nn);
@@ -786,26 +761,17 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
     nb = nnew;
     cur ^= 1;
     if constexpr (LM || LEX) used = __reduce_or_sync(0xffffffffu, lane < nnew ? 1u << nr : 0u);
-    if constexpr (LM && !kPbWlm<Lex...>) {
+    if constexpr (LM && !WLM) {
       if (em) {
         __syncwarp();
         lm_fill_rows(la, L, rows, __popc(em), C, unk, lane);
       }
     }
-    if constexpr (kPbWlm<Lex...>) {
+    if constexpr (LEX) {
       if (em) {
         __syncwarp();
-        const PbWlmArgs wa = pb_wlm_args(lex...);
-        PbLexWarp* X = pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
-        PbWlmWarp* Y = pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp);
-        wlm_fill_rows(la, wa, L, X, Y, rows, __popc(em), C, unk, lane);
-        lex_fill_rows<CPL, true>(wa.lex, L, X, __popc(em), C, lane, rows, Y->done, wa.smear, la.alpha);
-      }
-    } else if constexpr (LEX) {
-      if (em) {
-        __syncwarp();
-        lex_fill_rows<CPL>(pb_lex_args(lex...), L, pb_lex_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp),
-                           __popc(em), C, lane);
+        if constexpr (WLM) wlm_fill_rows(la, wa, L, X, Y, rows, __popc(em), C, unk, lane);
+        lex_fill_rows<CPL, WLM>(xa, L, X, __popc(em), C, lane, rows, Y->done, wa.smear, la.alpha);
       }
     }
 #pragma unroll
@@ -822,8 +788,8 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
     long long mk = LLONG_MIN;
     if (lane < nb) {
       const int r = L->row[cur][lane];
-      if constexpr (kPbWlm<Lex...>)                       // (every survivor is between words or at a word end)
-        fused = (g.tot[lane] + pb_wlm_warp(pb_smem, sizeof(PbWarp) + lm_bytes, warps, warp)->done[r]) + L->eos[r];
+      if constexpr (WLM)                                  // (every survivor is between words or at a word end)
+        fused = (g.tot[lane] + Y->done[r]) + L->eos[r];
       else
         fused = (g.tot[lane] + L->lm[r]) + L->eos[r];
       mk = pb_key(fused);
@@ -851,51 +817,29 @@ __global__ void __launch_bounds__(128, LEX ? 1 : 0) ctc_prefix_beam_kernel(const
     }
     for (int p = n; p < T; ++p) out[p] = 0;
     lens[b * K + slot] = live ? n : -1;
-    if constexpr (LM) {
-      scores[b * K + slot] = live ? fused : -INFINITY;
-      la.ctc_scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
-    } else {
-      scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
-      if constexpr (LEX) la.ctc_scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
-    }
+    scores[b * K + slot] = live ? (LM ? fused : g.tot[lane]) : -INFINITY;
+    if constexpr (LM || LEX) la.ctc_scores[b * K + slot] = live ? g.tot[lane] : -INFINITY;
   }
 }
 
-// Shared launcher: shared memory = per warp the beam state, the pool rows' state + the LM row pool (LM or LEX), the
-// lexicon state (LEX), the word-LM state (XA = PbWlmArgs) and the node array; fewer warps per CTA above 200 KB.
-template <bool LM, bool LEX, typename XA = PbLexArgs>
+// Shared launcher: shared memory as pb_smem_layout; fewer warps per CTA above 200 KB.
+template <bool LM, bool LEX, bool WLM>
 static int pb_launch(const float* log_probs, long long stride_b, long long stride_t, const int* lengths, int B, int T,
-                     int C, int K, int* ids, int* lens, double* scores, const PbLmArgs& la, const XA& xa,
-                     cudaStream_t stream) {
-  constexpr bool WLM = std::is_same<XA, PbWlmArgs>::value;
+                     int C, int K, int* ids, int* lens, double* scores, const PbLmArgs& la, const PbLexArgs& xa,
+                     const PbWlmArgs& wa, cudaStream_t stream) {
   if (B <= 0 || T <= 0 || C <= 0 || !log_probs || !ids || !lens || !scores) return HTRVT_ERR_SHAPE;
   if (K < 1 || K > kPbMaxK || C > 32 * kPbCpl || static_cast<long long>(T) * K >= 65535) return HTRVT_ERR_SHAPE;
   int warps = 4;
-  const size_t lm_bytes = ((LM || LEX) ? sizeof(PbLmWarp) : 0) + (LM ? sizeof(double) * 2 * K * C : 0) +
-                          (LEX ? sizeof(PbLexWarp) : 0) + (WLM ? sizeof(PbWlmWarp) : 0);
-  auto need = [&](int w) {
-    return static_cast<size_t>(w) * (sizeof(PbWarp) + lm_bytes + (static_cast<size_t>(T) * K + 1) * 4);
-  };
-  while (warps > 1 && need(warps) > 200 * 1024) warps >>= 1;
-  const size_t smem = need(warps);
+  while (warps > 1 && pb_smem_layout(LM, LEX, WLM, K, C, T, warps).bytes > 200 * 1024) warps >>= 1;
+  const size_t smem = pb_smem_layout(LM, LEX, WLM, K, C, T, warps).bytes;
   if (smem > 227 * 1024) return HTRVT_ERR_SHAPE;
   const dim3 grid((B + warps - 1) / warps), block(warps * 32);
-#define PB_KERNEL(CPL, ...)                                                                                    \
-  do {                                                                                                         \
-    if (smem > 48 * 1024 && !HTRVT_ENSURE_SMEM((ctc_prefix_beam_kernel<CPL, LM, __VA_ARGS__>), 227 * 1024))   \
-      return HTRVT_ERR_LAUNCH;                                                                                 \
-  } while (0)
 #define PB_LAUNCH(CPL)                                                                                         \
   do {                                                                                                         \
-    if constexpr (LEX) {                                                                                       \
-      PB_KERNEL(CPL, true, XA);                                                                                \
-      ctc_prefix_beam_kernel<CPL, LM, true, XA><<<grid, block, smem, stream>>>(                                \
-          log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa);                     \
-    } else {                                                                                                   \
-      PB_KERNEL(CPL, false);                                                                                   \
-      ctc_prefix_beam_kernel<CPL, LM, false><<<grid, block, smem, stream>>>(                                   \
-          log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la);                         \
-    }                                                                                                          \
+    if (smem > 48 * 1024 && !HTRVT_ENSURE_SMEM((ctc_prefix_beam_kernel<CPL, LM, LEX, WLM>), 227 * 1024))      \
+      return HTRVT_ERR_LAUNCH;                                                                                 \
+    ctc_prefix_beam_kernel<CPL, LM, LEX, WLM><<<grid, block, smem, stream>>>(                                  \
+        log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa, wa);                   \
   } while (0)
   if (C <= 32) PB_LAUNCH(1);
   else if (C <= 64) PB_LAUNCH(2);
@@ -903,7 +847,6 @@ static int pb_launch(const float* log_probs, long long stride_b, long long strid
   else if (C <= 128) PB_LAUNCH(4);
   else PB_LAUNCH(8);
 #undef PB_LAUNCH
-#undef PB_KERNEL
   HTRVT_LAUNCH_CHECK();
   return HTRVT_OK;
 }
@@ -927,8 +870,8 @@ static int pb_lm_args(const void* lm_table, long long lm_slots, int lm_order, co
 }
 
 // The trie arguments of htrvt_ctc_prefix_beam_lex / _lex_wlm, checked for presence
-static int pb_lex_args_checked(const int* first, const int* label, const int* child, const unsigned char* word_end,
-                               int n_nodes, const unsigned char* is_word, int n_class_map, PbLexArgs& xa) {
+static int pb_trie_args(const int* first, const int* label, const int* child, const unsigned char* word_end,
+                        int n_nodes, const unsigned char* is_word, int n_class_map, PbLexArgs& xa) {
   if (!first || !label || !child || !word_end || n_nodes < 1) return HTRVT_ERR_SHAPE;
   if (n_class_map < 0 || (n_class_map > 0 && !is_word)) return HTRVT_ERR_SHAPE;
   xa.first = first;
@@ -950,8 +893,8 @@ using namespace htrvt;
 extern "C" int htrvt_ctc_prefix_beam(const float* log_probs, long long stride_b, long long stride_t,
                                      const int* lengths, int B, int T, int C, int K, int* ids, int* lens,
                                      double* scores, cudaStream_t stream) {
-  return pb_launch<false, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, PbLmArgs{},
-                                 PbLexArgs{}, stream);
+  return pb_launch<false, false, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores,
+                                        PbLmArgs{}, PbLexArgs{}, PbWlmArgs{}, stream);
 }
 
 // The same search with a character n-gram LM fused into the ranking (header: include/htrvt.h).  lm_table: lm_slots
@@ -966,8 +909,8 @@ extern "C" int htrvt_ctc_prefix_beam_lm(const float* log_probs, long long stride
   PbLmArgs la;
   const int st = pb_lm_args(lm_table, lm_slots, lm_order, tok_map, n_tok_map, alpha, beta, ctc_scores, la);
   if (st != HTRVT_OK) return st;
-  return pb_launch<true, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, PbLexArgs{},
-                               stream);
+  return pb_launch<true, false, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la,
+                                       PbLexArgs{}, PbWlmArgs{}, stream);
 }
 
 // The same search constrained to a word lexicon, with or without the LM (header: include/htrvt.h).  The trie (CSR,
@@ -981,19 +924,20 @@ extern "C" int htrvt_ctc_prefix_beam_lex(const float* log_probs, long long strid
                                          int n_tok_map, double alpha, double beta, int* ids, int* lens,
                                          double* scores, double* ctc_scores, cudaStream_t stream) {
   PbLexArgs xa;
-  const int sx = pb_lex_args_checked(first, label, child, word_end, n_nodes, is_word, n_class_map, xa);
+  const int sx = pb_trie_args(first, label, child, word_end, n_nodes, is_word, n_class_map, xa);
   if (sx != HTRVT_OK || !ctc_scores) return HTRVT_ERR_SHAPE;
   if (!lm_table) {
     if (alpha != 0.0 || beta != 0.0) return HTRVT_ERR_SHAPE;
     PbLmArgs la{};
     la.ctc_scores = ctc_scores;
-    return pb_launch<false, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa,
-                                  stream);
+    return pb_launch<false, true, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la,
+                                         xa, PbWlmArgs{}, stream);
   }
   PbLmArgs la;
   const int st = pb_lm_args(lm_table, lm_slots, lm_order, tok_map, n_tok_map, alpha, beta, ctc_scores, la);
   if (st != HTRVT_OK) return st;
-  return pb_launch<true, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa, stream);
+  return pb_launch<true, true, false>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa,
+                                      PbWlmArgs{}, stream);
 }
 
 // The lexicon-constrained search with a word n-gram LM (header: include/htrvt.h).  Trie as htrvt_ctc_prefix_beam_lex;
@@ -1007,14 +951,16 @@ extern "C" int htrvt_ctc_prefix_beam_lex_wlm(const float* log_probs, long long s
                                              const int* node_tok, const float* smear, double alpha, double beta,
                                              int* ids, int* lens, double* scores, double* ctc_scores,
                                              cudaStream_t stream) {
-  PbWlmArgs wa;
-  if (pb_lex_args_checked(first, label, child, word_end, n_nodes, is_word, n_class_map, wa.lex) != HTRVT_OK)
+  PbLexArgs xa;
+  if (pb_trie_args(first, label, child, word_end, n_nodes, is_word, n_class_map, xa) != HTRVT_OK)
     return HTRVT_ERR_SHAPE;
   if (!node_tok || !smear || lm_order > kWlmMaxOrder) return HTRVT_ERR_SHAPE;
+  PbWlmArgs wa;
   wa.node_tok = node_tok;
   wa.smear = smear;
   PbLmArgs la;
   const int st = pb_lm_args(lm_table, lm_slots, lm_order, nullptr, 0, alpha, beta, ctc_scores, la);
   if (st != HTRVT_OK) return st;
-  return pb_launch<true, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, wa, stream);
+  return pb_launch<true, true, true>(log_probs, stride_b, stride_t, lengths, B, T, C, K, ids, lens, scores, la, xa, wa,
+                                     stream);
 }

@@ -161,6 +161,31 @@ def pack_table(lo, hi, logp, bow):
     return table
 
 
+def pack_grams(grams, tok_of, bits=16):
+    """The packed table of parse_arpa's grams with ARPA tokens mapped to token ids by tok_of, keys of bits-wide fields:
+    -> (table, n-grams kept, n-grams dropped).  An n-gram with a token tok_of does not map can never be queried and is
+    dropped; of a repeated n-gram the last listing wins; <unk> gets UNK_LOG10P when the file lists none."""
+    entries, dropped = {}, 0                          # token-id tuple -> (log10 p, log10 bow)
+    for gk in grams:
+        for toks, p, b in gk:
+            ids = tuple(tok_of.get(t, -1) for t in toks)
+            if min(ids) >= 0:
+                entries[ids] = (p, b)
+            else:
+                dropped += 1
+    entries.setdefault((UNK,), (UNK_LOG10P, 0.0))
+    lo, hi, ps, bs = [], [], [], []
+    for k in range(1, len(grams) + 1):
+        kk = [key for key in entries if len(key) == k]
+        l, h = pack_keys(np.array(kk, dtype=np.int64).reshape(-1, k), bits=bits)
+        lo.append(l)
+        hi.append(h)
+        ps.extend(entries[key][0] for key in kk)
+        bs.extend(entries[key][1] for key in kk)
+    lo, hi = np.concatenate(lo), np.concatenate(hi)
+    return pack_table(lo, hi, np.array(ps, dtype=np.float64), np.array(bs, dtype=np.float64)), len(lo), dropped
+
+
 def table_find(table, lo, hi):
     """Host lookup in a packed table (the kernel's probe): slot index per key, -1 when absent."""
     slots = table.shape[0]
@@ -217,24 +242,8 @@ class CharNGramLM(object):
             if word not in tok_of:
                 tok_of[word] = len(tok_of)
             tmap[c] = tok_of[word]
-        entries = {}                                      # token-id tuple -> (log10 p, log10 bow); a repeat wins
-        for gk in grams:
-            for toks, p, b in gk:
-                ids = tuple(tok_of.get(t, -1) for t in toks)
-                if min(ids) >= 0:                         # else: a token outside the alphabet, never queried
-                    entries[ids] = (p, b)
-        entries.setdefault((UNK,), (UNK_LOG10P, 0.0))
-        lo, hi, ps, bs = [], [], [], []
-        for k in range(1, order + 1):
-            kk = [key for key in entries if len(key) == k]
-            l, h = pack_keys(np.array(kk, dtype=np.int64).reshape(-1, k))
-            lo.append(l)
-            hi.append(h)
-            ps.extend(entries[key][0] for key in kk)
-            bs.extend(entries[key][1] for key in kk)
-        lo, hi = np.concatenate(lo), np.concatenate(hi)
-        table = pack_table(lo, hi, np.array(ps, dtype=np.float64), np.array(bs, dtype=np.float64))
-        return order, counts, table, tmap, len(lo)
+        table, kept, _ = pack_grams(grams, tok_of)
+        return order, counts, table, tmap, kept
 
     @classmethod
     def from_arpa(cls, path, converter, space_token="<space>"):

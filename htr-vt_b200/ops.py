@@ -346,13 +346,12 @@ def greedy_decode_ids(logits, n_character, lengths=None, layout="btc", want_raw=
     return ids, lens, raw
 
 
-def ctc_kbest_paths(log_probs, beam_size, lengths=None, layout="tbc"):
-    """K best alignment paths per line, collapsed (model_window/test_with_kenlm.py:25-51 on device).
-    log_probs fp32 [T,B,C] ("tbc", the reference's layout) or [B,T,C] ("btc").
-    Returns (ids [B,K,T] int32, lens [B,K] int32 (-1 = no such beam), scores [B,K] float64)."""
+def _beam_io(name, log_probs, beam_size, lengths, layout, ctc_scores=False):
+    """The common part of the beam decoders: checks the log-probs, -> (B, T, C, K, sb, st, lengths int32 | None, outs)
+    with outs = [ids [B,K,T] int32, lens [B,K] int32, scores [B,K] float64 (, ctc_scores [B,K] float64)]."""
     _need_cuda(log_probs)
     if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
-        raise HtrvtError("ctc_kbest_paths expects fp32 log-probs with a contiguous class axis")
+        raise HtrvtError("%s expects fp32 log-probs with a contiguous class axis" % name)
     if layout == "btc":
         B, T, C = log_probs.shape
         sb, st = log_probs.stride(0), log_probs.stride(1)
@@ -361,13 +360,20 @@ def ctc_kbest_paths(log_probs, beam_size, lengths=None, layout="tbc"):
         sb, st = log_probs.stride(1), log_probs.stride(0)
     dev = log_probs.device
     K = int(beam_size)
-    ids = torch.empty((B, K, T), dtype=torch.int32, device=dev)
-    lens = torch.empty((B, K), dtype=torch.int32, device=dev)
-    scores = torch.empty((B, K), dtype=torch.float64, device=dev)
+    outs = [torch.empty((B, K, T), dtype=torch.int32, device=dev), torch.empty((B, K), dtype=torch.int32, device=dev)]
+    outs += [torch.empty((B, K), dtype=torch.float64, device=dev) for _ in range(2 if ctc_scores else 1)]
     ln = None if lengths is None else lengths.to(device=dev, dtype=torch.int32).contiguous()
-    check(lib().htrvt_ctc_kbest_paths(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(ids), _p(lens), _p(scores),
-                                      _stream()), "htrvt_ctc_kbest_paths")
-    return ids, lens, scores
+    return B, T, C, K, sb, st, ln, outs
+
+
+def ctc_kbest_paths(log_probs, beam_size, lengths=None, layout="tbc"):
+    """K best alignment paths per line, collapsed (model_window/test_with_kenlm.py:25-51 on device).
+    log_probs fp32 [T,B,C] ("tbc", the reference's layout) or [B,T,C] ("btc").
+    Returns (ids [B,K,T] int32, lens [B,K] int32 (-1 = no such beam), scores [B,K] float64)."""
+    B, T, C, K, sb, st, ln, outs = _beam_io("ctc_kbest_paths", log_probs, beam_size, lengths, layout)
+    check(lib().htrvt_ctc_kbest_paths(_p(log_probs), sb, st, _p(ln), B, T, C, K, *map(_p, outs), _stream()),
+          "htrvt_ctc_kbest_paths")
+    return tuple(outs)
 
 
 def ctc_prefix_beam(log_probs, beam_size, lengths=None, layout="tbc"):
@@ -375,24 +381,10 @@ def ctc_prefix_beam(log_probs, beam_size, lengths=None, layout="tbc"):
     the summed probability of all its alignments - the search SURVEY.md 8(f) row 4 puts in place of the per-frame path
     beam of model_window/test_with_kenlm.py:25-59.  Same arguments and buffers as ctc_kbest_paths.
     Returns (ids [B,K,T] int32 zero padded, lens [B,K] int32 (-1 = no such prefix), scores [B,K] float64, best first)."""
-    _need_cuda(log_probs)
-    if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
-        raise HtrvtError("ctc_prefix_beam expects fp32 log-probs with a contiguous class axis")
-    if layout == "btc":
-        B, T, C = log_probs.shape
-        sb, st = log_probs.stride(0), log_probs.stride(1)
-    else:
-        T, B, C = log_probs.shape
-        sb, st = log_probs.stride(1), log_probs.stride(0)
-    dev = log_probs.device
-    K = int(beam_size)
-    ids = torch.empty((B, K, T), dtype=torch.int32, device=dev)
-    lens = torch.empty((B, K), dtype=torch.int32, device=dev)
-    scores = torch.empty((B, K), dtype=torch.float64, device=dev)
-    ln = None if lengths is None else lengths.to(device=dev, dtype=torch.int32).contiguous()
-    check(lib().htrvt_ctc_prefix_beam(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(ids), _p(lens), _p(scores),
-                                      _stream()), "htrvt_ctc_prefix_beam")
-    return ids, lens, scores
+    B, T, C, K, sb, st, ln, outs = _beam_io("ctc_prefix_beam", log_probs, beam_size, lengths, layout)
+    check(lib().htrvt_ctc_prefix_beam(_p(log_probs), sb, st, _p(ln), B, T, C, K, *map(_p, outs), _stream()),
+          "htrvt_ctc_prefix_beam")
+    return tuple(outs)
 
 
 def ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta=0.0, lengths=None, layout="tbc"):
@@ -402,29 +394,14 @@ def ctc_prefix_beam_lm(log_probs, beam_size, lm, alpha, beta=0.0, lengths=None, 
     order.  alpha = beta = 0 reproduces ctc_prefix_beam's ids, lens and scores bit for bit."""
     if isinstance(lm, WordNGramLM):
         raise ValueError("a word LM scores the words of a lexicon: use ctc_prefix_beam_lex")
-    _need_cuda(log_probs)
-    if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
-        raise HtrvtError("ctc_prefix_beam_lm expects fp32 log-probs with a contiguous class axis")
+    B, T, C, K, sb, st, ln, outs = _beam_io("ctc_prefix_beam_lm", log_probs, beam_size, lengths, layout, True)
     if lm.table.device != log_probs.device:
         raise HtrvtError("ctc_prefix_beam_lm: the LM table lives on %s, the log-probs on %s"
                          % (lm.table.device, log_probs.device))
-    if layout == "btc":
-        B, T, C = log_probs.shape
-        sb, st = log_probs.stride(0), log_probs.stride(1)
-    else:
-        T, B, C = log_probs.shape
-        sb, st = log_probs.stride(1), log_probs.stride(0)
-    dev = log_probs.device
-    K = int(beam_size)
-    ids = torch.empty((B, K, T), dtype=torch.int32, device=dev)
-    lens = torch.empty((B, K), dtype=torch.int32, device=dev)
-    scores = torch.empty((B, K), dtype=torch.float64, device=dev)
-    ctc_scores = torch.empty((B, K), dtype=torch.float64, device=dev)
-    ln = None if lengths is None else lengths.to(device=dev, dtype=torch.int32).contiguous()
     check(lib().htrvt_ctc_prefix_beam_lm(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(lm.table), lm.slots, lm.order,
-                                         _p(lm.token_map), lm.token_map.numel(), float(alpha), float(beta), _p(ids),
-                                         _p(lens), _p(scores), _p(ctc_scores), _stream()), "htrvt_ctc_prefix_beam_lm")
-    return ids, lens, scores, ctc_scores
+                                         _p(lm.token_map), lm.token_map.numel(), float(alpha), float(beta),
+                                         *map(_p, outs), _stream()), "htrvt_ctc_prefix_beam_lm")
+    return tuple(outs)
 
 
 def ctc_prefix_beam_lex(log_probs, beam_size, lexicon, lm=None, alpha=0.0, beta=0.0, lengths=None, layout="tbc"):
@@ -437,45 +414,29 @@ def ctc_prefix_beam_lex(log_probs, beam_size, lexicon, lm=None, alpha=0.0, beta=
     scores [B,K] float64 (fused; = ctc_scores without an LM), ctc_scores [B,K] float64)."""
     if isinstance(lm, WordNGramLM) and lm.lexicon is not lexicon:
         raise ValueError("ctc_prefix_beam_lex: the word LM was built on another lexicon")
-    _need_cuda(log_probs)
-    if log_probs.dtype != torch.float32 or log_probs.stride(-1) != 1:
-        raise HtrvtError("ctc_prefix_beam_lex expects fp32 log-probs with a contiguous class axis")
+    B, T, C, K, sb, st, ln, outs = _beam_io("ctc_prefix_beam_lex", log_probs, beam_size, lengths, layout, True)
     if lexicon.first.device != log_probs.device:
         raise HtrvtError("ctc_prefix_beam_lex: the lexicon lives on %s, the log-probs on %s"
                          % (lexicon.first.device, log_probs.device))
     if lm is not None and lm.table.device != log_probs.device:
         raise HtrvtError("ctc_prefix_beam_lex: the LM table lives on %s, the log-probs on %s"
                          % (lm.table.device, log_probs.device))
-    if layout == "btc":
-        B, T, C = log_probs.shape
-        sb, st = log_probs.stride(0), log_probs.stride(1)
-    else:
-        T, B, C = log_probs.shape
-        sb, st = log_probs.stride(1), log_probs.stride(0)
-    dev = log_probs.device
-    K = int(beam_size)
-    ids = torch.empty((B, K, T), dtype=torch.int32, device=dev)
-    lens = torch.empty((B, K), dtype=torch.int32, device=dev)
-    scores = torch.empty((B, K), dtype=torch.float64, device=dev)
-    ctc_scores = torch.empty((B, K), dtype=torch.float64, device=dev)
-    ln = None if lengths is None else lengths.to(device=dev, dtype=torch.int32).contiguous()
     lx = lexicon
     if isinstance(lm, WordNGramLM):
         check(lib().htrvt_ctc_prefix_beam_lex_wlm(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(lx.first),
                                                   _p(lx.label), _p(lx.child), _p(lx.word_end), lx.n_nodes,
                                                   _p(lx.is_word), lx.is_word.numel(), _p(lm.table), lm.slots, lm.order,
-                                                  _p(lm.node_tok), _p(lm.smear), float(alpha), float(beta), _p(ids),
-                                                  _p(lens), _p(scores), _p(ctc_scores), _stream()),
-              "htrvt_ctc_prefix_beam_lex_wlm")
-        return ids, lens, scores, ctc_scores
+                                                  _p(lm.node_tok), _p(lm.smear), float(alpha), float(beta),
+                                                  *map(_p, outs), _stream()), "htrvt_ctc_prefix_beam_lex_wlm")
+        return tuple(outs)
     lm_args = ((None, 0, 0, None, 0) if lm is None else
                (lm.table, lm.slots, lm.order, lm.token_map, lm.token_map.numel()))
     check(lib().htrvt_ctc_prefix_beam_lex(_p(log_probs), sb, st, _p(ln), B, T, C, K, _p(lx.first), _p(lx.label),
                                           _p(lx.child), _p(lx.word_end), lx.n_nodes, _p(lx.is_word),
                                           lx.is_word.numel(), _p(lm_args[0]), lm_args[1], lm_args[2], _p(lm_args[3]),
-                                          lm_args[4], float(alpha), float(beta), _p(ids), _p(lens), _p(scores),
-                                          _p(ctc_scores), _stream()), "htrvt_ctc_prefix_beam_lex")
-    return ids, lens, scores, ctc_scores
+                                          lm_args[4], float(alpha), float(beta), *map(_p, outs), _stream()),
+          "htrvt_ctc_prefix_beam_lex")
+    return tuple(outs)
 
 
 CtcAlignment = collections.namedtuple("CtcAlignment", "path frame_scores spans token_scores score status")

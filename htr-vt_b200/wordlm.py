@@ -22,7 +22,7 @@ keys hold up to 6 tokens of ids below 2^21 - 1.  Per trie node: node_tok (int32,
 import numpy as np
 import torch
 
-from .lm import UNK, UNK_LOG10P, _SPECIAL, pack_keys, pack_table, parse_arpa
+from .lm import UNK, _SPECIAL, pack_grams, pack_keys, parse_arpa, table_find, table_values
 
 MAX_ORDER = 6
 KEY_BITS = 21
@@ -81,34 +81,15 @@ class WordNGramLM(object):
         for i, w in enumerate(lexicon.words):
             if w in listed and w not in _SPECIAL:
                 tok_of[w] = word_tok[i] = 3 + i
-        entries, n_dropped = {}, 0                                # token-id tuple -> (log10 p, log10 bow); repeat wins
-        for gk in grams:
-            for toks, p, b in gk:
-                ids = tuple(tok_of.get(t, -1) for t in toks)
-                if min(ids) >= 0:
-                    entries[ids] = (p, b)
-                else:
-                    n_dropped += 1
-        entries.setdefault((UNK,), (UNK_LOG10P, 0.0))
-        lo, hi, ps, bs = [], [], [], []
-        for k in range(1, order + 1):
-            kk = [key for key in entries if len(key) == k]
-            l, h = pack_keys(np.array(kk, dtype=np.int64).reshape(-1, k), bits=KEY_BITS)
-            lo.append(l)
-            hi.append(h)
-            ps.extend(entries[key][0] for key in kk)
-            bs.extend(entries[key][1] for key in kk)
-        lo, hi = np.concatenate(lo), np.concatenate(hi)
-        table = pack_table(lo, hi, np.array(ps, dtype=np.float64), np.array(bs, dtype=np.float64))
+        table, kept, n_dropped = pack_grams(grams, tok_of, bits=KEY_BITS)
         first, _, child, word_end = lexicon.trie
         node_tok = np.full(len(word_end), -1, dtype=np.int32)
         node_tok[lexicon.word_node] = word_tok
-        unigram = np.array([entries[(t,)][0] for t in word_tok.tolist()], dtype=np.float64).astype(np.float32)
         node_p = np.full(len(word_end), -np.inf, dtype=np.float32)
-        node_p[lexicon.word_node] = unigram
+        node_p[lexicon.word_node] = table_values(table, table_find(table, *pack_keys(word_tok[:, None], KEY_BITS)))[0]
         smear = node_smear(first, child, node_p)
         n_unk = int((word_tok == UNK).sum())
-        return order, counts, table, node_tok, smear, len(lo), n_dropped, n_unk
+        return order, counts, table, node_tok, smear, kept, n_dropped, n_unk
 
     @classmethod
     def from_arpa(cls, path, lexicon):
